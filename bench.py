@@ -7,6 +7,7 @@ light (SURVEY.md 8(d) "C2"), one step = one IPixelIntegrator.Sample(64) of the w
   torchrun ... bench.py --gpus N ...                     frame stripe-sharded over N GPUs (one process each) + NCCL gather
   python bench.py --impl reference ...                   the reference's CPU algorithm (the oracle
                                                          restatement; .NET is not in this image)
+  --dump-outputs DIR                                     also write the frame of the last timed step (DIR/color.npy)
 
 value   : whole-job Mrays/s, scene + path state resident in HBM, result left in HBM (device timed)
 e2e     : same metric through the reference-facing call with HOST buffers -- scene upload + Sample -> Color[w,h] on the
@@ -54,7 +55,24 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C3/C4/C5 table (about a minute at N=1)")
     ap.add_argument("--no-primary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the Color[w,h] frame of the last timed step to DIR/color.npy (float32) to compare builds")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, color):
+    """Writes Color[w,h] as float32.  A frame above DUMP_LIMIT (the 4K configs) keeps every s-th pixel along both axes,
+    with the smallest s that fits, so the same arguments always select the same pixels."""
+    a = color.astype(np.float32)
+    s = 1
+    while a[::s, ::s].nbytes > DUMP_LIMIT:
+        s += 1
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "color.npy"), np.ascontiguousarray(a[::s, ::s]))
+    print(f"bench: wrote {out_dir}/color.npy, Color[w,h] of the last timed step, pixel stride {s}", file=sys.stderr, flush=True)
 
 
 def peaks():
@@ -135,6 +153,8 @@ def run_reference(args, rank, world):
     for k in range(args.steps):
         o.sample(REF_SPP, seed=1, first_sample=k * REF_SPP, out=tex, threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tex)
     # rays per step: count them with one instrumented (slower, untimed) step
     _, st = o.sample(REF_SPP, seed=1, stats=True, threads=cores)
     rays = st["closest_rays"] + st["wasted_rays"] + st["shadow_rays"]
@@ -266,6 +286,8 @@ def main():
         stats.append(st)
     sync_all()
     wall = time.perf_counter() - wall0
+    # the later legs render into the same frame
+    last_frame = sharded.frame.cpu().numpy() if args.dump_outputs and rank == 0 else None
     # a timed region shorter than a few sampling periods (8 GPUs: 5 x 10 ms) may hold no sample: keep the same load
     # running, untimed, until three rows exist (all ranks take part: the step has a collective)
     extra = 0
@@ -278,6 +300,8 @@ def main():
         step(0)
         extra += 1
     clk = clocks.stop(wall0) if rank == 0 else None
+    if last_frame is not None:
+        dump_outputs(args.dump_outputs, last_frame)
     if clk is not None:
         clk["window"] = "timed region" if extra == 0 else f"timed region + {extra} identical untimed steps (region shorter than the sampling period)"
 

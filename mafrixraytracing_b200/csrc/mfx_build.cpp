@@ -292,6 +292,27 @@ static void sah_build(SahCtx &c, int root, int par_depth)
     for (auto &f : spawned) f.get();
 }
 
+// The forked levels of sah_build take their node indices from one counter in whatever order the threads reach it; the
+// splits themselves do not depend on the schedule.  The reinsertion pass breaks ties by node index, so before it runs
+// the nodes are renumbered in the order a serial build allocates them: the same tree for any fork depth and schedule.
+static void sah_renumber_serial(std::vector<SahNode> &nodes)
+{
+    std::vector<SahNode> out(nodes.size());
+    std::vector<std::pair<int, int>> todo{ { 0, 0 } };         // (index in `nodes`, index in `out`)
+    int next = 1;
+    while (!todo.empty()) {
+        const auto [from, to] = todo.back(); todo.pop_back();
+        SahNode nd = nodes[from];
+        if (nd.count == 0) {
+            todo.push_back({ nd.right, next + 1 }); todo.push_back({ nd.left, next });
+            nd.left = next; nd.right = next + 1;
+            next += 2;
+        }
+        out[to] = nd;
+    }
+    nodes.swap(out);
+}
+
 // Insertion-based optimisation of the binary tree (after Bittner, Hapala, Havran 2013): take a subtree out, let its sibling
 // move up, and put it back where the sum of the interior nodes' areas grows least -- found by branch and bound from the
 // root (induced cost = what the ancestors of a candidate grow by; a subtree can never cost less than its own area).
@@ -402,6 +423,8 @@ void mfx_build_own_tree(const float *lo, const float *hi, int ns, int max_leaf, 
     nodes[0].first = 0; nodes[0].count = ns; nodes[0].left = nodes[0].right = -1;
     sah_bound(c, nodes[0]);
     sah_build(c, 0, par_depth);
+    sah_renumber_serial(nodes);
+    c.nodes = nodes.data();
     // MFX_TREE_OPT = reinsertion passes over the binary tree before it is collapsed (0: off), each over the
     // MFX_TREE_OPT_NODES largest subtrees; scenes above MFX_TREE_OPT_MAX primitives skip it (the pass is sequential)
     {

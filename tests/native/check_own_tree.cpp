@@ -40,7 +40,7 @@ int main(int argc, char **argv)
         }
     }
     MfxOwnTree t;
-    mfx_build_own_tree(lo.data(), hi.data(), n, max_leaf, 1.0f, 3, t);
+    mfx_build_own_tree(lo.data(), hi.data(), n, max_leaf, 1.0f, (int)mfx_env_long("MFX_BVH_BUILD_PAR_DEPTH", 3), t);
     REQUIRE((int)t.order.size() == n);
     std::vector<int> seen(n, 0);
     for (int v : t.order) { REQUIRE(v >= 0 && v < n); seen[v]++; }
@@ -94,7 +94,12 @@ int main(int argc, char **argv)
         const double x = rhi[0] - rlo[0], y = rhi[1] - rlo[1], z = rhi[2] - rlo[2];
         cost += x * y + y * z + z * x;
     }
-    printf("ok n=%d mode=%d records=%zu depth=%d cost=%.6g\n", n, mode, t.quads.size(), t.depth, cost);
+    // FNV-1a over the records and the slot order: equal trees print equal hashes
+    unsigned long long hash = 1469598103934665603ull;
+    auto mix = [&](const void *p, size_t bytes) { for (size_t k = 0; k < bytes; k++) hash = (hash ^ ((const unsigned char *)p)[k]) * 1099511628211ull; };
+    mix(t.quads.data(), t.quads.size() * sizeof(QuadF));
+    mix(t.order.data(), t.order.size() * sizeof(int));
+    printf("ok n=%d mode=%d records=%zu depth=%d cost=%.6g tree=%016llx\n", n, mode, t.quads.size(), t.depth, cost, hash);
     if (mode == 3) {
         long kids[5] = { 0, 0, 0, 0, 0 }, leafsz[8] = { 0, 0, 0, 0, 0, 0, 0, 0 }, leaves = 0, inner = 0;
         for (const QuadF &q : t.quads) {

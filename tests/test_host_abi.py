@@ -54,14 +54,19 @@ int main(void) {
     assert got == want
 
 
-def test_own_tree_builder_is_a_valid_bvh(tmp_path):
-    """The fast path's own SAH tree (csrc/mfx_build.cpp) compiled for the host alone and checked structurally: every
-    slot exactly once, every stored box contains its subtree, leaves <= 4, links and depth consistent -- for random
-    boxes, coincident boxes (no centroid spread to split on) and a few huge boxes among many small ones."""
+def _build_check_own_tree(tmp_path):
     exe = str(tmp_path / "check_own_tree")
     csrc = os.path.join(ROOT, "mafrixraytracing_b200", "csrc")
     subprocess.check_call(["/usr/bin/g++", "-std=c++17", "-O2", "-pthread", "-I", "/usr/local/cuda/include", "-I", csrc, "-o", exe,
                            os.path.join(ROOT, "tests", "native", "check_own_tree.cpp"), os.path.join(csrc, "mfx_build.cpp")])
+    return exe
+
+
+def test_own_tree_builder_is_a_valid_bvh(tmp_path):
+    """The fast path's own SAH tree (csrc/mfx_build.cpp) compiled for the host alone and checked structurally: every
+    slot exactly once, every stored box contains its subtree, leaves <= 4, links and depth consistent -- for random
+    boxes, coincident boxes (no centroid spread to split on) and a few huge boxes among many small ones."""
+    exe = _build_check_own_tree(tmp_path)
     for n, mode in [(1, 0), (2, 0), (3, 0), (5, 0), (17, 0), (1000, 0), (150000, 0), (3000, 1), (5000, 2)]:
         out = subprocess.check_output([exe, str(n), str(mode)], text=True)
         assert out.startswith(f"ok n={n} mode={mode}"), out
@@ -70,7 +75,7 @@ def test_own_tree_builder_is_a_valid_bvh(tmp_path):
     def cost(n, mode, **env):
         out = subprocess.check_output([exe, str(n), str(mode)], text=True, env=dict(os.environ, **env))
         assert out.startswith(f"ok n={n} mode={mode}"), (env, out)
-        return float(out.split("cost=")[1])
+        return float(out.split("cost=")[1].split()[0])
     for n, mode in [(5, 0), (17, 0), (1000, 0), (40000, 0), (3000, 1), (5000, 2)]:
         base = cost(n, mode, MFX_TREE_OPT="0")
         for env in (dict(MFX_TREE_OPT="1"), dict(MFX_TREE_OPT="4"), dict(MFX_TREE_OPT="2", MFX_TREE_OPT_NODES="50"), dict(MFX_TREE_OPT="2", MFX_TREE_OPT_MAX="10")):
@@ -84,6 +89,26 @@ def test_own_tree_builder_is_a_valid_bvh(tmp_path):
         for n, mode in [(1, 0), (3, 0), (5, 0), (17, 0), (1000, 0), (40000, 0), (3000, 1), (5000, 2)]:
             out = subprocess.check_output([exe, str(n), str(mode)], text=True, env=dict(os.environ, MFX_COLLAPSE_DP=dp))
             assert out.startswith(f"ok n={n} mode={mode}"), (dp, out)
+
+
+def test_own_tree_does_not_depend_on_the_fork_depth(tmp_path):
+    """The builder forks its top levels over threads.  The tree must be the same for any fork depth and any schedule of
+    those threads: the spot mesh of C2 has many subtrees of equal area, where the reinsertion pass breaks ties by node
+    index, so node indices handed out in the threads' order would change the tree from run to run."""
+    exe = _build_check_own_tree(tmp_path)
+    tris = []
+    for p in scenes.c2_spot().prims:
+        tris.append(p["v"][:9])
+        if p["kind"] == 1:                                    # a Rect is two triangles, as the fast path slots it
+            tris.append(np.concatenate([p["v"][0:3], p["v"][6:9], p["v"][9:12]]))
+    path = str(tmp_path / "tris.bin")
+    np.array(tris, np.float64).tofile(path)
+    trees = set()
+    for depth in ("0", "1", "2", "3", "3", "5", "5", "5"):
+        out = subprocess.check_output([exe, str(len(tris)), "3", path], text=True, env=dict(os.environ, MFX_BVH_BUILD_PAR_DEPTH=depth))
+        assert out.startswith(f"ok n={len(tris)} mode=3"), out
+        trees.add(out.split("tree=")[1].split()[0])
+    assert len(trees) == 1, trees
 
 
 def test_fsharp_shim_offsets_match_the_header():
