@@ -605,6 +605,7 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
 #define STACK_PUT(I, K)                                                                                              \
             { const int i_ = (I); const uint2 v_ = make_uint2((K), (unsigned)node);                                  \
               DBG_CHECK(i_ >= 0 && i_ < 3 * sc.own_depth, w.counts);                                                  \
+              DBG_CHECK(i_ < S || blockIdx.x * FAST_BLOCK + threadIdx.x < (unsigned)sc.spill_threads, w.counts);       \
               if (i_ < S) my_stack[(size_t)i_ * FAST_BLOCK] = v_; else my_spill[(size_t)(i_ - S) * spill_stride] = v_; }
             if (m >= 1) STACK_PUT(sp + m - 1, p0)
             if (m >= 2) STACK_PUT(sp + m - 2, p1)
@@ -1237,6 +1238,7 @@ static void launch_trace5(const LaunchCfg &c, const SceneF &sc, const WaveF &w, 
     if (sc.has_big_sphere) launch_trace5b<ANY, true, RT, LT, NS>(c, sc, w, bounce);
     else launch_trace5b<ANY, false, RT, LT, NS>(c, sc, w, bounce);
 }
+static_assert(MFX_STACK_SMEM_MAX * FAST_BLOCK * sizeof(uint2) <= 48 * 1024, "the own-tree stack must launch without a shared-memory opt-in");
 template <bool ANY, bool BIG, int RT, int LT, int NS, int NL, int MB, bool CNT = false, bool CMP = false, bool TAIL = false>
 static void launch_trace6b(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr = nullptr, const SkyCtx &sky = SkyCtx{})
 {

@@ -181,6 +181,7 @@ struct MfxScene {
     cudaStream_t stream2 = nullptr;          // shadow queries of bounce b run beside the closest hits of bounce b+1 (run_sample)
     float4 *sh2[3] = { nullptr, nullptr, nullptr };   // second shadow queue (sh_o, sh_d, sh_c) of the two-stream mode
     int sh2_P = 0;
+    uint2 *spill2 = nullptr;                 // the shadow launches' own stack spill columns in that mode (sized like sf.stack_spill)
     std::vector<MfxPrim> prims;
     std::vector<MfxMaterial> mats;
     std::vector<MfxBvhNode> nodes;
@@ -919,7 +920,7 @@ static int flatten_fast(MfxScene *s)
     sf.root_meta = -1;
     sf.own_tree = 1; sf.own_depth = host->depth;
     const int need = 3 * host->depth;
-    sf.stack_smem = (int)std::min((long)need, std::max(1L, env_long("MFX_STACK_SMEM", 12)));
+    sf.stack_smem = (int)std::min((long)std::min(need, MFX_STACK_SMEM_MAX), std::max(1L, env_long("MFX_STACK_SMEM", 12)));
     sf.spill_threads = s->sm_count * 16 * 128;                  // most threads a persistent 128-thread grid can hold
     if (need > sf.stack_smem) {
         MFX_TRY(dev_alloc_t(s, &sf.stack_spill, (size_t)(need - sf.stack_smem) * sf.spill_threads));
@@ -1397,6 +1398,16 @@ static int launch_sample(MfxScene *s, const MfxSampleParams *p, double *d_color_
     }
     WaveF wf_alt = s->wf;
     if (two) { wf_alt.sh_o = s->sh2[0]; wf_alt.sh_d = s->sh2[1]; wf_alt.sh_c = s->sh2[2]; }
+    // ... and spill columns of their own: a thread's stack column is picked by its block and lane, so a shadow grid and a
+    // closest-hit grid beside it would push and pop each other's deferred subtrees (missed occluders, wrong hits)
+    const SceneF *sfp_sh = sfp;
+    SceneF sf_sh;
+    if (two && sfp->stack_spill) {
+        if (!s->spill2) MFX_TRY(dev_alloc_t(s, &s->spill2, (size_t)(3 * sfp->own_depth - sfp->stack_smem) * sfp->spill_threads));
+        sf_sh = *sfp;
+        sf_sh.stack_spill = s->spill2;
+        sfp_sh = &sf_sh;
+    }
     cudaEvent_t e_shadow_done[2] = { nullptr, nullptr };
 
     const int P = exact ? s->wx.P : s->wf.P;
@@ -1482,7 +1493,7 @@ static int launch_sample(MfxScene *s, const MfxSampleParams *p, double *d_color_
                 MFX_TRY(timed(1, st2));
                 if (exact && hyb_x) mfx_h_shadow_x(cfg, s->sx, s->sf_ref, s->sh, s->wx, b);
                 else if (exact) mfx_x_shadow(cfg, s->sx, s->wx, b, ctr);
-                else mfx_f_shadow(cfg2, *sfp, wq, b, ctr);
+                else mfx_f_shadow(cfg2, *sfp_sh, wq, b, ctr);
                 MFX_TRY(timed_end(st2));
                 if (two) {
                     MFX_TRY(get_event(job, ev++, &e_shadow_done[b & 1]));

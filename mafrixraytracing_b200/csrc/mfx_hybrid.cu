@@ -253,6 +253,7 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_h_trace(SceneF sc, const N
 #define STACK_PUT(I, K)                                                                                              \
             { const int i_ = (I); const uint2 v_ = make_uint2((K), (unsigned)node);                                  \
               DBG_CHECK(i_ >= 0 && i_ < 3 * sc.own_depth, w.counts);                                                  \
+              DBG_CHECK(i_ < S || blockIdx.x * FAST_BLOCK + threadIdx.x < (unsigned)sc.spill_threads, w.counts);       \
               if (i_ < S) my_stack[(size_t)i_ * FAST_BLOCK] = v_; else my_spill[(size_t)(i_ - S) * spill_stride] = v_; }
             if (m >= 1) STACK_PUT(sp + m - 1, k1)
             if (m >= 2) STACK_PUT(sp + m - 2, k2)

@@ -11,6 +11,8 @@
 #define MFX_MODE_SKY 2             // MFX_SKY_TRACER: GetColor of RenderTest/Sample/RayTracing.fs:367-382
 #define MFX_SKY_TMIN 0.00001       // ListHit(hitable, ray, 0.00001, 10000000), RayTracing.fs:368
 #define MFX_SKY_TMAX 10000000.
+#define MFX_STACK_SMEM_MAX 48      // own-tree stack entries in shared memory: [48][128 threads] x 8 B = the 48 KB a block
+                                   // gets without opting in to more (MFX_STACK_SMEM is capped there)
 
 // ------------------------------------------------------------------ exact (f64) device layout
 // One BvhNode, heap-indexed like the reference (children 2i+1 / 2i+2).  64 B.
@@ -155,8 +157,9 @@ struct SceneF {
     int    qpar;            // 0: quads at even depths; 1: 2-slot pseudo root + quads at odd depths (odd leaf depth)
     int    own_tree;        // 0: pairs/quads follow the reference tree (heap-indexed); 1: quads are the SAH 4-wide tree
     int    own_depth;       // own tree: number of quad levels (deferred-hit stack holds <= 3 per level)
-    int    stack_smem;      // own tree: stack entries kept in shared memory per thread
-    uint2 *stack_spill;     // own tree: [3*own_depth - stack_smem][spill_threads] overflow entries (null if none)
+    int    stack_smem;      // own tree: stack entries kept in shared memory per thread (<= MFX_STACK_SMEM_MAX)
+    uint2 *stack_spill;     // own tree: [3*own_depth - stack_smem][spill_threads] overflow entries (null if none); every
+                            // launch that may run beside another one needs columns of its own
     int    spill_threads;
 };
 

@@ -4,6 +4,9 @@
 // 4-wide node step, nearest child first (shadow queries: farthest first), deferred hits culled by their entry distance
 // at pop time, leaves of the chosen child tested at once, first hit ends a shadow ray, a ray never re-hits the triangle
 // it starts on.  One thread, f32.
+// It also reports the traversal stack's height per query kind: the peak, and how many rays push deeper than the
+// entries the kernels keep in shared memory (MFX_STACK_SMEM, default 12) and so use the spill columns in global memory,
+// against 3*depth, the bound those columns are sized for (csrc/mfx_host.cpp flatten_fast).
 // The GPU's own counters (MFX_SAMPLE_COUNT_OWN_TREE, bench.py `own_tree`) are what validates this model: C2 measures
 // 3.35 records + 2.07 triangle tests per closest-hit ray and, with shadow queries still nearest-first
 // (SIM_ANY_NEAREST=1 here), 4.19 + 1.65 per shadow ray.
@@ -13,6 +16,7 @@
 // usage:  own_tree_sim tris.bin n [width height [camera and light, see main]]      tris.bin = n x 9 doubles (tools/own_tree_sim.py)
 // env:    MFX_COLLAPSE_DP / MFX_SAH_MAX_LEAF / MFX_SAH_TRAV_COST_PCT   the builder's knobs
 //         SIM_ANY_NEAREST=1         shadow queries visit the nearest child first (the kernel up to the last GPU run of round 1)
+//         MFX_STACK_SMEM=k          the stack entries kept in shared memory, for the count of rays above it (default 12)
 //         SIM_SHADOW_FROM_LIGHT=1   trace every shadow ray from the light sample towards the surface point instead (same
 //                                   segment, same answer); the run always prints both directions split by outcome
 #include "mfx_build.h"
@@ -42,9 +46,10 @@ static unsigned as_uint(float f) { unsigned i; memcpy(&i, &f, 4); return i; }
 static float as_float(unsigned u) { float f; memcpy(&f, &u, 4); return f; }
 
 static bool g_any_nearest = false;
+static int g_smem = 12;         // MFX_STACK_SMEM
 static int g_quant = 0;          // SIM_QUANT: 1 = boxes replaced by their 8-bit grid planes (QuadC), 2 = plus the kernel's one-fma plane arithmetic
 struct Tri { V v0, e1, e2, n; };
-struct Counts { double rays = 0, records = 0, tris = 0, leaf_visits = 0; };
+struct Counts { double rays = 0, records = 0, tris = 0, leaf_visits = 0, deep = 0; int peak = 0; };   // deep: rays whose stack rose above g_smem
 
 struct Sim {
     const MfxOwnTree *t;
@@ -79,7 +84,7 @@ struct Sim {
         const V ood = { o.x * id.x, o.y * id.y, o.z * id.z };
         float best = tmax; int best_slot = -1;
         struct E { unsigned key; int rec; };
-        E stack[256]; int sp = 0;
+        E stack[256]; int sp = 0, peak = 0;
         int node = 0, leaf = -1; bool need_pop = false;
         c.rays++;
         for (;;) {
@@ -113,6 +118,7 @@ struct Sim {
                 }
                 std::sort(key, key + 4);
                 for (int k = 3; k >= 1; k--) if (key[k] != 0x7f800000u) stack[sp++] = { key[k], node };      // nearest on top
+                peak = std::max(peak, sp);
                 need_pop = true;
                 if (key[0] != 0x7f800000u) {
                     const int link = as_int((&q.meta.x)[key[0] & 3u]);
@@ -138,6 +144,8 @@ struct Sim {
                 if (!got) break;
             }
         }
+        c.peak = std::max(c.peak, peak);
+        if (peak > g_smem) c.deep++;
         t_out = best;
         return best_slot;
     }
@@ -149,6 +157,7 @@ int main(int argc, char **argv)
     if (argc < 3) { fprintf(stderr, "usage: own_tree_sim tris.bin n [width height]\n"); return 2; }
     const int n = atoi(argv[2]);
     g_any_nearest = getenv("SIM_ANY_NEAREST") != nullptr;
+    g_smem = (int)std::max(1L, mfx_env_long("MFX_STACK_SMEM", 12));
     const int W = argc > 3 ? atoi(argv[3]) : 480, H = argc > 4 ? atoi(argv[4]) : 270;
     FILE *f = fopen(argv[1], "rb");
     if (!f) { fprintf(stderr, "cannot open %s\n", argv[1]); return 2; }
@@ -246,6 +255,7 @@ int main(int argc, char **argv)
                 g_st[occ][0][0] += a.records; g_st[occ][0][1] += a.tris; g_st[occ][1][0] += r.records; g_st[occ][1][1] += r.tris;
                 const Counts &use = getenv("SIM_SHADOW_FROM_LIGHT") ? r : a;
                 sh[b].rays += 1; sh[b].records += use.records; sh[b].tris += use.tris;
+                sh[b].deep += use.deep; sh[b].peak = std::max(sh[b].peak, use.peak);
             }
             // uniform hemisphere about the (unflipped) geometric normal
             const float z = 1.f - 2.f * U(rng), r = std::sqrt(std::max(0.f, 1.f - z * z)), ph = 6.2831853f * U(rng);
@@ -262,8 +272,14 @@ int main(int argc, char **argv)
         printf("bounce %d: closest %9.0f rays %.3f records %.3f tris | shadow %9.0f rays %.3f records %.3f tris\n", b, cl[b].rays,
                cl[b].records / std::max(cl[b].rays, 1.0), cl[b].tris / std::max(cl[b].rays, 1.0), sh[b].rays, sh[b].records / std::max(sh[b].rays, 1.0), sh[b].tris / std::max(sh[b].rays, 1.0));
         C.rays += cl[b].rays; C.records += cl[b].records; C.tris += cl[b].tris; S.rays += sh[b].rays; S.records += sh[b].records; S.tris += sh[b].tris;
+        C.deep += cl[b].deep; S.deep += sh[b].deep; C.peak = std::max(C.peak, cl[b].peak); S.peak = std::max(S.peak, sh[b].peak);
     }
     printf("all: closest %.3f records + %.3f tris per ray (GPU counters on C2: 3.35 + 2.07); shadow %.3f + %.3f (GPU, nearest-first shadow queries: 4.19 + 1.65)\n",
            C.records / C.rays, C.tris / C.rays, S.records / S.rays, S.tris / S.rays);
+    for (int k = 0; k < 2; k++) {
+        const Counts &q = k ? S : C;
+        printf("stack, %s: peak %d entries, 3*depth %d; %.0f of %.0f rays above %d entries (%.4f)\n", k ? "shadow" : "closest", q.peak, 3 * tree.depth,
+               q.deep, q.rays, g_smem, q.deep / std::max(q.rays, 1.0));
+    }
     return 0;
 }
