@@ -87,10 +87,14 @@ __device__ __forceinline__ bool leaf_f3(const SceneF &sc, const RayF &r, int met
                 const float t1 = (q != 0.f) ? cc / q : q;
                 lo = fminf(q, t1); hi = fmaxf(q, t1);
             }
+            // a ray leaving a convex surface outward cannot re-hit it; one entering takes the far root.  Near grazing the
+            // f32 discriminant of a ray that starts on the sphere (hb^2, against rounding of r^2) can come out <= 0:
+            // the entering ray then takes the chord -2 hb, which an origin on the surface gives exactly
+            const bool src = (prim == r.src);
+            if (src && !real && hb < 0.f) { real = true; hi = -2.f * hb; }
             if (real) {
                 bool skip = false;
-                // a ray leaving a convex surface outward cannot re-hit it; one entering takes the far root
-                if (prim == r.src) { skip = (hb >= 0.f); lo = -1.f; }
+                if (src) { skip = (hb >= 0.f); lo = -1.f; }
                 float t = -1.f;
                 if (lo >= r.tmin && lo < best_t) t = lo;
                 else if (hi > r.tmin && hi < best_t) t = hi;
