@@ -546,52 +546,3 @@ void mfx_build_own_tree(const float *lo, const float *hi, int ns, int max_leaf, 
     }
     out.depth = own_depth;
 }
-
-// QuadF -> QuadC: per record and axis a grid of 256 planes (f32 origin, power-of-two step) that holds every child plane
-// with half a step to spare on both sides; min planes go down, max planes up.
-void mfx_compress_quads(const std::vector<QuadF> &quads, std::vector<QuadC> &out)
-{
-    out.resize(quads.size());
-    const size_t nq = quads.size();
-    const unsigned nthr = (unsigned)std::max(1L, std::min(16L, (long)(nq / 65536)));
-    auto work = [&](size_t q0, size_t q1) {
-        for (size_t qi = q0; qi < q1; qi++) {
-            const QuadF &q = quads[qi];
-            QuadC c; memset(&c, 0, sizeof(c));
-            const float *lo[3] = { &q.lox.x, &q.loy.x, &q.loz.x }, *hi[3] = { &q.hix.x, &q.hiy.x, &q.hiz.x };
-            const int *meta = reinterpret_cast<const int *>(&q.meta);
-            float org[3], stp[3]; unsigned wl[3], wh[3];
-            for (int a = 0; a < 3; a++) {
-                double nlo = 1e300, nhi = -1e300;
-                for (int k = 0; k < 4; k++) if (meta[k] != MFX_QUAD_EMPTY) { nlo = std::min(nlo, (double)lo[a][k]); nhi = std::max(nhi, (double)hi[a][k]); }
-                if (nlo > nhi) { nlo = nhi = 0.; }
-                const double ext = nhi - nlo, mag = std::max(std::fabs(nlo), std::fabs(nhi));
-                int e = ext > 0. ? (int)std::ceil(std::log2(ext / 252.)) : -100;
-                if (mag > 0.) e = std::max(e, (int)std::floor(std::log2(mag)) - 21);    // the f32 origin must resolve the step
-                e = std::max(-100, std::min(100, e));
-                for (;; e++) {
-                    const double step = std::ldexp(1., e);
-                    float of = (float)(nlo - step);
-                    if ((double)of > nlo - step) of = std::nextafterf(of, -INFINITY);
-                    bool ok = true; unsigned l = 0, h = 0;
-                    for (int k = 0; k < 4 && ok; k++) {
-                        if (meta[k] == MFX_QUAD_EMPTY) continue;
-                        const double ql = std::floor(((double)lo[a][k] - (double)of) / step - 0.5), qh = std::ceil(((double)hi[a][k] - (double)of) / step + 0.5);
-                        if (ql < 0. || qh > 255.) ok = false;
-                        else { l |= (unsigned)ql << (8 * k); h |= (unsigned)qh << (8 * k); }
-                    }
-                    if (ok || e >= 120) { org[a] = of; stp[a] = (float)step; wl[a] = l; wh[a] = h; break; }
-                }
-            }
-            c.ox = org[0]; c.oy = org[1]; c.oz = org[2]; c.sx = stp[0]; c.sy = stp[1]; c.sz = stp[2];
-            c.lox = wl[0]; c.loy = wl[1]; c.loz = wl[2]; c.hix = wh[0]; c.hiy = wh[1]; c.hiz = wh[2];
-            for (int k = 0; k < 4; k++) c.meta[k] = meta[k];
-            out[qi] = c;
-        }
-    };
-    if (nthr <= 1) { work(0, nq); return; }
-    std::vector<std::thread> th;
-    for (unsigned t = 0; t < nthr; t++) th.emplace_back(work, nq * t / nthr, nq * (t + 1) / nthr);
-    for (auto &x : th) x.join();
-}
-

@@ -16,5 +16,3 @@ struct MfxOwnTree {
     int depth = 0;              // number of record levels (the traversal stack holds <= 3 entries per level)
 };
 void mfx_build_own_tree(const float *lo, const float *hi, int n, int max_leaf, float trav_cost, int par_depth, MfxOwnTree &out);
-// the same records on 8-bit grids (QuadC, mfx_internal.h): planes moved outward by half a step more than quantisation needs
-void mfx_compress_quads(const std::vector<QuadF> &quads, std::vector<QuadC> &out);

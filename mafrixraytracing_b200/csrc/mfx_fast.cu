@@ -3,13 +3,12 @@
 // Layouts (mfx_internal.h, built by mfx_host.cpp / mfx_build.cpp):
 //   * own tree (default): 128 B records of four child boxes + links over a binned-SAH BVH of the fast slots,
 //     48 B primitive slots in that tree's leaf order, 16 B normal+material side array for the shade kernel;
-//   * reference tree (instrumented counting runs, cross-check variants): 64 B children pairs and 128 B
-//     grandchildren quads indexed by the reference's heap index (BvhNode.fs:40-41), slots in its leaf order.
+//   * reference tree (instrumented counting runs): 64 B children pairs indexed by the reference's heap index
+//     (BvhNode.fs:40-41), slots in its leaf order.
 // Traversal kernels: one ray per lane in persistent warps, ordered descent, t-shrink, ray replacement from the
 // bounce's queue, vote-postponed leaf tests.
 //   k_f_trace6  own tree, sorted 4-wide node step, stack of (key, record) entries in shared memory   <- shipped
-//   k_f_trace5  reference tree, two levels per fetch, stackless (2 bits per level trail + heap index)
-//   k_f_trace4  reference tree, binary, stackless (1 bit per level); also the COUNT-instrumented kernel
+//   k_f_trace4  reference tree, binary, stackless (1 bit per level): the COUNT-instrumented kernel
 // Path state lives at QUEUE POSITIONS (WaveF, mfx_internal.h): entry i of buffer b & 1 is the i-th ray of bounce b, the
 // shade kernel writes its survivors densely into the other buffer and its shadow rays densely into sh_*; no queue of
 // path ids, no gathers.
@@ -170,10 +169,10 @@ __global__ void __launch_bounds__(256) k_f_raygen(SceneF sc, WaveF w, TileMap tm
 // ---------------------------------------------------------------- persistent-warp traversal
 // The first kernel (one ray per thread, grid-stride) kept only 5-8 of 32 lanes busy on secondary
 // bounces (profiles/r01_v1_baseline_summary.md).  This one keeps every warp resident and
-//   (1) REPLACES finished rays: when >= REFILL_T lanes are idle the warp claims that many queue
+//   (1) REPLACES finished rays: when >= TRACE4_REFILL_T lanes are idle the warp claims that many queue
 //       entries with one atomicAdd (ballot/popc/shuffle) and the idle lanes start new rays;
 //   (2) POSTPONES leaf tests by vote: a lane that reached leaves parks them (two leaf metas in
-//       registers) and idles until >= LEAF_T lanes hold leaves or nobody has node work left, so
+//       registers) and idles until >= TRACE4_LEAF_T lanes hold leaves or nobody has node work left, so
 //       the (branch-free) triangle tests run with many lanes instead of one or two;
 //   (3) keeps the node step branch-light: the descend decision is a handful of selects, the push
 //       of the far child is a predicated shared store, the level is tracked in a register; only
@@ -182,7 +181,9 @@ __global__ void __launch_bounds__(256) k_f_raygen(SceneF sc, WaveF w, TileMap tm
 // Per-lane traversal state: heap index, 32-bit trail, level, best hit -- all registers; the far
 // child's entry distance per level sits in shared memory ([level][thread], conflict free).
 // A watchdog bounds the loop so a logic error can never hang the GPU (flag in counts[]).
-template <bool ANY, bool COUNT, bool BIG, int REFILL_T, int LEAF_T, int NSTEP>
+// The kernel runs the instrumented counting runs only: it always counts (records fetched, triangle and sphere tests).
+constexpr int TRACE4_REFILL_T = 12, TRACE4_LEAF_T = 16, TRACE4_NSTEP = 2;
+template <bool ANY, bool BIG>
 __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int bounce, TravCounters *ctr)
 {
     extern __shared__ float s_dyn[];
@@ -207,7 +208,7 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
         const unsigned idle = __ballot_sync(FULL, pid < 0);
         unsigned idle_now = idle;
         if (++iters > (1u << 22)) { if (lane == 0) atomicAdd(&w.counts[MFX_COUNTS_LEN - 1], 1); break; }   // watchdog
-        if (!exhausted && __popc(idle) >= REFILL_T) {
+        if (!exhausted && __popc(idle) >= TRACE4_REFILL_T) {
             const int nidle = __popc(idle);
             int base = 0;
             if (lane == 0) base = atomicAdd(cursor, nidle);
@@ -223,7 +224,7 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
                     best_t = ANY ? d.w - 1e-6f : w.tmax;                // shadow: dist - 1e-6 (Integrators.fs:44); closest: tMax (:108)
                     best_slot = -1; pend = 0u; leafA = leafB = -1; h = 1u; depth = 0u;
                     float e;
-                    if (COUNT) local[0]++;
+                    local[0]++;
                     const bool in = box_f(r, sc.root_min[0], sc.root_min[1], sc.root_min[2], sc.root_max[0], sc.root_max[1], sc.root_max[2], best_t, e);
                     needPop = !in || sc.root_meta >= 0;     // nothing to descend into: the (empty) trail pop ends the ray
                     if (in && sc.root_meta >= 0) leafA = sc.root_meta;
@@ -233,14 +234,14 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
         }
         if (idle_now == FULL) { if (exhausted) break; continue; }
 
-        // ---- node step(s) (lanes holding a node to visit and no parked leaves); NSTEP > 1 amortises the
+        // ---- node step(s) (lanes holding a node to visit and no parked leaves); TRACE4_NSTEP > 1 amortises the
         //      loop skeleton (ballots, vote, refill test) over several tree levels
 #pragma unroll
-        for (int rep = 0; rep < NSTEP; rep++)
+        for (int rep = 0; rep < TRACE4_NSTEP; rep++)
         if (pid >= 0 && leafA < 0 && !needPop) {
             const PairF *pp = sc.pairs + h;
             const float4 q0 = ldg4(&pp->q0), q1 = ldg4(&pp->q1), q2 = ldg4(&pp->q2), q3 = ldg4(&pp->q3);
-            if (COUNT) local[0] += 2;
+            local[0] += 2;
             const int metaL = __float_as_int(q3.x), metaR = __float_as_int(q3.y);
             float eL, eR;
             const bool hitL = box_f(r, q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, best_t, eL);
@@ -266,10 +267,10 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
         const unsigned lp = __ballot_sync(FULL, pid >= 0 && leafA >= 0);
         if (lp) {
             const unsigned nd = ~idle_now & ~lp;
-            if (__popc(lp) >= LEAF_T || nd == 0u) {
+            if (__popc(lp) >= TRACE4_LEAF_T || nd == 0u) {
                 if (pid >= 0 && leafA >= 0) {
-                    bool found = leaf_f3<COUNT, BIG>(sc, r, leafA, best_t, best_slot, local);
-                    if (leafB >= 0 && !(ANY && found) && eB <= best_t) found |= leaf_f3<COUNT, BIG>(sc, r, leafB, best_t, best_slot, local);
+                    bool found = leaf_f3<true, BIG>(sc, r, leafA, best_t, best_slot, local);
+                    if (leafB >= 0 && !(ANY && found) && eB <= best_t) found |= leaf_f3<true, BIG>(sc, r, leafB, best_t, best_slot, local);
                     leafA = leafB = -1;
                     if (ANY && found) finished = true;
                 }
@@ -295,173 +296,13 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
             pid = -1;
         }
     }
-    if (COUNT) { for (int k = 0; k < 3; k++) if (local[k]) atomicAdd(&ctr->v[ANY ? 1 : 0][k], local[k]); }
+    for (int k = 0; k < 3; k++) if (local[k]) atomicAdd(&ctr->v[ANY ? 1 : 0][k], local[k]);
 }
 
-
-// ---------------------------------------------------------------- two levels per step (QuadF)
-// Same persistent loop as k_f_trace4 (refill -> node step(s) -> leaf vote -> pop) but every node
-// step fetches ONE 128 B record with the four grandchildren boxes of an even-depth node, so a ray
-// makes half as many dependent steps and the loop skeleton is paid half as often.
-//   * the (<= 4) hits are ordered with a 5-comparator integer min/max network on keys
-//     (entry-distance bits & ~7) | leaf << 2 | slot  (entry >= tMin > 0, so integer order == float order);
-//   * nearest hit interior -> descend; nearest (and second nearest) hit leaves -> parked for the vote;
-//   * the other hits are deferred: their keys go to shared memory [level][3][thread], nearest on
-//     top, and a 2-bit-per-level count lives in a 64-bit trail register; the pop loop takes the
-//     deepest non-empty level, culls by the stored (rounded-down, conservative) entry distance and
-//     rebuilds the heap index from the ancestor: child = 4 * (h >> (depth - 2L)) + slot.
-// Quad levels.  PAR = 0: quad nodes sit at even depths 0,2,4,...  PAR = 1 (trees whose deepest leaves are at an odd
-// depth): the root is a 2-slot pseudo quad (its two children) and the real quads sit at odd depths 1,3,5,... so that
-// the bottom quads still hold four leaf grandchildren.  Level L <-> depth: PAR=0: 2L;  PAR=1: 0, 1, 3, 5, ...
-template <int PAR> __device__ __forceinline__ unsigned qlevel(unsigned depth) { return PAR ? ((depth + 1u) >> 1) : (depth >> 1); }
-template <int PAR> __device__ __forceinline__ unsigned qdepth(unsigned L) { return PAR ? (L ? 2u * L - 1u : 0u) : 2u * L; }
-template <int PAR> __device__ __forceinline__ size_t quad_index(unsigned h, unsigned depth)
-{
-    if (PAR) return depth ? (size_t)(h + 1u - ((4u << (depth - 1u)) + 2u) / 3u) : (size_t)0;
-    return (size_t)(h - ((2u << depth) + 1u) / 3u);
-}
-// heap index / depth of the child in slot `id` of quad node (h, depth)
-template <int PAR> __device__ __forceinline__ void quad_child(unsigned &h, unsigned &depth, unsigned id)
-{
-    if (PAR && depth == 0u) { h = 2u * h + id; depth = 1u; }
-    else { h = 4u * h + id; depth += 2u; }
-}
-
-template <bool ANY, bool BIG, int PAR, int REFILL_T, int LEAF_T, int NSTEP>
-__global__ void __launch_bounds__(FAST_BLOCK) k_f_trace5(SceneF sc, WaveF w, int bounce)
-{
-    extern __shared__ unsigned s_pend[];            // [qlevels][3][FAST_BLOCK]
-    unsigned *my_pend = s_pend + threadIdx.x;
-    const unsigned FULL = 0xffffffffu;
-    const unsigned lane = threadIdx.x & 31u;
-    const int n = ANY ? w.counts[CNT_SH(bounce)] : w.counts[bounce];
-    const float4 *ro = ANY ? w.sh_o : w.ray_o[bounce & 1], *rd = ANY ? w.sh_d : w.ray_d[bounce & 1];
-    int *cursor = &w.counts[ANY ? CUR_SH(bounce) : CUR_EXT(bounce)];
-
-    int pid = -1;
-    RayF r;
-    float best_t = 0.f; int best_slot = -1;
-    unsigned h = 1u, depth = 0u;                    // current quad node (1-based heap index, even depth)
-    unsigned long long trail = 0ull;                // 2 bits per quad level: deferred hits of that level's node
-    bool needPop = false;
-    int leafA = -1, leafB = -1; float eB = 0.f;
-    bool exhausted = false;
-    unsigned iters = 0u;
-
-    for (;;) {
-        const unsigned idle = __ballot_sync(FULL, pid < 0);
-        unsigned idle_now = idle;
-        if (++iters > (1u << 22)) { if (lane == 0) atomicAdd(&w.counts[MFX_COUNTS_LEN - 1], 1); break; }   // watchdog
-        if (!exhausted && __popc(idle) >= REFILL_T) {
-            const int nidle = __popc(idle);
-            int base = 0;
-            if (lane == 0) base = atomicAdd(cursor, nidle);
-            base = __shfl_sync(FULL, base, 0);
-            if (base + nidle >= n) exhausted = true;
-            if (pid < 0) {
-                const int idx = base + __popc(idle & ((1u << lane) - 1u));
-                if (idx < n) {
-                    pid = idx;                                          // the ray lives at its queue position
-                    const float4 o = ro[pid];
-                    const float4 d = rd[pid];
-                    r = make_ray_fast(f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), w.tmin, __float_as_int(o.w));
-                    best_t = ANY ? d.w - 1e-6f : w.tmax;                // shadow: dist - 1e-6 (Integrators.fs:44); closest: tMax (:108)
-                    // no root-box test: the root quad's four boxes lie inside it, a ray that misses the scene simply
-                    // finds no hit slot in its first node step and pops an empty trail (one-leaf trees never get here)
-                    best_slot = -1; trail = 0ull; leafA = leafB = -1; h = 1u; depth = 0u; needPop = false;
-                }
-            }
-            idle_now = __ballot_sync(FULL, pid < 0);
-        }
-        if (idle_now == FULL) { if (exhausted) break; continue; }
-
-#pragma unroll
-        for (int rep = 0; rep < NSTEP; rep++)
-        if (pid >= 0 && leafA < 0 && !needPop) {
-            const QuadF *qp = sc.quads + quad_index<PAR>(h, depth);
-            const float4 lox = ldg4(&qp->lox), hix = ldg4(&qp->hix), loy = ldg4(&qp->loy), hiy = ldg4(&qp->hiy);
-            const float4 loz = ldg4(&qp->loz), hiz = ldg4(&qp->hiz), m4 = ldg4(&qp->meta);
-            unsigned key[4];
-#define QUAD_SLOT(S, C)                                                                                              \
-            {                                                                                                        \
-                const float x0 = fmaf(lox.C, r.idir.x, -r.ood.x), x1 = fmaf(hix.C, r.idir.x, -r.ood.x);              \
-                const float y0 = fmaf(loy.C, r.idir.y, -r.ood.y), y1 = fmaf(hiy.C, r.idir.y, -r.ood.y);              \
-                const float z0 = fmaf(loz.C, r.idir.z, -r.ood.z), z1 = fmaf(hiz.C, r.idir.z, -r.ood.z);              \
-                const float tn = fmaxf(fmaxf(fminf(x0, x1), fminf(y0, y1)), fmaxf(fminf(z0, z1), r.tmin));           \
-                const float tf = fminf(fminf(fmaxf(x0, x1), fmaxf(y0, y1)), fminf(fmaxf(z0, z1), best_t));           \
-                const int mt = __float_as_int(m4.C);                                                                 \
-                key[S] = (tn <= tf && mt != -2) ? ((__float_as_uint(tn) & ~7u) | (mt >= 0 ? 4u : 0u) | (unsigned)S) : KEY_INF; \
-            }
-            QUAD_SLOT(0, x) QUAD_SLOT(1, y) QUAD_SLOT(2, z) QUAD_SLOT(3, w)
-#undef QUAD_SLOT
-            // sorting network (0,1)(2,3)(0,2)(1,3)(1,2)
-            unsigned a0 = umin_(key[0], key[1]), a1 = umax_(key[0], key[1]);
-            unsigned a2 = umin_(key[2], key[3]), a3 = umax_(key[2], key[3]);
-            const unsigned k0 = umin_(a0, a2), t2 = umax_(a0, a2);
-            const unsigned t1 = umin_(a1, a3), k3 = umax_(a1, a3);
-            const unsigned k1 = umin_(t1, t2), k2 = umax_(t1, t2);
-            const bool any0 = k0 != KEY_INF;
-            const bool leaf0 = any0 && (k0 & 4u), leaf1 = leaf0 && (k1 != KEY_INF) && (k1 & 4u);
-            leafA = leaf0 ? pick4(m4, k0 & 3u) : -1;
-            leafB = leaf1 ? pick4(m4, k1 & 3u) : -1;
-            eB = __uint_as_float(k1 & ~7u);
-            // deferred hits: everything behind the one(s) consumed now, nearest on top of the level's column
-            const unsigned p0 = leaf1 ? k2 : k1, p1 = leaf1 ? k3 : k2, p2 = leaf1 ? KEY_INF : k3;
-            const unsigned m = (p0 != KEY_INF ? 1u : 0u) + (p1 != KEY_INF ? 1u : 0u) + (p2 != KEY_INF ? 1u : 0u);
-            const unsigned L = qlevel<PAR>(depth);
-            unsigned *col = my_pend + (size_t)L * 3u * FAST_BLOCK;
-            if (m >= 1u) col[(m - 1u) * FAST_BLOCK] = p0;
-            if (m >= 2u) col[(m - 2u) * FAST_BLOCK] = p1;
-            if (m >= 3u) col[0] = p2;
-            trail |= (unsigned long long)m << (2u * L);
-            const bool descend = any0 && !leaf0;
-            needPop = !descend;
-            if (descend) quad_child<PAR>(h, depth, k0 & 3u);
-        }
-        bool finished = false;
-        const unsigned lp = __ballot_sync(FULL, pid >= 0 && leafA >= 0);
-        if (lp) {
-            const unsigned nd = ~idle_now & ~lp;
-            if (__popc(lp) >= LEAF_T || nd == 0u) {
-                if (pid >= 0 && leafA >= 0) {
-                    bool found = leaf_f3<false, BIG>(sc, r, leafA, best_t, best_slot, nullptr);
-                    if (leafB >= 0 && !(ANY && found) && eB <= best_t) found |= leaf_f3<false, BIG>(sc, r, leafB, best_t, best_slot, nullptr);
-                    leafA = leafB = -1;
-                    if (ANY && found) finished = true;
-                }
-            }
-        }
-        if (pid >= 0 && needPop && leafA < 0 && !finished) {
-            for (;;) {
-                if (trail == 0ull) { finished = true; break; }
-                const unsigned L = (63u - (unsigned)__clzll((long long)trail)) >> 1;
-                const unsigned cnt = (unsigned)(trail >> (2u * L)) & 3u;
-                trail -= 1ull << (2u * L);
-                const unsigned wv = my_pend[((size_t)L * 3u + (cnt - 1u)) * FAST_BLOCK];
-                if (ANY || __uint_as_float(wv & ~7u) <= best_t) {
-                    const unsigned dL = qdepth<PAR>(L);
-                    const unsigned Q = h >> (depth - dL);                // ancestor (or self) at quad level L
-                    h = Q; depth = dL;
-                    if (!(wv & 4u)) { quad_child<PAR>(h, depth, wv & 3u); needPop = false; }
-                    else {                                               // a deferred leaf: its meta sits in Q's record
-                        const float4 m4 = ldg4(&sc.quads[quad_index<PAR>(Q, dL)].meta);
-                        leafA = pick4(m4, wv & 3u); leafB = -1;
-                    }
-                    break;
-                }
-            }
-        }
-        if (finished) {
-            if (!ANY) w.hit[pid] = make_float2(best_t, __int_as_float(best_slot));
-            else if (best_slot < 0) { const float4 c = w.sh_c[pid]; float4 *ap = w.rad + __float_as_int(c.w); float4 a = *ap; a.x += c.x; a.y += c.y; a.z += c.z; *ap = a; }
-            pid = -1;
-        }
-    }
-}
 
 // ---------------------------------------------------------------- own tree: SAH, four children per record, child links
-// Same warp organisation as k_f_trace5 (ray replacement, two node steps per iteration, vote-postponed
-// leaves, sorted 4-wide node step) over the library's own binned-SAH tree (SceneF.own_tree, built by
+// Same warp organisation as k_f_trace4 (ray replacement, two node steps per iteration, vote-postponed
+// leaves), with a sorted 4-wide node step over the library's own binned-SAH tree (SceneF.own_tree, built by
 // flatten_fast_own in mfx_host.cpp).  The tree is not heap-shaped, so the deferred hits go to a real stack:
 // 8-byte entries (sort key, record that holds the child) in shared memory [entry][thread]; trees deeper than the
 // shared-memory budget overflow into a per-thread global column.  A pop re-reads the child link (one 4-byte load
@@ -479,12 +320,11 @@ struct SkyCtx {
 template <bool DIRECT>
 __device__ bool sky_scatter_f(const SkyCtx &c, int k, int pid, int fs, float t, F3 o, F3 d, float4 &thr, float4 &st_o, float4 &st_d);
 
-// CMP: the 64-byte records (QuadC) -- two sectors per node step instead of four.  A plane's distance is
-// (o + q*s - ray.o) / d = q*S + C with S = s/d, C = (o - ray.o)/d; the byte q becomes a float by being dropped into the
-// mantissa of 2^23 (one PRMT, which also picks the near or the far word by the octant and the child's byte), and the
-// 2^23 goes into the constant: t = (2^23 + q)*S + (C - 2^23*S), one fma.  The constant is rounded at the magnitude of
-// 2^23*S, i.e. to within half a step: the builder moved every plane outward by that much (compress_quads).
-template <bool ANY, bool BIG, int REFILL_T, int LEAF_T, int NSTEP, int NLEAF, int MINB, bool COUNT, bool CMP = false, bool TAIL = false>
+// Refill batches of 16 lanes, a leaf vote of 10 lanes, two node steps per iteration and one parked leaf per lane (the
+// second nearest hit goes to the stack like any other) measured best in round 2 (profiles/); refill batches of 20 / 24 /
+// 28 / 32 lanes (more sector sharing near the root, more idle lanes) measured -3 / -10 / -18 / -30 % on C2.
+constexpr int TRACE6_REFILL_T = 16, TRACE6_LEAF_T = 10, TRACE6_NSTEP = 2;
+template <bool ANY, bool BIG, int MINB, bool COUNT, bool TAIL = false>
 __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF w, int bounce, TravCounters *ctr, SkyCtx sky)
 {
     extern __shared__ uint2 s_stack[];              // [stack_smem][FAST_BLOCK]
@@ -504,7 +344,7 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
     float best_t = 0.f; int best_slot = -1;
     int node = 0, sp = 0;                           // current record, stack height
     bool needPop = false;
-    int leafA = -1, leafB = -1; float eB = 0.f;
+    int leafA = -1;
     bool exhausted = false;
     unsigned iters = 0u;
     unsigned long long local[3] = { 0ull, 0ull, 0ull };   // COUNT: 128 B records fetched, triangle tests, sphere tests
@@ -515,7 +355,7 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
         const unsigned idle = __ballot_sync(FULL, pid < 0);
         unsigned idle_now = idle;
         if (++iters > (TAIL ? (1u << 26) : (1u << 22))) { if (lane == 0) atomicAdd(&w.counts[MFX_COUNTS_LEN - 1], 1); break; }   // watchdog
-        if (!exhausted && __popc(idle) >= REFILL_T) {
+        if (!exhausted && __popc(idle) >= TRACE6_REFILL_T) {
             const int nidle = __popc(idle);
             int base = 0;
             if (lane == 0) base = atomicAdd(cursor, nidle);
@@ -529,12 +369,8 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
                     if (!cam0) o = ro[pid];
                     const float4 d = rd[pid];
                     r = make_ray_fast(f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), w.tmin, __float_as_int(o.w));
-                    if (CMP) {      // 2^23 * step / d must stay finite
-                        r.idir = f3(fminf(fmaxf(r.idir.x, -1e24f), 1e24f), fminf(fmaxf(r.idir.y, -1e24f), 1e24f), fminf(fmaxf(r.idir.z, -1e24f), 1e24f));
-                        r.ood = f3(r.o.x * r.idir.x, r.o.y * r.idir.y, r.o.z * r.idir.z);
-                    }
                     best_t = ANY ? d.w - 1e-6f : w.tmax;                // shadow: dist - 1e-6 (Integrators.fs:44); closest: tMax (:108)
-                    best_slot = -1; sp = 0; leafA = leafB = -1; node = 0; needPop = false;
+                    best_slot = -1; sp = 0; leafA = -1; node = 0; needPop = false;
                     if (TAIL) { path = __float_as_int(d.w); bnc = bounce; thr = w.thr[bounce & 1][pid]; }
                 }
             }
@@ -543,36 +379,12 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
         if (idle_now == FULL) { if (exhausted) break; continue; }
 
 #pragma unroll
-        for (int rep = 0; rep < NSTEP; rep++)
+        for (int rep = 0; rep < TRACE6_NSTEP; rep++)
         if (pid >= 0 && leafA < 0 && !needPop) {
             if (COUNT) local[0]++;
+            const QuadF *qp = sc.quads + node;
             float4 lox, hix, loy, hiy, loz, hiz, m4, pad4;
             unsigned key[4];
-            if (CMP) {
-                const float4 *qc = reinterpret_cast<const float4 *>(sc.cquads + node);
-                ldg8(qc, lox, hix); ldg8(qc + 2, loy, m4);                      // (o, sx | sy, sz, lox, loy) (loz, hix, hiy, hiz | meta)
-                const float Sx = lox.w * r.idir.x, Sy = hix.x * r.idir.y, Sz = hix.y * r.idir.z;
-                const float Cx = fmaf(-8388608.f, Sx, fmaf(lox.x, r.idir.x, -r.ood.x));
-                const float Cy = fmaf(-8388608.f, Sy, fmaf(lox.y, r.idir.y, -r.ood.y));
-                const float Cz = fmaf(-8388608.f, Sz, fmaf(lox.z, r.idir.z, -r.ood.z));
-                const bool px = r.idir.x >= 0.f, py = r.idir.y >= 0.f, pz = r.idir.z >= 0.f;
-                const unsigned wlx = __float_as_uint(hix.z), wly = __float_as_uint(hix.w), wlz = __float_as_uint(loy.x);
-                const unsigned whx = __float_as_uint(loy.y), why = __float_as_uint(loy.z), whz = __float_as_uint(loy.w);
-                const unsigned nx = px ? wlx : whx, fx = px ? whx : wlx, ny = py ? wly : why, fy = py ? why : wly, nz = pz ? wlz : whz, fz = pz ? whz : wlz;
-#define CQ_PLANE(W, S_, SC, CC) fmaf(__uint_as_float(__byte_perm((W), 0x4B000000u, 0x7440u | (unsigned)(S_))), (SC), (CC))
-#define CQUAD_SLOT(S_, C)                                                                                            \
-                {                                                                                                    \
-                    const float tn = fmaxf(fmaxf(CQ_PLANE(nx, S_, Sx, Cx), CQ_PLANE(ny, S_, Sy, Cy)), fmaxf(CQ_PLANE(nz, S_, Sz, Cz), r.tmin));   \
-                    const float tf = fminf(fminf(CQ_PLANE(fx, S_, Sx, Cx), CQ_PLANE(fy, S_, Sy, Cy)), fminf(CQ_PLANE(fz, S_, Sz, Cz), best_t));   \
-                    const int mt = __float_as_int(m4.C);                                                             \
-                    const unsigned ord = ANY ? (0x7f7ffff8u - (__float_as_uint(tn) & ~7u)) : (__float_as_uint(tn) & ~7u);   \
-                    key[S_] = (tn <= tf && mt != MFX_QUAD_EMPTY) ? (ord | (mt >= 0 ? 4u : 0u) | (unsigned)S_) : KEY_INF;   \
-                }
-                CQUAD_SLOT(0, x) CQUAD_SLOT(1, y) CQUAD_SLOT(2, z) CQUAD_SLOT(3, w)
-#undef CQUAD_SLOT
-#undef CQ_PLANE
-            } else {
-            const QuadF *qp = sc.quads + node;
             ldg8(&qp->lox, lox, hix); ldg8(&qp->loy, loy, hiy); ldg8(&qp->loz, loz, hiz); ldg8(&qp->meta, m4, pad4);
 #define QUAD_SLOT(S_, C)                                                                                             \
             {                                                                                                        \
@@ -591,7 +403,6 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
             }
             QUAD_SLOT(0, x) QUAD_SLOT(1, y) QUAD_SLOT(2, z) QUAD_SLOT(3, w)
 #undef QUAD_SLOT
-            }
             // sorting network (0,1)(2,3)(0,2)(1,3)(1,2)
             unsigned a0 = umin_(key[0], key[1]), a1 = umax_(key[0], key[1]);
             unsigned a2 = umin_(key[2], key[3]), a3 = umax_(key[2], key[3]);
@@ -599,21 +410,19 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
             const unsigned t1 = umin_(a1, a3), k3 = umax_(a1, a3);
             const unsigned k1 = umin_(t1, t2), k2 = umax_(t1, t2);
             const bool any0 = k0 != KEY_INF;
-            const bool leaf0 = any0 && (k0 & 4u), leaf1 = (NLEAF > 1) && leaf0 && (k1 != KEY_INF) && (k1 & 4u);
+            const bool leaf0 = any0 && (k0 & 4u);
             const int c0 = pick4(m4, k0 & 3u);
             leafA = leaf0 ? c0 : -1;
-            if (NLEAF > 1) { leafB = leaf1 ? pick4(m4, k1 & 3u) : -1; eB = __uint_as_float(k1 & ~7u); }
-            // deferred hits: everything behind the one(s) consumed now, nearest on top of the stack
-            const unsigned p0 = leaf1 ? k2 : k1, p1 = leaf1 ? k3 : k2, p2 = leaf1 ? KEY_INF : k3;
-            const int m = (p0 != KEY_INF ? 1 : 0) + (p1 != KEY_INF ? 1 : 0) + (p2 != KEY_INF ? 1 : 0);
+            // deferred hits: everything behind the one consumed now, nearest on top of the stack
+            const int m = (k1 != KEY_INF ? 1 : 0) + (k2 != KEY_INF ? 1 : 0) + (k3 != KEY_INF ? 1 : 0);
 #define STACK_PUT(I, K)                                                                                              \
             { const int i_ = (I); const uint2 v_ = make_uint2((K), (unsigned)node);                                  \
               DBG_CHECK(i_ >= 0 && i_ < 3 * sc.own_depth, w.counts);                                                  \
               DBG_CHECK(i_ < S || blockIdx.x * FAST_BLOCK + threadIdx.x < (unsigned)sc.spill_threads, w.counts);       \
               if (i_ < S) my_stack[(size_t)i_ * FAST_BLOCK] = v_; else my_spill[(size_t)(i_ - S) * spill_stride] = v_; }
-            if (m >= 1) STACK_PUT(sp + m - 1, p0)
-            if (m >= 2) STACK_PUT(sp + m - 2, p1)
-            if (m >= 3) STACK_PUT(sp, p2)
+            if (m >= 1) STACK_PUT(sp + m - 1, k1)
+            if (m >= 2) STACK_PUT(sp + m - 2, k2)
+            if (m >= 3) STACK_PUT(sp, k3)
 #undef STACK_PUT
             sp += m;
             const bool descend = any0 && !leaf0;
@@ -626,12 +435,10 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
         const unsigned lp = __ballot_sync(FULL, pid >= 0 && leafA >= 0);
         if (lp) {
             const unsigned nd = ~idle_now & ~lp;
-            if (__popc(lp) >= LEAF_T || nd == 0u) {
+            if (__popc(lp) >= TRACE6_LEAF_T || nd == 0u) {
                 if (pid >= 0 && leafA >= 0) {
-                    bool found = leaf_f3<COUNT, BIG>(sc, r, leafA, best_t, best_slot, local);
-                    // (a shadow query's keys are not distances and its best_t never shrinks: no cull for it)
-                    if (NLEAF > 1 && leafB >= 0 && !(ANY && found) && (ANY || eB <= best_t)) found |= leaf_f3<COUNT, BIG>(sc, r, leafB, best_t, best_slot, local);
-                    leafA = leafB = -1;
+                    const bool found = leaf_f3<COUNT, BIG>(sc, r, leafA, best_t, best_slot, local);
+                    leafA = -1;
                     if (ANY && found) finished = true;
                 }
             }
@@ -642,8 +449,8 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
                 --sp;
                 const uint2 e = (sp < S) ? my_stack[(size_t)sp * FAST_BLOCK] : my_spill[(size_t)(sp - S) * spill_stride];
                 if (ANY || __uint_as_float(e.x & ~7u) <= best_t) {
-                    const int link = CMP ? __ldg(&sc.cquads[e.y].meta[e.x & 3u]) : __ldg(reinterpret_cast<const int *>(&sc.quads[e.y].meta) + (e.x & 3u));
-                    if (e.x & 4u) { leafA = link; leafB = -1; }
+                    const int link = __ldg(reinterpret_cast<const int *>(&sc.quads[e.y].meta) + (e.x & 3u));
+                    if (e.x & 4u) leafA = link;
                     else { node = ~link; needPop = false; }
                     DBG_CHECK(e.y < (unsigned)sc.n_quads && ((e.x & 4u) ? (link >= 0 && (link >> 3) + (link & 7) <= sc.n_slots) : (unsigned)~link < (unsigned)sc.n_quads), w.counts);
                     break;
@@ -662,11 +469,7 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
                 float4 so, sd;
                 if (sky_scatter_f<true>(sky, bnc, path, best_slot, best_t, r.o, r.d, thr, so, sd)) {
                     r = make_ray_fast(f3(so.x, so.y, so.z), f3(sd.x, sd.y, sd.z), w.tmin, __float_as_int(so.w));
-                    if (CMP) {
-                        r.idir = f3(fminf(fmaxf(r.idir.x, -1e24f), 1e24f), fminf(fmaxf(r.idir.y, -1e24f), 1e24f), fminf(fmaxf(r.idir.z, -1e24f), 1e24f));
-                        r.ood = f3(r.o.x * r.idir.x, r.o.y * r.idir.y, r.o.z * r.idir.z);
-                    }
-                    best_t = w.tmax; best_slot = -1; sp = 0; leafA = leafB = -1; node = 0; needPop = false;
+                    best_t = w.tmax; best_slot = -1; sp = 0; leafA = -1; node = 0; needPop = false;
                     bnc++; traced_on++; again = true;
                 }
             }
@@ -1078,7 +881,7 @@ __global__ void __launch_bounds__(256) k_f_resolve(SceneF sc, WaveF w, TileMap t
 }
 
 // Finer seams (Bvh.Hit, GetRay + Hit) routed through the PRODUCTION traversal kernel: rays are written
-// into the wave's queues, traced by k_f_trace5 / k_f_trace4, and read back.
+// into the wave's queues, traced by k_f_trace6, and read back.
 __global__ void __launch_bounds__(256) k_f_seam_setup(SceneF sc, WaveF w, int n, const double *o, const double *d, const double *uv,
                                                       long long first, float tmax, int any_hit)
 {
@@ -1212,98 +1015,46 @@ void mfx_f_raygen(const LaunchCfg &c, const SceneF &sc, const WaveF &w, TileMap 
 {
     k_f_raygen<<<persistent_blocks(k_f_raygen, 256, c.blocks), 256, 0, c.stream>>>(sc, w, tm, pix0, npix, s0, S, seed);
 }
-template <bool ANY, bool BIG, int RT, int LT, int NS>
-static void launch_trace4b(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr)
-{
-    const size_t smem = ANY ? 0 : (size_t)sc.levels * FAST_BLOCK * sizeof(float);
-    if (ctr) k_f_trace4<ANY, true, BIG, RT, LT, NS><<<persistent_blocks(k_f_trace4<ANY, true, BIG, RT, LT, NS>, FAST_BLOCK, c.blocks, smem), FAST_BLOCK, smem, c.stream>>>(sc, w, bounce, ctr);
-    else k_f_trace4<ANY, false, BIG, RT, LT, NS><<<persistent_blocks(k_f_trace4<ANY, false, BIG, RT, LT, NS>, FAST_BLOCK, c.blocks, smem), FAST_BLOCK, smem, c.stream>>>(sc, w, bounce, ctr);
-}
-// scenes without a big (f64) sphere get the kernel compiled without that branch (48 instead of 64+ registers)
-template <bool ANY, int RT, int LT, int NS = 1>
+template <bool ANY, bool BIG>
 static void launch_trace4(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr)
 {
-    if (sc.has_big_sphere) launch_trace4b<ANY, true, RT, LT, NS>(c, sc, w, bounce, ctr);
-    else launch_trace4b<ANY, false, RT, LT, NS>(c, sc, w, bounce, ctr);
-}
-template <bool ANY, bool BIG, int RT, int LT, int NS>
-static void launch_trace5b(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce)
-{
-    const size_t smem = (size_t)sc.qlevels * 3 * FAST_BLOCK * sizeof(unsigned);
-    if (sc.qpar) k_f_trace5<ANY, BIG, 1, RT, LT, NS><<<persistent_blocks(k_f_trace5<ANY, BIG, 1, RT, LT, NS>, FAST_BLOCK, c.blocks, smem), FAST_BLOCK, smem, c.stream>>>(sc, w, bounce);
-    else k_f_trace5<ANY, BIG, 0, RT, LT, NS><<<persistent_blocks(k_f_trace5<ANY, BIG, 0, RT, LT, NS>, FAST_BLOCK, c.blocks, smem), FAST_BLOCK, smem, c.stream>>>(sc, w, bounce);
-}
-template <bool ANY, int RT, int LT, int NS>
-static void launch_trace5(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr)
-{
-    // instrumented (counting) runs and one-leaf trees use the binary kernel: the algorithmic record
-    // counts of the roofline are defined on the reference's binary tree
-    if (ctr || sc.root_meta >= 0) { launch_trace4<ANY, 12, 16, 2>(c, sc, w, bounce, ctr); return; }
-    if (sc.has_big_sphere) launch_trace5b<ANY, true, RT, LT, NS>(c, sc, w, bounce);
-    else launch_trace5b<ANY, false, RT, LT, NS>(c, sc, w, bounce);
+    const size_t smem = ANY ? 0 : (size_t)sc.levels * FAST_BLOCK * sizeof(float);
+    k_f_trace4<ANY, BIG><<<persistent_blocks(k_f_trace4<ANY, BIG>, FAST_BLOCK, c.blocks, smem), FAST_BLOCK, smem, c.stream>>>(sc, w, bounce, ctr);
 }
 static_assert(MFX_STACK_SMEM_MAX * FAST_BLOCK * sizeof(uint2) <= 48 * 1024, "the own-tree stack must launch without a shared-memory opt-in");
-template <bool ANY, bool BIG, int RT, int LT, int NS, int NL, int MB, bool CNT = false, bool CMP = false, bool TAIL = false>
-static void launch_trace6b(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr = nullptr, const SkyCtx &sky = SkyCtx{})
+template <bool ANY, bool BIG, int MB, bool CNT, bool TAIL = false>
+static void launch_trace6(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr, const SkyCtx &sky = SkyCtx{})
 {
     const size_t smem = (size_t)sc.stack_smem * FAST_BLOCK * sizeof(uint2);
     // the spill columns were sized for spill_threads: never launch more threads than that
-    int blocks = persistent_blocks(k_f_trace6<ANY, BIG, RT, LT, NS, NL, MB, CNT, CMP, TAIL>, FAST_BLOCK, c.blocks, smem);
+    int blocks = persistent_blocks(k_f_trace6<ANY, BIG, MB, CNT, TAIL>, FAST_BLOCK, c.blocks, smem);
     if (sc.stack_spill && blocks * FAST_BLOCK > sc.spill_threads) blocks = sc.spill_threads / FAST_BLOCK;
     if (c.max_items > 0) blocks = std::max(1, std::min(blocks, (c.max_items + FAST_BLOCK - 1) / FAST_BLOCK));
-    k_f_trace6<ANY, BIG, RT, LT, NS, NL, MB, CNT, CMP, TAIL><<<blocks, FAST_BLOCK, smem, c.stream>>>(sc, w, bounce, ctr, sky);
+    k_f_trace6<ANY, BIG, MB, CNT, TAIL><<<blocks, FAST_BLOCK, smem, c.stream>>>(sc, w, bounce, ctr, sky);
 }
-template <bool ANY, int RT, int LT, int NS, int NL = 2, int MB = 1, bool CMP = false>
-static void launch_trace6(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce)
-{
-    if (sc.has_big_sphere) launch_trace6b<ANY, true, RT, LT, NS, NL, MB, false, CMP>(c, sc, w, bounce);
-    else launch_trace6b<ANY, false, RT, LT, NS, NL, MB, false, CMP>(c, sc, w, bounce);
-}
+// The layout decides the kernel: the reference tree is passed for the instrumented counting runs (the algorithmic record
+// counts of the roofline are defined on the reference's binary tree) and takes k_f_trace4; the library's SAH tree takes
+// k_f_trace6, instrumented when counters were asked for (MFX_SAMPLE_COUNT_OWN_TREE).  Scenes without a big (f64) sphere
+// get the kernels compiled without that branch.
 template <bool ANY>
-static void launch_trace_variant(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr)
+static void launch_trace(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr)
 {
-    if (sc.own_tree) {          // the library's SAH tree (default); the host passes the reference-tree layout for the others
-        if (ctr) {              // MFX_SAMPLE_COUNT_OWN_TREE: the shipped configuration, instrumented
-            if (c.variant == 7 || c.variant == 71) {
-                if (sc.has_big_sphere) launch_trace6b<ANY, true, 16, 10, 2, 1, 1, true, true>(c, sc, w, bounce, ctr);
-                else launch_trace6b<ANY, false, 16, 10, 2, 1, 1, true, true>(c, sc, w, bounce, ctr);
-                return;
-            }
-            if (sc.has_big_sphere) launch_trace6b<ANY, true, 16, 10, 2, 1, 1, true>(c, sc, w, bounce, ctr);
-            else launch_trace6b<ANY, false, 16, 10, 2, 1, 1, true>(c, sc, w, bounce, ctr);
-            return;
-        }
-        switch (c.variant) {
-        case 7: launch_trace6<ANY, 16, 10, 2, 1, 8, true>(c, sc, w, bounce); break;      // 64-byte records (QuadC)
-        case 71: launch_trace6<ANY, 16, 10, 2, 1, 6, true>(c, sc, w, bounce); break;    // tuning knobs kept for A/B runs (tools/ab_env.py MFX_TRACE_VARIANT ...); the default is the measured best (profiles/)
-        case 61: launch_trace6<ANY, 8, 12, 2, 2>(c, sc, w, bounce); break;      // two parked leaves
-        case 62: launch_trace6<ANY, 12, 16, 1, 2>(c, sc, w, bounce); break;     // one node step per iteration
-        case 65: launch_trace6<ANY, 8, 12, 2, 1>(c, sc, w, bounce); break;
-        case 84: launch_trace6<ANY, 12, 12, 2, 1>(c, sc, w, bounce); break;
-        case 85: launch_trace6<ANY, 16, 8, 2, 1>(c, sc, w, bounce); break;
-        // refill batches of 20 / 24 / 28 / 32 lanes (more sector sharing near the root, more idle lanes) measured -3 / -10 /
-        // -18 / -30 % on C2 in round 2: 16 stays
-        default: launch_trace6<ANY, 16, 10, 2, 1, 8>(c, sc, w, bounce); break;    // 8 blocks/SM: 64 registers
-        }
-        return;
-    }
-    switch (c.variant) {        // tuning knob (MFX_TRACE_VARIANT); the default comes from measurements (profiles/)
-    case 4: launch_trace4<ANY, 12, 16, 2>(c, sc, w, bounce, ctr); break;     // binary steps (one 64 B pair per fetch)
-    case 51: launch_trace5<ANY, 8, 12, 2>(c, sc, w, bounce, ctr); break;
-    case 52: launch_trace5<ANY, 12, 16, 1>(c, sc, w, bounce, ctr); break;
-    default: launch_trace5<ANY, 12, 16, 2>(c, sc, w, bounce, ctr); break;    // two levels per fetch (128 B quad)
-    }
+    const bool big = sc.has_big_sphere != 0;
+    if (!sc.own_tree) { if (big) launch_trace4<ANY, true>(c, sc, w, bounce, ctr); else launch_trace4<ANY, false>(c, sc, w, bounce, ctr); }
+    else if (ctr) { if (big) launch_trace6<ANY, true, 1, true>(c, sc, w, bounce, ctr); else launch_trace6<ANY, false, 1, true>(c, sc, w, bounce, ctr); }
+    else if (big) launch_trace6<ANY, true, 8, false>(c, sc, w, bounce, nullptr);        // 8 blocks/SM: 64 registers
+    else launch_trace6<ANY, false, 8, false>(c, sc, w, bounce, nullptr);
 }
 void mfx_f_extend(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr)
 {
-    launch_trace_variant<false>(c, sc, w, bounce, ctr);
+    launch_trace<false>(c, sc, w, bounce, ctr);
 }
 // MFX_SKY_TRACER: every path in the extend queue of `bounce` traced AND shaded to its end in one launch (k_f_trace6<TAIL>)
 void mfx_f_sky_tail(const LaunchCfg &c, const SceneF &sc, const WaveF &w, TileMap tm, int pix0, int npix, int s0, int bounce, uint64_t seed)
 {
     const SkyCtx sky{ sc.slots, sc.slot_nrm, sc.mats, sc.perlin_rf, sc.perlin_perm, tm, sc.width, pix0, npix, s0, (uint32_t)seed, (uint32_t)(seed >> 32) };
-    if (sc.has_big_sphere) launch_trace6b<false, true, 16, 10, 2, 1, 4, false, false, true>(c, sc, w, bounce, nullptr, sky);
-    else launch_trace6b<false, false, 16, 10, 2, 1, 4, false, false, true>(c, sc, w, bounce, nullptr, sky);
+    if (sc.has_big_sphere) launch_trace6<false, true, 4, false, true>(c, sc, w, bounce, nullptr, sky);
+    else launch_trace6<false, false, 4, false, true>(c, sc, w, bounce, nullptr, sky);
 }
 void mfx_f_shade(const LaunchCfg &c, const SceneF &sc, const WaveF &w, TileMap tm, int pix0, int npix, int s0, int bounce, uint64_t seed)
 {
@@ -1319,7 +1070,7 @@ void mfx_f_shade_sky(const LaunchCfg &c, const SceneF &sc, const WaveF &w, TileM
 }
 void mfx_f_shadow(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr)
 {
-    launch_trace_variant<true>(c, sc, w, bounce, ctr);
+    launch_trace<true>(c, sc, w, bounce, ctr);
 }
 void mfx_f_resolve(const LaunchCfg &c, const SceneF &sc, const WaveF &w, TileMap tm, int pix0, int npix, int S, double *pixsum)
 {

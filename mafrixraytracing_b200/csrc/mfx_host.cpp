@@ -659,8 +659,8 @@ static void make_fast_slots(const MfxPrim &p, int id, std::vector<SlotF> &slots,
     }
 }
 
-// Reference-tree layout (children pairs + heap-indexed quads): used by the instrumented counting runs (the roofline's
-// record counts are defined on the reference tree) and by the k_f_trace4 / k_f_trace5 variants.
+// Reference-tree layout (children pairs indexed by the heap index): used by the instrumented counting runs (k_f_trace4:
+// the roofline's record counts are defined on the reference tree) and by the exact shadow walk (k_h_shadow_x).
 static int flatten_fast_ref(MfxScene *s)
 {
     if (s->fr_ready) return MFX_OK;
@@ -707,77 +707,10 @@ static int flatten_fast_ref(MfxScene *s)
             if (ri) todo.push_back(2 * i + 2);
         }
     }
-    // quad records: two tree levels per fetch (QuadF in mfx_internal.h)
-    std::vector<QuadF> quads;
-    int qlevels = 0, qpar = 0;
-    if (root.count > MFX_LEAF_NODE_COUNT) {
-        // deepest leaf depth decides the parity so that the bottom quads hold four leaf grandchildren
-        {
-            unsigned maxh = 1;
-            for (size_t i = 0; i < s->nodes.size(); i++) if (s->nodes[i].count > 0) maxh = (unsigned)i + 1u;
-            unsigned D = 0; for (unsigned v = maxh; v > 1u; v >>= 1) D++;
-            qpar = (int)(D & 1u);
-        }
-        auto qindex = [&](unsigned h, unsigned depth) -> size_t {
-            if (qpar) return depth ? (size_t)(h + 1u - ((4u << (depth - 1u)) + 2u) / 3u) : (size_t)0;
-            return (size_t)(h - ((2u << depth) + 1u) / 3u);
-        };
-        auto qlevel = [&](unsigned depth) { return qpar ? (int)((depth + 1u) >> 1) : (int)(depth >> 1); };
-        struct QItem { unsigned h, depth; };
-        std::vector<QItem> todo{ { 1u, 0u } };
-        const float FAR = 1e30f;
-        while (!todo.empty()) {
-            const QItem it = todo.back(); todo.pop_back();
-            const size_t qi = qindex(it.h, it.depth);
-            if (qi >= quads.size()) {
-                QuadF z; memset(&z, 0, sizeof(z));
-                z.lox = z.hix = z.loy = z.hiy = z.loz = z.hiz = make_float4(FAR, FAR, FAR, FAR);
-                z.meta = make_float4(int_bits(-2), int_bits(-2), int_bits(-2), int_bits(-2));
-                quads.resize(qi + 1, z);
-            }
-            qlevels = std::max(qlevels, qlevel(it.depth) + 1);
-            float lo[3][4], hi[3][4]; int meta[4];
-            for (int sl = 0; sl < 4; sl++) { for (int a = 0; a < 3; a++) { lo[a][sl] = FAR; hi[a][sl] = FAR; } meta[sl] = -2; }
-            auto put = [&](int sl, const MfxBvhNode &nd, int m) {
-                for (int a = 0; a < 3; a++) { lo[a][sl] = round_down(nd.pmin[a]); hi[a][sl] = round_up(nd.pmax[a]); }
-                meta[sl] = m;
-            };
-            if (qpar && it.depth == 0u) {
-                // pseudo root: slots 0/1 are the root's own children (child heap index 2h + slot)
-                for (unsigned ci = 0; ci < 2; ci++) {
-                    const unsigned c = 2u * it.h + ci;
-                    const MfxBvhNode &C = s->nodes[c - 1];
-                    const bool interior = C.count > MFX_LEAF_NODE_COUNT;
-                    put((int)ci, C, interior ? -1 : leaf_meta(C));
-                    if (interior) todo.push_back({ c, 1u });
-                }
-            } else {
-                for (unsigned ci = 0; ci < 2; ci++) {
-                    const unsigned c = 2u * it.h + ci;                       // 1-based child
-                    const MfxBvhNode &C = s->nodes[c - 1];
-                    if (C.count <= MFX_LEAF_NODE_COUNT) { put(2 * ci, C, leaf_meta(C)); continue; }
-                    for (unsigned gi = 0; gi < 2; gi++) {
-                        const unsigned g = 2u * c + gi;                      // 1-based grandchild = 4h + 2ci + gi
-                        const MfxBvhNode &G = s->nodes[g - 1];
-                        const bool interior = G.count > MFX_LEAF_NODE_COUNT;
-                        put(2 * ci + gi, G, interior ? -1 : leaf_meta(G));
-                        if (interior) todo.push_back({ g, it.depth + 2u });
-                    }
-                }
-            }
-            QuadF &q = quads[qi];
-            q.lox = make_float4(lo[0][0], lo[0][1], lo[0][2], lo[0][3]); q.hix = make_float4(hi[0][0], hi[0][1], hi[0][2], hi[0][3]);
-            q.loy = make_float4(lo[1][0], lo[1][1], lo[1][2], lo[1][3]); q.hiy = make_float4(hi[1][0], hi[1][1], hi[1][2], hi[1][3]);
-            q.loz = make_float4(lo[2][0], lo[2][1], lo[2][2], lo[2][3]); q.hiz = make_float4(hi[2][0], hi[2][1], hi[2][2], hi[2][3]);
-            q.meta = make_float4(int_bits(meta[0]), int_bits(meta[1]), int_bits(meta[2]), int_bits(meta[3]));
-        }
-    }
-    PairF *dpairs; SlotF *dslots; float4 *dnrm; int *dref; QuadF *dquads;
-    MFX_TRY(upload(s, &dquads, quads));
+    PairF *dpairs; SlotF *dslots; float4 *dnrm; int *dref;
     MFX_TRY(upload(s, &dpairs, pairs)); MFX_TRY(upload(s, &dslots, slots)); MFX_TRY(upload(s, &dnrm, nrm));
     MFX_TRY(upload(s, &dref, ref));
-    s->fr_bytes = quads.size() * sizeof(QuadF) + pairs.size() * sizeof(PairF) + slots.size() * sizeof(SlotF) + nrm.size() * 16 + ref.size() * 4;
-    sf.quads = dquads; sf.qlevels = qlevels; sf.qpar = qpar; sf.n_quads = (int)quads.size();
+    s->fr_bytes = pairs.size() * sizeof(PairF) + slots.size() * sizeof(SlotF) + nrm.size() * 16 + ref.size() * 4;
     sf.pairs = dpairs; sf.slots = dslots; sf.slot_nrm = dnrm; sf.ref_id = dref; sf.slot_prim = nullptr;
     MFX_TRY(fill_fast_common(s, sf));
     sf.n_slots = (int)slots.size();
@@ -794,12 +727,11 @@ static int flatten_fast_ref(MfxScene *s)
 // key the cache; a handful of entries, bounded in bytes, least recently used goes first.
 struct OwnTreeHost {
     std::vector<QuadF> quads;
-    std::vector<QuadC> cquads;          // the same records on 8-bit grids (QuadC)
     std::vector<SlotF> slots;
     std::vector<float4> nrm;
     std::vector<int> slot_prim;         // own-tree fast slot -> primitive index, bit 30 = second triangle of a Rect
     int depth = 0, has_big = 0;
-    size_t bytes() const { return quads.size() * sizeof(QuadF) + cquads.size() * sizeof(QuadC) + slots.size() * sizeof(SlotF) + nrm.size() * 16 + slot_prim.size() * 4; }
+    size_t bytes() const { return quads.size() * sizeof(QuadF) + slots.size() * sizeof(SlotF) + nrm.size() * 16 + slot_prim.size() * 4; }
 };
 struct TreeKey {
     uint64_t h1, h2; size_t n; long max_leaf, trav, collapse;
@@ -935,22 +867,11 @@ static int flatten_fast(MfxScene *s)
 }
 
 // Which fast layout a call runs on: the own tree, unless the caller asked for traversal counters (defined on the
-// reference tree) or pinned one of the reference-tree kernels with MFX_TRACE_VARIANT (4, 5, 51, 52).
-static int fast_layout(MfxScene *s, bool counting, int variant, const SceneF **out)
+// reference tree).
+static int fast_layout(MfxScene *s, bool counting, const SceneF **out)
 {
-    const bool ref = counting || variant == 4 || variant == 5 || variant == 51 || variant == 52;
-    if (ref) { MFX_TRY(flatten_fast_ref(s)); *out = &s->sf_ref; }
+    if (counting) { MFX_TRY(flatten_fast_ref(s)); *out = &s->sf_ref; }
     else { MFX_TRY(flatten_fast(s)); *out = &s->sf; }
-    if (!ref && (variant == 7 || variant == 71) && !s->sf.cquads) {       // the 64-byte records: an experiment (DESIGN.md 7), built on demand
-        {
-            std::lock_guard<std::mutex> g(g_tree_mu);
-            if (s->own_host->cquads.empty()) mfx_compress_quads(s->own_host->quads, s->own_host->cquads);
-        }
-        QuadC *dc;
-        MFX_TRY(upload(s, &dc, s->own_host->cquads));
-        s->sf.cquads = dc;
-        s->f_bytes += s->own_host->cquads.size() * sizeof(QuadC);
-    }
     return MFX_OK;
 }
 
@@ -1317,9 +1238,8 @@ static int launch_sample(MfxScene *s, const MfxSampleParams *p, double *d_color_
     if (exact) { MFX_TRY(flatten_exact(s)); MFX_TRY(ensure_wave_exact(s)); }
     const bool count_ref = (p->flags & MFX_SAMPLE_COUNT_TRAVERSAL) != 0;
     const bool counting = count_ref || (p->flags & MFX_SAMPLE_COUNT_OWN_TREE) != 0;
-    const int variant = (int)env_long("MFX_TRACE_VARIANT", -1);
     const SceneF *sfp = nullptr;
-    if (!exact) MFX_TRY(fast_layout(s, count_ref, variant, &sfp));
+    if (!exact) MFX_TRY(fast_layout(s, count_ref, &sfp));
     MFX_TRY(ensure_frame_buffers(s));
     TileMap tm;
     MFX_TRY(get_tilemap(s, p->tile_size, p->rank, p->world, (p->flags & MFX_SAMPLE_STRIPES) != 0, &tm));
@@ -1345,7 +1265,7 @@ static int launch_sample(MfxScene *s, const MfxSampleParams *p, double *d_color_
     if (!exact) s->wf.cam_origin = (sfp->own_tree && !counting && !(sky && s->lens.lens_radius != 0.0)) ? 1 : 0;
     const size_t npx = (size_t)s->width * s->height;
     cudaStream_t st = s->stream;
-    LaunchCfg cfg{ s->sm_count, 128, st, variant, (p->flags & MFX_SAMPLE_REFERENCE_STREAM) ? 1 : 0, 0, (int)env_long("MFX_HYB_VARIANT", 0) };
+    LaunchCfg cfg{ s->sm_count, 128, st, (p->flags & MFX_SAMPLE_REFERENCE_STREAM) ? 1 : 0, 0 };
 
     CUDA_TRY(cudaMemsetAsync(s->d_pixsum, 0, 4 * npx * sizeof(double), st));
     CUDA_TRY(cudaMemsetAsync(job.d_totals, 0, 8 * sizeof(unsigned long long), st));
@@ -1774,17 +1694,17 @@ extern "C" int mfx_bvh_hit(MfxScene *s, int32_t precision, int32_t any_hit, int6
     if (!s || !origins || !dirs || !prim || !t) return fail(MFX_ERR_INVALID_ARGUMENT, "mfx_bvh_hit: null argument");
     if (n <= 0) return MFX_OK;
     MFX_TRY(bind_device(s->device));
-    LaunchCfg cfg{ s->sm_count, 128, s->stream, (int)env_long("MFX_TRACE_VARIANT", -1), 0, 0, (int)env_long("MFX_HYB_VARIANT", 0) };
+    LaunchCfg cfg{ s->sm_count, 128, s->stream, 0, 0 };
     if (precision == MFX_EXACT_F64) {
         MFX_TRY(flatten_exact(s));
         return with_ray_buffers(s, n, origins, 3, dirs, 3, prim, sub, t, [&](double *o, double *d, int *p, int *sb, double *tt) {
             mfx_x_bvh_hit(cfg, s->sx, any_hit, n, o, d, tmin, tmax, p, sb, tt);
         });
     } else if (precision == MFX_FAST_F32) {
-        const SceneF *sfp = nullptr;
-        MFX_TRY(fast_layout(s, false, cfg.variant, &sfp));
+        MFX_TRY(flatten_fast(s));
+        const SceneF *sfp = &s->sf;
         MFX_TRY(ensure_wave_fast(s, (size_t)n));
-        const bool hyb = !any_hit && sfp->own_tree && use_hybrid(0);
+        const bool hyb = !any_hit && use_hybrid(0);
         if (hyb) { MFX_TRY(flatten_hybrid(s)); MFX_TRY(ensure_wave_hybrid(s)); }
         return with_ray_buffers(s, n, origins, 3, dirs, 3, prim, sub, t, [&](double *o, double *d, int *p, int *sb, double *tt) {
             if (hyb) hybrid_seam(s, sfp, cfg, n, o, d, nullptr, tmin, tmax, p, sb, tt);
@@ -1800,17 +1720,17 @@ extern "C" int mfx_trace_primary(MfxScene *s, int32_t precision, int64_t n, cons
     if (!uv && n != (int64_t)s->width * s->height) return fail(MFX_ERR_INVALID_ARGUMENT, "uv == NULL needs n == width*height");
     if (n <= 0) return MFX_OK;
     MFX_TRY(bind_device(s->device));
-    LaunchCfg cfg{ s->sm_count, 128, s->stream, (int)env_long("MFX_TRACE_VARIANT", -1), 0, 0, (int)env_long("MFX_HYB_VARIANT", 0) };
+    LaunchCfg cfg{ s->sm_count, 128, s->stream, 0, 0 };
     if (precision == MFX_EXACT_F64) {
         MFX_TRY(flatten_exact(s));
         return with_ray_buffers(s, n, uv, 2, nullptr, 0, prim, nullptr, t, [&](double *u, double *, int *p, int *, double *tt) {
             mfx_x_primary(cfg, s->sx, n, u, p, tt);
         });
     } else if (precision == MFX_FAST_F32) {
-        const SceneF *sfp = nullptr;
-        MFX_TRY(fast_layout(s, false, cfg.variant, &sfp));
+        MFX_TRY(flatten_fast(s));
+        const SceneF *sfp = &s->sf;
         MFX_TRY(ensure_wave_fast(s, (size_t)n));
-        const bool hyb = sfp->own_tree && use_hybrid(0);
+        const bool hyb = use_hybrid(0);
         if (hyb) { MFX_TRY(flatten_hybrid(s)); MFX_TRY(ensure_wave_hybrid(s)); }
         return with_ray_buffers(s, n, uv, 2, nullptr, 0, prim, nullptr, t, [&](double *u, double *, int *p, int *, double *tt) {
             const bool sky = (s->integrator == MFX_SKY_TRACER);      // ListHit(ray, 0.00001, 10000000), RayTracing.fs:368

@@ -163,10 +163,12 @@ __device__ __forceinline__ D3 hyb_origin(const WaveH &wh, const D3 &cam_o, int c
 }
 
 // seam != 0 (Bvh.Hit / GetRay + Hit seams): the exact slot and the f64 t are kept; frames only need w.hit.
-template <int REFILL_T, int LEAF_T, int NSTEP, int MINB>
-__global__ void __launch_bounds__(FAST_BLOCK, MINB) k_h_trace(SceneF sc, const NodeX *nodes, const int *ref_id,
-                                                              SceneH sh, WaveF w, WaveH wh, int bounce, HybQuery q, D3 cam_o, int cam0, int seam)
+// Refill batches of 16 lanes, a leaf vote of 10 lanes, two node steps per iteration, 5 blocks per SM (96 registers): a
+// sweep in round 2 found other thresholds at most 1.5 % faster on primary rays, 0.2 % of a frame (profiles/r02_summary.md).
+__global__ void __launch_bounds__(FAST_BLOCK, 5) k_h_trace(SceneF sc, const NodeX *nodes, const int *ref_id,
+                                                          SceneH sh, WaveF w, WaveH wh, int bounce, HybQuery q, D3 cam_o, int cam0, int seam)
 {
+    constexpr int REFILL_T = 16, LEAF_T = 10, NSTEP = 2;
     extern __shared__ uint2 s_stack[];              // [stack_smem][FAST_BLOCK]
     uint2 *my_stack = s_stack + threadIdx.x;
     const int S = sc.stack_smem;
@@ -535,33 +537,15 @@ void mfx_h_seam_setup(const LaunchCfg &c, const SceneX &sx, const WaveF &w, cons
 {
     k_h_seam_setup<<<persistent_blocks(k_h_seam_setup, 256, c.blocks), 256, 0, c.stream>>>(sx, w, wh, n, o, d, uv, first);
 }
-template <int RT, int LT, int NS, int MB>
-static void launch_h_trace(const LaunchCfg &c, const SceneF &sc, const SceneX &sx, const SceneH &sh, const WaveF &w, const WaveH &wh, int bounce, HybQuery q, int seam)
-{
-    const size_t smem = (size_t)sc.stack_smem * FAST_BLOCK * sizeof(uint2);
-    auto kern = k_h_trace<RT, LT, NS, MB>;
-    int blocks = persistent_blocks(kern, FAST_BLOCK, c.blocks, smem);
-    if (sc.stack_spill && blocks * FAST_BLOCK > sc.spill_threads) blocks = sc.spill_threads / FAST_BLOCK;
-    if (c.max_items > 0) blocks = std::max(1, std::min(blocks, (c.max_items + FAST_BLOCK - 1) / FAST_BLOCK));
-    D3 cam_o; cam_o.x = sx.cam.pos[0]; cam_o.y = sx.cam.pos[1]; cam_o.z = sx.cam.pos[2];
-    kern<<<blocks, FAST_BLOCK, smem, c.stream>>>(sc, sx.nodes, sx.ref_id, sh, w, wh, bounce, q, cam_o, w.cam_origin, seam);
-}
 void mfx_h_extend(const LaunchCfg &c, const SceneF &sc, const SceneX &sx, const SceneH &sh, const WaveF &w, const WaveH &wh, int bounce, HybQuery q, int seam)
 {
     cudaMemsetAsync(wh.fix_n, 0, sizeof(int), c.stream);
-    switch (c.hyb_variant) {        // tuning knob (MFX_HYB_VARIANT, tools/hyb_sweep.py); <refill, leaf vote, node steps, blocks/SM>
-    case 1: launch_h_trace<16, 10, 2, 4>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 2: launch_h_trace<16, 10, 2, 3>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 3: launch_h_trace<16, 16, 2, 4>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 4: launch_h_trace<16, 10, 2, 6>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 5: launch_h_trace<16, 10, 1, 5>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 6: launch_h_trace<8, 10, 2, 5>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 7: launch_h_trace<24, 16, 2, 5>(c, sc, sx, sh, w, wh, bounce, q, seam); break;     // (7..10: thresholds for the coherent warps the path-id order gives)
-    case 8: launch_h_trace<16, 16, 2, 5>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 9: launch_h_trace<24, 10, 2, 5>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    case 10: launch_h_trace<28, 20, 2, 5>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    default: launch_h_trace<16, 10, 2, 5>(c, sc, sx, sh, w, wh, bounce, q, seam); break;
-    }
+    const size_t smem = (size_t)sc.stack_smem * FAST_BLOCK * sizeof(uint2);
+    int blocks = persistent_blocks(k_h_trace, FAST_BLOCK, c.blocks, smem);
+    if (sc.stack_spill && blocks * FAST_BLOCK > sc.spill_threads) blocks = sc.spill_threads / FAST_BLOCK;
+    if (c.max_items > 0) blocks = std::max(1, std::min(blocks, (c.max_items + FAST_BLOCK - 1) / FAST_BLOCK));
+    D3 cam_o; cam_o.x = sx.cam.pos[0]; cam_o.y = sx.cam.pos[1]; cam_o.z = sx.cam.pos[2];
+    k_h_trace<<<blocks, FAST_BLOCK, smem, c.stream>>>(sc, sx.nodes, sx.ref_id, sh, w, wh, bounce, q, cam_o, w.cam_origin, seam);
     k_h_fixup<<<c.blocks * 4, 128, 0, c.stream>>>(sx, sh, w, wh, bounce, q, w.cam_origin, seam);
 }
 void mfx_h_extend_x(const LaunchCfg &c, const SceneF &sc, const SceneX &sx, const SceneH &sh, const WaveX &wx, const WaveF &w, const WaveH &wh, int bounce, HybQuery q)

@@ -95,19 +95,13 @@ struct WaveX {
 // meta >= 0: leaf,  first<<3 | count (count <= 6 fast slots);  meta < 0: interior.
 // Boxes are rounded outward from the f64 bounds.
 struct __align__(16) PairF { float4 q0, q1, q2, q3; };
-// Two tree levels per fetch: one 128 B record per interior node at an EVEN depth holding the boxes
-// of its (up to) four grandchildren, SoA so one lane tests four boxes from seven 16 B loads.
-//   slot s <-> grandchild 4h+s (1-based heap index) when child 2h+(s>>1) is interior;
-//   a LEAF child occupies slot 2*(s>>1) itself, the other slot of that half is empty.
-//   meta >= 0: leaf (first<<3 | count), -1: interior (itself a quad node), -2: empty slot.
-// Records are stored compactly: index = h - ((2 << depth) + 1) / 3 (quads at even depths); for trees whose deepest
-// leaves sit at an odd depth the root is a 2-slot pseudo quad and the quads sit at odd depths (SceneF.qpar).
-struct __align__(16) QuadF { float4 lox, hix, loy, hiy, loz, hiz, meta, pad; };
-// The same 128 B record also carries the library's OWN tree (SceneF.own_tree = 1): a binned-SAH BVH over the fast
-// slots collapsed to four children per node.  The tree only decides the visiting order -- a nearest-hit query has one
+// One 128 B record per node of the library's OWN tree (SceneF.own_tree = 1): the boxes of its (up to) four children,
+// SoA so one lane tests four boxes from four 32 B loads.  The tree is a binned-SAH BVH over the fast slots collapsed to
+// four children per node.  The tree only decides the visiting order -- a nearest-hit query has one
 // answer whichever BVH finds it -- so MFX_FAST_F32 is free to use a better one than the reference's median split
-// (BvhNode.fs:42-61), which MFX_EXACT_F64 keeps because its tie rules are tree-shaped (quirk Q1).  Own-tree meta:
+// (BvhNode.fs:42-61), which MFX_EXACT_F64 keeps because its tie rules are tree-shaped (quirk Q1).  Meta:
 //   meta >= 0: leaf (first<<3 | count), MFX_QUAD_EMPTY: empty slot, other negatives: interior, child record = ~meta.
+struct __align__(16) QuadF { float4 lox, hix, loy, hiy, loz, hiz, meta, pad; };
 #define MFX_QUAD_EMPTY ((int)0x80000000)
 // One fast primitive slot, 48 B = 3 x float4, leaf order.
 //   triangle: a = (v0.xyz, kind bits), b = (e1.xyz, -), c = (e2.xyz, -)
@@ -124,17 +118,9 @@ struct LightF {
 };
 struct CamF { float pos[3], topleft[3], right[3], down[3]; };
 
-// The own tree again, 64 bytes per record (two 32-byte sectors instead of four): child planes as 8-bit offsets on a
-// per-record grid, origin o and power-of-two step s per axis -- plane = o + q*s, the min planes rounded down and the
-// max planes up by half a step more than the quantisation needs (the kernel folds the int->float conversion into one
-// fma whose constant carries up to half a step of rounding: mfx_fast.cu, k_f_trace6<CMP>).  Byte c of each word
-// belongs to child c; meta as in QuadF.
-struct __align__(32) QuadC { float ox, oy, oz, sx, sy, sz; unsigned lox, loy, loz, hix, hiy, hiz; int meta[4]; };
-
 struct SceneF {
     const PairF *pairs;     // indexed by the interior node's 1-based heap index h (siblings share a 128 B line)
-    const QuadF *quads;     // compact, even-depth interior nodes (see QuadF)
-    const QuadC *cquads;    // own tree only: the same records in 64 bytes (null unless built)
+    const QuadF *quads;     // own tree only: its records (see QuadF)
     const SlotF *slots;     // leaf order (rects split in two)
     const int   *slot_prim; // slot -> leaf-order primitive (exact slot) ; sub in bit 30
     const int   *ref_id;    // exact slot -> original primitive index
@@ -153,9 +139,7 @@ struct SceneF {
     int    n_quads, n_mats;     // record / material counts (bounds of the debug build's checks)
     int    levels;          // entries of the per-level entry-distance column (deepest child depth + 1)
     int    has_big_sphere;  // any kind-3 slot (selects the kernel variant with the f64 sphere branch)
-    int    qlevels;         // number of quad levels
-    int    qpar;            // 0: quads at even depths; 1: 2-slot pseudo root + quads at odd depths (odd leaf depth)
-    int    own_tree;        // 0: pairs/quads follow the reference tree (heap-indexed); 1: quads are the SAH 4-wide tree
+    int    own_tree;        // 0: pairs follow the reference tree (heap-indexed); 1: quads are the SAH 4-wide tree
     int    own_depth;       // own tree: number of quad levels (deferred-hit stack holds <= 3 per level)
     int    stack_smem;      // own tree: stack entries kept in shared memory per thread (<= MFX_STACK_SMEM_MAX)
     uint2 *stack_spill;     // own tree: [3*own_depth - stack_smem][spill_threads] overflow entries (null if none); every
@@ -252,7 +236,7 @@ struct TileMap {
 // ------------------------------------------------------------------ launchers (defined in the .cu TUs)
 // max_items > 0: the host knows an upper bound of the queue this launch works on (sky tracer, late bounces): the
 // persistent grid is clamped to the blocks that many entries can occupy
-struct LaunchCfg { int blocks; int threads; cudaStream_t stream; int variant; int reference_stream; int max_items; int hyb_variant; };
+struct LaunchCfg { int blocks; int threads; cudaStream_t stream; int reference_stream; int max_items; };
 
 // exact
 void mfx_x_raygen(const LaunchCfg &, const SceneX &, const WaveX &, TileMap tm, int pix0, int npix, int s0, int S,

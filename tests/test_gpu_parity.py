@@ -567,7 +567,9 @@ def test_traversal_counters_match_oracle_ordered_counts():
 
 def test_own_tree_counters_and_image_match_the_reference_tree_run():
     """MFX_SAMPLE_COUNT_OWN_TREE instruments the shipped kernel on the library's SAH tree: it must fetch far fewer
-    records than the reference tree has node tests, and render the same frame as the uninstrumented run."""
+    records than the reference tree has node tests, and render the same frame as the uninstrumented run.  The
+    reference-tree run (k_f_trace4) must render that frame too: a nearest-hit query has one answer whichever tree finds
+    it, so only pixels behind one of the rare tie-broken hits may change."""
     desc = _desc("c2_spot", width=240, height=135)
     s = Scene(desc)
     integ = CudaPixelIntegrator(s, precision=FAST_F32, seed=2)
@@ -575,8 +577,9 @@ def test_own_tree_counters_and_image_match_the_reference_tree_run():
     own = integ.Sample(2, flags=_lib.SAMPLE_COUNT_OWN_TREE).copy()
     so = dict(integ.stats)
     assert np.array_equal(plain, own)
-    integ.Sample(2, flags=_lib.SAMPLE_COUNT_TRAVERSAL)
+    ref = integ.Sample(2, flags=_lib.SAMPLE_COUNT_TRAVERSAL).copy()
     sr = dict(integ.stats)
+    assert (plain != ref).any(axis=2).mean() <= 5e-3
     assert so["closest_rays"] == sr["closest_rays"] or abs(so["closest_rays"] / sr["closest_rays"] - 1) < 1e-3
     for c, rays in ((0, "closest_rays"), (1, "shadow_rays")):
         rec, ref_nodes = so["nodes"][c] / so[rays], sr["nodes"][c] / sr[rays]
@@ -747,29 +750,6 @@ def test_cpp_host_driver_matches_python_host(tmp_path):
         target = film.GetFrame(integ, 2, first_sample=2 * f)
     want = np.transpose(target[:, :, :3], (1, 0, 2)).astype(np.float32)
     assert np.array_equal(img, want)
-
-
-@pytest.mark.parametrize("variant", ["4", "5", "51", "61", "62", "7"])
-def test_every_traversal_kernel_variant_gives_the_same_hits(monkeypatch, variant):
-    """The shipped kernel (default: own SAH tree, k_f_trace6), the reference-tree kernels (MFX_TRACE_VARIANT=4 binary --
-    also the instrumented counting kernel -- and 5 heap-indexed quads), other refill/vote thresholds and the 64-byte
-    quantised records (7: boxes only ever grow) must find the
-    same closest hits and frames: a nearest-hit query has one answer whichever tree finds it."""
-    desc = _desc("c3_renault", width=200, height=112)
-    s = Scene(desc)
-    rng = np.random.default_rng(8)
-    uv = rng.random((100000, 2))
-    monkeypatch.delenv("MFX_TRACE_VARIANT", raising=False)
-    monkeypatch.setenv("MFX_F32_PRIMARY", "1")            # like with like: the f32 primitive tests of every variant
-    p0, t0 = s.TracePrimary(uv, precision=FAST_F32)
-    img0 = CudaPixelIntegrator(s, precision=FAST_F32, seed=3).Sample(4).copy()
-    monkeypatch.setenv("MFX_TRACE_VARIANT", variant)
-    p1, t1 = s.TracePrimary(uv, precision=FAST_F32)
-    img1 = CudaPixelIntegrator(s, precision=FAST_F32, seed=3).Sample(4).copy()
-    # box tests differ in rounding between the layouts only through the order of visits: ties aside, same hits
-    assert (p0 != p1).mean() <= 1e-4 and np.allclose(t0[p0 == p1], t1[p0 == p1], rtol=1e-6, atol=1e-7)
-    # paths are deterministic given their hits: only pixels behind one of the rare tie-broken hits may change
-    assert (img0 != img1).any(axis=2).mean() <= 5e-3
 
 
 def test_film_checkpoint_resume_is_exact():

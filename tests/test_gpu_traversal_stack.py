@@ -1,6 +1,6 @@
 """The own-tree traversal stack and its spill columns.
 
-The own-tree kernels (k_f_trace6 in every variant, <CMP> and <TAIL> included, and the id-exact k_h_trace) keep the
+The own-tree kernels (k_f_trace6, <TAIL> included, and the id-exact k_h_trace) keep the
 first MFX_STACK_SMEM deferred-hit entries of a lane (default 12) in shared memory and everything deeper in a per-thread
 column of a global buffer, sized for 3*depth entries, the most a walk of the tree can push.  Where a value lives must
 not change an answer: every query and every frame below is compared bit for bit across shared-memory budgets of 1, 2
@@ -146,10 +146,10 @@ def test_seams_do_not_depend_on_the_shared_stack_budget(monkeypatch, name, kw):
     assert _fast_bytes(monkeypatch, desc, "1") > _fast_bytes(monkeypatch, desc, ALL_SHARED)      # the small budgets did spill
 
 
-def _frame(monkeypatch, desc, spp, seed=3, smem=None, two=None, variant=None):
+def _frame(monkeypatch, desc, spp, seed=3, smem=None, two=None):
     """One fast Sample on a fresh scene under the given knobs: (frame, closest rays, shadow rays)."""
     from mafrixraytracing_b200 import Scene, CudaPixelIntegrator, FAST_F32
-    for var, val in (("MFX_STACK_SMEM", smem), ("MFX_TWO_STREAMS", two), ("MFX_TRACE_VARIANT", variant)):
+    for var, val in (("MFX_STACK_SMEM", smem), ("MFX_TWO_STREAMS", two)):
         if val is None:
             monkeypatch.delenv(var, raising=False)
         else:
@@ -162,13 +162,13 @@ def _frame(monkeypatch, desc, spp, seed=3, smem=None, two=None, variant=None):
     return img, st["closest_rays"], st["shadow_rays"]
 
 
-def _all_budgets_and_streams_agree(monkeypatch, desc, spp, variant=None):
-    want = _frame(monkeypatch, desc, spp, smem=ALL_SHARED, two="0", variant=variant)
+def _all_budgets_and_streams_agree(monkeypatch, desc, spp):
+    want = _frame(monkeypatch, desc, spp, smem=ALL_SHARED, two="0")
     assert want[0][:, :, :3].mean() > 0 and want[2] > 0
     bad = []
     for smem in (ALL_SHARED, "12", "3", "1"):
         for two in ("0", "1"):
-            img, closest, shadow = _frame(monkeypatch, desc, spp, smem=smem, two=two, variant=variant)
+            img, closest, shadow = _frame(monkeypatch, desc, spp, smem=smem, two=two)
             if not (np.array_equal(img, want[0]) and closest == want[1] and shadow == want[2]):
                 bad.append(f"MFX_STACK_SMEM={smem} MFX_TWO_STREAMS={two}: {int((img != want[0]).any(axis=2).sum())} pixels, "
                            f"rays {closest}/{shadow} against {want[1]}/{want[2]}")
@@ -182,14 +182,6 @@ def test_frames_do_not_depend_on_the_stack_budget_or_the_streams(monkeypatch, na
     """Fast frames at 16 spp with 1, 3, 12 and all stack entries in shared memory, each on one stream and on two (shadow
     queries of bounce b beside the closest hits of bounce b+1): the same frame and the same ray counts every time."""
     _all_budgets_and_streams_agree(monkeypatch, _desc(name, **kw), 16)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("variant", ["7", "62"])
-def test_other_trace_variants_do_not_depend_on_the_stack_budget_or_the_streams(monkeypatch, variant):
-    """The same for the 64-byte records (k_f_trace6<CMP>) and the one-step, two-leaf kernel, each against its own
-    all-in-shared one-stream frame."""
-    _all_budgets_and_streams_agree(monkeypatch, _haystack(width=160, height=90), 16, variant=variant)
 
 
 @pytest.mark.gpu

@@ -71,19 +71,3 @@ def test_shadow_query_order_is_answer_invariant_and_cheaper_in_the_cpu_model(wor
     if workload == "c2_spot":
         assert 3.0 < tot_near[0] < 3.7 and 3.6 < tot_near[2] < 4.7     # the GPU measures 3.35 and 4.19 records per ray
         assert tot_far[2] < 0.9 * tot_near[2]
-
-
-@pytest.mark.parametrize("workload", ["c2_spot", "cornell"])
-def test_quantised_records_are_conservative_and_cost_primitive_tests_in_the_cpu_model(workload):
-    """The 64-byte records (QuadC, mfx_compress_quads: child planes on an 8-bit grid per record) must only ever GROW a
-    box -- the simulator refuses a grid plane inside the box it replaces -- and give the same answers as the f32 records,
-    with the kernel's one-fma plane arithmetic too (SIM_QUANT=2); the price that keeps them out of the shipped path is
-    visible without a GPU: more primitive tests per ray (DESIGN.md 7, profiles/r02_compressed_records_negative.jsonl)."""
-    occ0, tot0 = _own_tree_sim(workload)
-    occ1, tot1 = _own_tree_sim(workload, {"SIM_QUANT": "1"})
-    occ2, tot2 = _own_tree_sim(workload, {"SIM_QUANT": "2"})
-    assert occ0[0] == occ1[0] == occ2[0] and occ1[5] == 0 and occ2[5] == 0      # the same shadow rays are occluded
-    assert tot1[0] >= tot0[0] and tot1[1] >= tot0[1] and tot2[0] >= tot0[0] and tot2[1] >= tot0[1]
-    assert abs(tot2[0] - tot1[0]) < 0.05 * tot1[0] and abs(tot2[1] - tot1[1]) < 0.05 * tot1[1]
-    if workload == "c2_spot":
-        assert tot1[1] > 1.2 * tot0[1]                   # the GPU measures 2.07 -> 3.10 primitive tests per closest-hit ray

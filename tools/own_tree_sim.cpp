@@ -47,13 +47,11 @@ static float as_float(unsigned u) { float f; memcpy(&f, &u, 4); return f; }
 
 static bool g_any_nearest = false;
 static int g_smem = 12;         // MFX_STACK_SMEM
-static int g_quant = 0;          // SIM_QUANT: 1 = boxes replaced by their 8-bit grid planes (QuadC), 2 = plus the kernel's one-fma plane arithmetic
 struct Tri { V v0, e1, e2, n; };
 struct Counts { double rays = 0, records = 0, tris = 0, leaf_visits = 0, deep = 0; int peak = 0; };   // deep: rays whose stack rose above g_smem
 
 struct Sim {
     const MfxOwnTree *t;
-    const std::vector<QuadC> *cq = nullptr;
     std::vector<Tri> tri;        // leaf order
     bool test_leaf(int leaf, V o, V d, float tmin, int src, float &best, int &best_slot, Counts &c) const
     {
@@ -94,21 +92,9 @@ struct Sim {
                 const float *lo[3] = { &q.lox.x, &q.loy.x, &q.loz.x }, *hi[3] = { &q.hix.x, &q.hiy.x, &q.hiz.x };
                 unsigned key[4];
                 for (int s = 0; s < 4; s++) {
-                    float x0 = lo[0][s] * id.x - ood.x, x1 = hi[0][s] * id.x - ood.x;
-                    float y0 = lo[1][s] * id.y - ood.y, y1 = hi[1][s] * id.y - ood.y;
-                    float z0 = lo[2][s] * id.z - ood.z, z1 = hi[2][s] * id.z - ood.z;
-                    if (g_quant == 2) {         // k_f_trace6<CMP>: t = (2^23 + q) * S + (C - 2^23 * S)
-                        const QuadC &c = (*cq)[node];
-                        const float S[3] = { c.sx * id.x, c.sy * id.y, c.sz * id.z };
-                        const float Cc[3] = { std::fmaf(-8388608.f, S[0], std::fmaf(c.ox, id.x, -ood.x)), std::fmaf(-8388608.f, S[1], std::fmaf(c.oy, id.y, -ood.y)),
-                                              std::fmaf(-8388608.f, S[2], std::fmaf(c.oz, id.z, -ood.z)) };
-                        const unsigned wl[3] = { c.lox, c.loy, c.loz }, wh[3] = { c.hix, c.hiy, c.hiz };
-                        float *out[3][2] = { { &x0, &x1 }, { &y0, &y1 }, { &z0, &z1 } };
-                        for (int a = 0; a < 3; a++) {
-                            *out[a][0] = std::fmaf(as_float(0x4B000000u | ((wl[a] >> (8 * s)) & 255u)), S[a], Cc[a]);
-                            *out[a][1] = std::fmaf(as_float(0x4B000000u | ((wh[a] >> (8 * s)) & 255u)), S[a], Cc[a]);
-                        }
-                    }
+                    const float x0 = lo[0][s] * id.x - ood.x, x1 = hi[0][s] * id.x - ood.x;
+                    const float y0 = lo[1][s] * id.y - ood.y, y1 = hi[1][s] * id.y - ood.y;
+                    const float z0 = lo[2][s] * id.z - ood.z, z1 = hi[2][s] * id.z - ood.z;
                     const float tn = std::max(std::max(std::min(x0, x1), std::min(y0, y1)), std::max(std::min(z0, z1), tmin));
                     const float tf = std::min(std::min(std::max(x0, x1), std::max(y0, y1)), std::min(std::max(z0, z1), best));
                     const int mt = as_int((&q.meta.x)[s]);
@@ -173,35 +159,8 @@ int main(int argc, char **argv)
     MfxOwnTree tree;
     const auto tb0 = std::chrono::steady_clock::now();
     mfx_build_own_tree(lo.data(), hi.data(), n, (int)mfx_env_long("MFX_SAH_MAX_LEAF", 4), (float)mfx_env_long("MFX_SAH_TRAV_COST_PCT", 100) * 0.01f, 3, tree);
-    g_quant = (int)mfx_env_long("SIM_QUANT", 0);
-    std::vector<QuadC> cq;
-    if (g_quant) {
-        mfx_compress_quads(tree.quads, cq);
-        double infl[2] = { 0, 0 }, cnt[2] = { 0, 0 };
-        for (size_t i = 0; i < cq.size(); i++) {
-            QuadF &q = tree.quads[i]; const QuadC &c = cq[i];
-            float *lo[3] = { &q.lox.x, &q.loy.x, &q.loz.x }, *hi[3] = { &q.hix.x, &q.hiy.x, &q.hiz.x };
-            const float org[3] = { c.ox, c.oy, c.oz }, st[3] = { c.sx, c.sy, c.sz };
-            const unsigned wl[3] = { c.lox, c.loy, c.loz }, wh[3] = { c.hix, c.hiy, c.hiz };
-            for (int s = 0; s < 4; s++) {
-                const int m = as_int((&q.meta.x)[s]);
-                if (m == MFX_QUAD_EMPTY) continue;
-                double e0[3], e1[3];
-                for (int a = 0; a < 3; a++) {
-                    e0[a] = (double)hi[a][s] - lo[a][s];
-                    const float nl = org[a] + (float)((wl[a] >> (8 * s)) & 255u) * st[a], nh = org[a] + (float)((wh[a] >> (8 * s)) & 255u) * st[a];
-                    if (nl > lo[a][s] || nh < hi[a][s]) { fprintf(stderr, "record %zu child %d axis %d: grid planes inside the box\n", i, s, a); return 1; }
-                    lo[a][s] = nl; hi[a][s] = nh;
-                    e1[a] = (double)nh - nl;
-                }
-                const double a0 = e0[0] * e0[1] + e0[1] * e0[2] + e0[2] * e0[0], a1 = e1[0] * e1[1] + e1[1] * e1[2] + e1[2] * e1[0];
-                if (a0 > 0.) { infl[m >= 0] += a1 / a0; cnt[m >= 0] += 1; }
-            }
-        }
-        printf("8-bit grids: mean surface-area ratio of a child box, interior %.4f, leaf %.4f\n", infl[0] / cnt[0], infl[1] / cnt[1]);
-    }
     printf("own tree built in %.2f ms\n", std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tb0).count());
-    Sim sim; sim.t = &tree; sim.cq = &cq; sim.tri.resize(n);
+    Sim sim; sim.t = &tree; sim.tri.resize(n);
     for (int k = 0; k < n; k++) {
         const double *p = &raw[9 * (size_t)tree.order[k]];
         const V v0 = { (float)p[0], (float)p[1], (float)p[2] };

@@ -1,5 +1,5 @@
 """Small end-to-end run for compute-sanitizer: every fast/exact/hybrid kernel, all three integrators, spheres incl. the f64
-big one, own-tree counters, reference-tree variants, Film + tone map / sky display, seams (id-exact and f32, incl. the
+big one, own-tree and reference-tree counters, Film + tone map / sky display, seams (id-exact and f32, incl. the
 exact fixup of axis-parallel rays), tiles and stripes, the async entry point, mfx_multi_* on the visible devices."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
