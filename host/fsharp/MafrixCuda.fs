@@ -55,6 +55,14 @@ module Native =
     [<DllImport(Lib)>] extern int mfx_film_destroy(nativeint film)
     [<DllImport(Lib)>] extern int mfx_film_get_frame(nativeint film, MfxSampleParams& p, nativeint texture)
     [<DllImport(Lib)>] extern int mfx_film_post_process(nativeint film, nativeint rgba8)
+    // the Film over the N GPUs of an mfx_multi handle: every device accumulates and tone-maps its own stripes
+    [<DllImport(Lib)>] extern int mfx_multi_film_create(nativeint multi, nativeint& film)
+    [<DllImport(Lib)>] extern int mfx_multi_film_destroy(nativeint film)
+    [<DllImport(Lib)>] extern int mfx_multi_film_reset(nativeint film)
+    [<DllImport(Lib)>] extern int mfx_multi_film_get_frame(nativeint film, MfxSampleParams& p, nativeint texture)
+    [<DllImport(Lib)>] extern int mfx_multi_film_post_process(nativeint film, nativeint rgba8)
+    [<DllImport(Lib)>] extern int mfx_multi_film_export(nativeint film, nativeint sum, double& frameCount)
+    [<DllImport(Lib)>] extern int mfx_multi_film_import(nativeint film, nativeint sum, double frameCount)
     // the sphere sample (RenderTest/Sample/RayTracing.fs, MFX_SKY_TRACER): RayTraceCamera's constructor -> MfxLensCamera (152 B)
     [<DllImport(Lib)>] extern int mfx_camera_lens(double[] lookfrom, double[] lookat, double[] vup, double vfov, double aspect, double aperture, double focusDist, nativeint out)
 
@@ -154,13 +162,19 @@ type CudaPixelIntegrator(width:int, height:int, cam:PinholeCamera, bvh:Bvh, ligh
             h
         finally
             for p in [ d; pPrims; pMats; pNodes; pIdx ] do Marshal.FreeHGlobal p
+    /// the scene handle (an MfxMulti when gpus > 1) and the params of the next n samples: fresh samples every displayed frame
+    member this.Handle = scene
+    member this.Gpus = nGpus
+    member this.NextParams(n:int) =
+        let mutable p = MfxSampleParams()
+        p.precision <- (if defaultArg fast true then 1 else 0)
+        p.spp <- n; p.seed <- defaultArg seed 1UL
+        p.firstSample <- frame; p.world <- 1
+        frame <- frame + n
+        p
     interface IPixelIntegrator with
         member this.Sample(n:int) =                              // Integrators.fs:160-172
-            let mutable p = MfxSampleParams()
-            p.precision <- (if defaultArg fast true then 1 else 0)
-            p.spp <- n; p.seed <- defaultArg seed 1UL
-            p.firstSample <- frame; p.world <- 1
-            frame <- frame + n                                   // fresh samples every displayed frame
+            let mutable p = this.NextParams n
             if nGpus > 1 then check (Native.mfx_multi_sample(scene, &p, pin.AddrOfPinnedObject()))   // every device DMAs its stripes
             else check (Native.mfx_pixel_integrator_sample(scene, &p, pin.AddrOfPinnedObject()))
             tex2d
@@ -169,3 +183,30 @@ type CudaPixelIntegrator(width:int, height:int, cam:PinholeCamera, bvh:Bvh, ligh
             Native.mfx_host_unregister(pin.AddrOfPinnedObject()) |> ignore
             (if nGpus > 1 then Native.mfx_multi_destroy scene else Native.mfx_scene_destroy scene) |> ignore
             pin.Free()
+
+/// Film.GetFrame + PostProcessAndToScreenBuffer kept on the GPU(s) (Film.fs:18-34, Scene.fs:315-330).  The window loop of
+/// Scene.Render (:331-333) becomes `film.GetFrame 1; film.PostProcess buffer`: only the RGBA8 screen crosses PCIe.  With
+/// gpus > 1 every device keeps the Film of its own column stripes (mfx_multi_film_*), bit-identical to one GPU.
+/// Dispose it before the integrator.
+type CudaFilm(integrator:CudaPixelIntegrator) =
+    let multi = integrator.Gpus > 1
+    let film =
+        let mutable h = 0n
+        if multi then check (Native.mfx_multi_film_create(integrator.Handle, &h))
+        else check (Native.mfx_film_create(integrator.Handle, &h))
+        h
+    /// Film.GetFrame(integrator, n): the target stays on the device(s)
+    member this.GetFrame(n:int) =
+        let mutable p = integrator.NextParams n
+        if multi then check (Native.mfx_multi_film_get_frame(film, &p, 0n))
+        else check (Native.mfx_film_get_frame(film, &p, 0n))
+    /// PostProcessAndToScreenBuffer into the window's w*h*4 byte buffer
+    member this.PostProcess(buffer:byte[]) =
+        let pin = GCHandle.Alloc(buffer, GCHandleType.Pinned)
+        try
+            if multi then check (Native.mfx_multi_film_post_process(film, pin.AddrOfPinnedObject()))
+            else check (Native.mfx_film_post_process(film, pin.AddrOfPinnedObject()))
+        finally pin.Free()
+    interface IDisposable with
+        member this.Dispose() =
+            (if multi then Native.mfx_multi_film_destroy film else Native.mfx_film_destroy film) |> ignore

@@ -6,8 +6,9 @@
 //
 //   render_test [--obj file.obj] [--frames N] [--spp S] [--size WxH] [--depth D] [--exact] [--gpus N] [--out prefix]
 //
-// --gpus N (N > 1): the same single-threaded loop over mfx_multi_* -- the library replicates the scene on N devices and
-// fills the one Texture2D<Color>; Film.AddSample (Film.fs:18-23) then runs on the host like in the reference.
+// --gpus N: the same single-threaded loop over mfx_multi_* -- the library replicates the scene on N devices and
+// every device keeps the Film (Film.fs:13-34) of its own stripes (mfx_multi_film_*); only the last frame's texture and
+// the screen cross PCIe.
 //
 // Without --obj it renders the reference's default scene: the Cornell box of Scene.xml
 // (RayTracing4.fs:9-72: camera (0,1,3) looking -z, fov 120, 300x300, three Lambert materials,
@@ -130,7 +131,7 @@ static void write_ppm(const std::string &path, const std::vector<uint8_t> &rgba,
 int main(int argc, char **argv)
 {
     std::string obj, out = "render_test";
-    int frames = 16, spp = 1, w = 300, h = 300, depth = 3, precision = MFX_FAST_F32, gpus = 1;
+    int frames = 16, spp = 1, w = 300, h = 300, depth = 3, precision = MFX_FAST_F32, gpus = 0;
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         if (a == "--obj" && i + 1 < argc) obj = argv[++i];
@@ -182,31 +183,29 @@ int main(int argc, char **argv)
     CHECK(mfx_camera_pinhole(pos, dir, 120.0, (double)w / h, &desc.camera));   // PinholeCamera(pos, dir, 120, aspect)
     desc.width = w; desc.height = h; desc.max_depth = depth; desc.integrator = MFX_PATH_INTEGRATOR;
 
-    if (gpus > 1) {
+    if (gpus > 0) {
         // N GPUs behind the same single-threaded host loop: the library shards, this thread sees IPixelIntegrator.Sample
         if (mfx_device_count() < gpus) { fprintf(stderr, "render_test: --gpus %d but %d device(s) visible\n", gpus, mfx_device_count()); return 1; }
-        MfxMulti *multi = nullptr;
+        MfxMulti *multi = nullptr; MfxMultiFilm *film = nullptr;
         CHECK(mfx_multi_create(&desc, nullptr, gpus, &multi));
-        std::vector<double> frame((size_t)w * h * 4), sum((size_t)w * h * 4, 0.0), target((size_t)w * h * 4, 0.0);
-        CHECK(mfx_host_register(frame.data(), frame.size() * sizeof(double)));      // the host keeps ONE texture (Integrators.fs:147)
+        CHECK(mfx_multi_film_create(multi, &film));                 // every device keeps the Film of its own stripes
+        std::vector<double> target((size_t)w * h * 4);
+        std::vector<uint8_t> screen((size_t)w * h * 4);
         double ms = 0; uint64_t rays = 0;
         for (int f = 0; f < frames; f++) {
             MfxSampleParams sp; memset(&sp, 0, sizeof(sp));
             sp.precision = precision; sp.spp = spp; sp.seed = 1; sp.first_sample = f * spp; sp.world = 1;
-            CHECK(mfx_multi_sample(multi, &sp, frame.data()));
-            const double fc = (double)(f + 1);
-            for (size_t i = 0; i < sum.size(); i += 4) {            // Film.AddSample, Film.fs:18-23
-                for (int c = 0; c < 3; c++) { const double v = sum[i + c] + frame[i + c]; sum[i + c] = v; target[i + c] = v / fc; }
-                target[i + 3] = 1.0;
-            }
+            CHECK(mfx_multi_film_get_frame(film, &sp, f + 1 == frames ? target.data() : nullptr));   // Film.GetFrame(integrator, spp)
             MfxStats st; CHECK(mfx_multi_get_stats(multi, &st, nullptr));
             ms += st.ms_total; rays += st.closest_rays + st.shadow_rays;
         }
-        CHECK(mfx_host_unregister(frame.data()));
+        CHECK(mfx_multi_film_post_process(film, screen.data()));     // PostProcessAndToScreenBuffer
         write_pfm(out + ".pfm", target, w, h);
-        printf("%s: %zu primitives, %dx%d, %d frames x %d spp, depth %d, %s, %d GPUs: %.2f ms on the slowest device, %.1f Mrays/s -> %s.pfm\n",
+        write_ppm(out + ".ppm", screen, w, h);
+        printf("%s: %zu primitives, %dx%d, %d frames x %d spp, depth %d, %s, %d GPUs: %.2f ms on the slowest device, %.1f Mrays/s -> %s.pfm / .ppm\n",
                obj.empty() ? "cornell" : obj.c_str(), prims.size(), w, h, frames, spp, depth,
                precision == MFX_FAST_F32 ? "f32" : "f64", gpus, ms, rays / (ms * 1e3), out.c_str());
+        mfx_multi_film_destroy(film);
         mfx_multi_destroy(multi);
         return 0;
     }

@@ -322,6 +322,30 @@ MFX_API int mfx_film_frame_count(const MfxFilm *film, double *out);
 MFX_API int mfx_film_export(MfxFilm *film, double *sum_color_wh, double *frame_count);
 MFX_API int mfx_film_import(MfxFilm *film, const double *sum_color_wh, double frame_count);
 
+/* ---- Film over several GPUs (Film.fs:13-34 on an MfxMulti handle) --------------------------------
+ * Every device accumulates, divides and tone-maps only the column stripes it owns, in its own HBM (a full-frame sum,
+ * target and RGBA8 buffer per device, of which only the owned stripes are touched), and copies only its stripes of
+ * what the caller asks for.  Every result is bit-identical to the one-GPU mfx_film_* on the same scene, params and seed.
+ * Rules: mfx_multi_destroy fails with MFX_ERR_INVALID_ARGUMENT while a film of the handle is alive; a film call while an
+ * mfx_multi_sample_async of the handle has not been waited for is refused; a plain mfx_multi_sample between film frames
+ * leaves the film untouched. */
+typedef struct MfxMultiFilm MfxMultiFilm;
+MFX_API int mfx_multi_film_create(MfxMulti *multi, MfxMultiFilm **out);
+MFX_API int mfx_multi_film_destroy(MfxMultiFilm *film);
+MFX_API int mfx_multi_film_reset(MfxMultiFilm *film);                        /* Film.Reset, Film.fs:26-30 */
+/* Film.GetFrame, Film.fs:18-23,32-34: Sample over all devices, sum += frame, target = sum / frameCount; texture
+ * (Color[w,h], may be NULL) receives target.  params are read as mfx_multi_sample reads them: rank, world and
+ * tile_size are ignored, world > 1 is refused. */
+MFX_API int mfx_multi_film_get_frame(MfxMultiFilm *film, const MfxSampleParams *params, double *texture);
+/* mfx_film_post_process over the devices' stripes (Scene.fs:315-330; RayTracing.fs:456-460 under MFX_SKY_TRACER),
+ * byte for byte the same RGBA8 at x*4 + y*width*4. */
+MFX_API int mfx_multi_film_post_process(MfxMultiFilm *film, uint8_t *rgba8);
+MFX_API int mfx_multi_film_frame_count(const MfxMultiFilm *film, double *out);
+/* The same checkpoint as mfx_film_export / _import (full Color[w,h] running sum + frameCount): a film exported from
+ * N devices resumes on M devices or on a one-GPU MfxFilm, and the other way round. */
+MFX_API int mfx_multi_film_export(MfxMultiFilm *film, double *sum_color_wh, double *frame_count);
+MFX_API int mfx_multi_film_import(MfxMultiFilm *film, const double *sum_color_wh, double frame_count);
+
 #ifdef __cplusplus
 }
 #endif

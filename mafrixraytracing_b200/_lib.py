@@ -112,6 +112,14 @@ SYMBOLS = {
     "mfx_film_frame_count": (C.c_int, [_P, C.POINTER(C.c_double)]),
     "mfx_film_export": (C.c_int, [_P, _P, C.POINTER(C.c_double)]),
     "mfx_film_import": (C.c_int, [_P, _P, C.c_double]),
+    "mfx_multi_film_create": (C.c_int, [_P, C.POINTER(_P)]),
+    "mfx_multi_film_destroy": (C.c_int, [_P]),
+    "mfx_multi_film_reset": (C.c_int, [_P]),
+    "mfx_multi_film_get_frame": (C.c_int, [_P, C.POINTER(MfxSampleParams), _P]),
+    "mfx_multi_film_post_process": (C.c_int, [_P, _P]),
+    "mfx_multi_film_frame_count": (C.c_int, [_P, C.POINTER(C.c_double)]),
+    "mfx_multi_film_export": (C.c_int, [_P, _P, C.POINTER(C.c_double)]),
+    "mfx_multi_film_import": (C.c_int, [_P, _P, C.c_double]),
 }
 
 _lib = None

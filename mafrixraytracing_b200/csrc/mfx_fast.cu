@@ -950,10 +950,16 @@ __global__ void k_accum_totals(const int *counts, int ext_lo, int ext_n, int sh_
     totals[5] += (unsigned)counts[MFX_DBG_SLOT];            // violations counted by a debug build (MFX_DEBUG_CHECKS)
 }
 
+// The film kernels work on the pixels `tm` owns (pixel_of): a device of mfx_multi_film_* touches its own column stripes
+// only, the one-GPU film passes one stripe as wide as the frame.  Color[w,h] buffers are x-major (x*H+y), RGBA8 row-major.
+
 // Film.AddSample (Film.fs:18-23): c = sum + frame; sum <- c; target <- c / frameCount
-__global__ void __launch_bounds__(256) k_film_add(double *sum, const double *frame, double *target, long long n_pixels, double fc)
+__global__ void __launch_bounds__(256) k_film_add(TileMap tm, int width, double *sum, const double *frame, double *target, double fc)
 {
-    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < n_pixels; p += (long long)gridDim.x * blockDim.x) {
+    for (int pl = blockIdx.x * blockDim.x + threadIdx.x; pl < tm.n_pix; pl += gridDim.x * blockDim.x) {
+        int pix, x, y;
+        pixel_of(tm, width, pl, pix, x, y);
+        const size_t p = (size_t)x * tm.height + y;
         for (int c = 0; c < 3; c++) {
             const double v = sum[4 * p + c] + frame[4 * p + c];
             sum[4 * p + c] = v;
@@ -969,12 +975,12 @@ __device__ __forceinline__ double clamp01(double x) { return x < 0. ? 0. : (x > 
 
 // ACESFilmToneMapping + sqrt + int(255.99 c) (Scene.fs:273-289,315-330).  target is Color[w,h]
 // x-major; out is RGBA8 at x*4 + y*width*4.  f64 with explicit non-fused operations.
-__global__ void __launch_bounds__(256) k_film_tonemap(const double *target, int width, int height, uint8_t *rgba8)
+__global__ void __launch_bounds__(256) k_film_tonemap(TileMap tm, int width, const double *target, uint8_t *rgba8)
 {
-    const long long n = (long long)width * height;
-    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (long long)gridDim.x * blockDim.x) {
-        const int y = (int)(p / width), x = (int)(p - (long long)y * width);
-        const double *px = target + ((size_t)x * height + y) * 4;
+    for (int pl = blockIdx.x * blockDim.x + threadIdx.x; pl < tm.n_pix; pl += gridDim.x * blockDim.x) {
+        int pix, x, y;
+        pixel_of(tm, width, pl, pix, x, y);
+        const double *px = target + ((size_t)x * tm.height + y) * 4;
         uint8_t out[4];
         for (int c = 0; c < 3; c++) {
             const double v = px[c];
@@ -984,24 +990,25 @@ __global__ void __launch_bounds__(256) k_film_tonemap(const double *target, int 
             out[c] = (uint8_t)(int)__dmul_rn(255.99, q);
         }
         out[3] = 255;
-        *reinterpret_cast<uchar4 *>(rgba8 + 4 * p) = make_uchar4(out[0], out[1], out[2], out[3]);
+        *reinterpret_cast<uchar4 *>(rgba8 + 4 * (size_t)pix) = make_uchar4(out[0], out[1], out[2], out[3]);
     }
 }
 
 // The sphere sample's display transform (RenderTest/Sample/RayTracing.fs:456-460): sqrt, int(255.99 c), and
-// screen[i, (ny-1)-j]: row j of the texture (v grows upwards from lowerLeftCorner) lands on screen row ny-1-j.
-__global__ void __launch_bounds__(256) k_film_display_sky(const double *target, int width, int height, uint8_t *rgba8)
+// screen[i, (ny-1)-j]: row j of the texture (v grows upwards from lowerLeftCorner) lands on screen row ny-1-j.  The flip
+// keeps the column, so a device's stripes of the screen come from its own stripes of the texture.
+__global__ void __launch_bounds__(256) k_film_display_sky(TileMap tm, int width, const double *target, uint8_t *rgba8)
 {
-    const long long n = (long long)width * height;
-    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (long long)gridDim.x * blockDim.x) {
-        const int y = (int)(p / width), x = (int)(p - (long long)y * width);
-        const double *px = target + ((size_t)x * height + (height - 1 - y)) * 4;
+    for (int pl = blockIdx.x * blockDim.x + threadIdx.x; pl < tm.n_pix; pl += gridDim.x * blockDim.x) {
+        int pix, x, y;
+        pixel_of(tm, width, pl, pix, x, y);
+        const double *px = target + ((size_t)x * tm.height + (tm.height - 1 - y)) * 4;
         uint8_t out[3];
         for (int c = 0; c < 3; c++) {
             const double v = __dmul_rn(255.99, sqrt(px[c]));
             out[c] = (v == v) ? (uint8_t)(int)v : 0;
         }
-        *reinterpret_cast<uchar4 *>(rgba8 + 4 * p) = make_uchar4(out[0], out[1], out[2], 255);
+        *reinterpret_cast<uchar4 *>(rgba8 + 4 * (size_t)pix) = make_uchar4(out[0], out[1], out[2], 255);
     }
 }
 
@@ -1089,17 +1096,17 @@ void mfx_accum_ray_totals(cudaStream_t s, const int *counts, int ext_lo, int ext
 {
     k_accum_totals<<<1, 1, 0, s>>>(counts, ext_lo, ext_n, sh_lo, sh_n, totals);
 }
-void mfx_film_add(cudaStream_t s, double *sum, const double *frame, double *target, long long n_pixels, double fc)
+void mfx_film_add(cudaStream_t s, TileMap tm, int width, double *sum, const double *frame, double *target, double fc)
 {
-    k_film_add<<<592, 256, 0, s>>>(sum, frame, target, n_pixels, fc);
+    k_film_add<<<592, 256, 0, s>>>(tm, width, sum, frame, target, fc);
 }
-void mfx_film_tonemap(cudaStream_t s, const double *target_wh, int width, int height, uint8_t *rgba8)
+void mfx_film_tonemap(cudaStream_t s, TileMap tm, int width, const double *target_wh, uint8_t *rgba8)
 {
-    k_film_tonemap<<<592, 256, 0, s>>>(target_wh, width, height, rgba8);
+    k_film_tonemap<<<592, 256, 0, s>>>(tm, width, target_wh, rgba8);
 }
-void mfx_film_display_sky(cudaStream_t s, const double *target_wh, int width, int height, uint8_t *rgba8)
+void mfx_film_display_sky(cudaStream_t s, TileMap tm, int width, const double *target_wh, uint8_t *rgba8)
 {
-    k_film_display_sky<<<592, 256, 0, s>>>(target_wh, width, height, rgba8);
+    k_film_display_sky<<<592, 256, 0, s>>>(tm, width, target_wh, rgba8);
 }
 void mfx_fill_zero_f64(cudaStream_t s, double *p, long long n)
 {

@@ -1749,6 +1749,18 @@ struct MfxFilm {
     double frame_count = 0.;
 };
 
+// The pixels a film kernel works on: `rank`'s column stripes out of `world`; world 1 = the whole frame (pixel_of's identity).
+static TileMap film_tilemap(int width, int height, int stripe, int rank, int world)
+{
+    TileMap tm;
+    memset(&tm, 0, sizeof(tm));
+    tm.height = height;
+    if (world <= 1) { tm.n_pix = width * height; return tm; }
+    tm.stripe = stripe; tm.rank = rank; tm.world = world;
+    tm.n_pix = stripe_pixels(width, height, stripe, rank, world);
+    return tm;
+}
+
 extern "C" int mfx_film_create(MfxScene *s, MfxFilm **out)
 {
     if (!s || !out) return fail(MFX_ERR_INVALID_ARGUMENT, "null argument");
@@ -1806,7 +1818,7 @@ extern "C" int mfx_film_get_frame(MfxFilm *f, const MfxSampleParams *p, double *
     MFX_TRY(run_sample(s, p, s->d_color_wh, nullptr));
     f->frame_count += 1.;
     const size_t npx = (size_t)s->width * s->height;
-    mfx_film_add(s->stream, f->d_sum, s->d_color_wh, f->d_target, (long long)npx, f->frame_count);
+    mfx_film_add(s->stream, film_tilemap(s->width, s->height, 0, 0, 1), s->width, f->d_sum, s->d_color_wh, f->d_target, f->frame_count);
     CUDA_TRY(cudaGetLastError());
     if (texture) return copy_out(s, texture, f->d_target, npx * 4 * sizeof(double));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
@@ -1819,8 +1831,9 @@ extern "C" int mfx_film_post_process(MfxFilm *f, uint8_t *rgba8)   // Scene.fs:3
     MfxScene *s = f->scene;
     MFX_TRY(bind_device(f->scene->device));
     // MFX_SKY_TRACER: the sphere sample shows sqrt(c) flipped vertically (RayTracing.fs:456-460), no ACES curve
-    if (s->integrator == MFX_SKY_TRACER) mfx_film_display_sky(s->stream, f->d_target, s->width, s->height, f->d_rgba8);
-    else mfx_film_tonemap(s->stream, f->d_target, s->width, s->height, f->d_rgba8);
+    const TileMap tm = film_tilemap(s->width, s->height, 0, 0, 1);
+    if (s->integrator == MFX_SKY_TRACER) mfx_film_display_sky(s->stream, tm, s->width, f->d_target, f->d_rgba8);
+    else mfx_film_tonemap(s->stream, tm, s->width, f->d_target, f->d_rgba8);
     CUDA_TRY(cudaGetLastError());
     return copy_out(s, rgba8, f->d_rgba8, (size_t)s->width * s->height * 4);
 }
@@ -1853,7 +1866,7 @@ extern "C" int mfx_film_import(MfxFilm *f, const double *sum, double frame_count
         MFX_TRY(ensure_frame_buffers(s));
         CUDA_TRY(cudaMemsetAsync(s->d_color_wh, 0, npx * 4 * sizeof(double), s->stream));
         // reuse Film.AddSample with a zero frame and the restored count: sum + 0, target = sum / count
-        mfx_film_add(s->stream, f->d_sum, s->d_color_wh, f->d_target, (long long)npx, frame_count);
+        mfx_film_add(s->stream, film_tilemap(s->width, s->height, 0, 0, 1), s->width, f->d_sum, s->d_color_wh, f->d_target, frame_count);
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaStreamSynchronize(s->stream));
     }

@@ -290,7 +290,8 @@ void mfx_h_extend_x(const LaunchCfg &, const SceneF &, const SceneX &, const Sce
 // totals[0] += sum counts[ext_lo..+ext_n), totals[1] += sum counts[sh_lo..+sh_n), totals[2] += counts[0]
 void mfx_accum_ray_totals(cudaStream_t, const int *counts, int ext_lo, int ext_n, int sh_lo, int sh_n,
                           unsigned long long *totals);
-void mfx_film_add(cudaStream_t, double *sum, const double *frame, double *target, long long n_pixels, double frame_count);
-void mfx_film_tonemap(cudaStream_t, const double *target_wh, int width, int height, uint8_t *rgba8);
-void mfx_film_display_sky(cudaStream_t, const double *target_wh, int width, int height, uint8_t *rgba8);
+// Film kernels over the pixels tm owns (column stripes; one stripe of the frame's width = the whole frame)
+void mfx_film_add(cudaStream_t, TileMap tm, int width, double *sum, const double *frame, double *target, double frame_count);
+void mfx_film_tonemap(cudaStream_t, TileMap tm, int width, const double *target_wh, uint8_t *rgba8);
+void mfx_film_display_sky(cudaStream_t, TileMap tm, int width, const double *target_wh, uint8_t *rgba8);
 void mfx_fill_zero_f64(cudaStream_t, double *p, long long n);

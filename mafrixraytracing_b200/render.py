@@ -13,7 +13,7 @@ import sys
 
 import numpy as np
 
-from . import Scene, CudaPixelIntegrator, Film, EXACT_F64, FAST_F32
+from . import Scene, CudaPixelIntegrator, Film, MultiGpuPixelIntegrator, MultiGpuFilm, EXACT_F64, FAST_F32
 from .imageio import texture_to_rows, write_pfm, write_png
 from .ingest import init_scene_state
 
@@ -28,6 +28,7 @@ def main(argv=None):
     ap.add_argument("--exact", action="store_true", help="MFX_EXACT_F64 instead of MFX_FAST_F32")
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--out", default="frame")
+    ap.add_argument("--gpus", type=int, default=None, help="the same loop over the first N devices (MultiGpuFilm)")
     a = ap.parse_args(argv)
     sky = (a.scene == "sphere-sample")
     if sky:
@@ -36,12 +37,22 @@ def main(argv=None):
     else:
         with open(a.scene, "r", encoding="utf-8-sig") as fh:
             desc = init_scene_state(fh.read(), base_dir=os.path.dirname(os.path.abspath(a.scene)))
-    scene = Scene(desc)
-    integ = CudaPixelIntegrator(scene, precision=EXACT_F64 if a.exact else FAST_F32, seed=a.seed)
-    film = Film(scene)
+    precision = EXACT_F64 if a.exact else FAST_F32
+    if a.gpus:                          # one host thread, N devices: each keeps the Film of its own stripes
+        scene = integ = MultiGpuPixelIntegrator(desc, n_devices=a.gpus, precision=precision, seed=a.seed)
+        if integ.n_devices < a.gpus:
+            integ.close()
+            raise SystemExit(f"--gpus {a.gpus} but {integ.n_devices} device(s) visible")
+        film = MultiGpuFilm(integ)
+        get_frame = lambda f: film.GetFrame(a.spp, first_sample=f * a.spp, download=(f + 1 == a.frames))
+    else:
+        scene = Scene(desc)
+        integ = CudaPixelIntegrator(scene, precision=precision, seed=a.seed)
+        film = Film(scene)
+        get_frame = lambda f: film.GetFrame(integ, a.spp, first_sample=f * a.spp)
     rays = ms = 0.0
     for f in range(a.frames):
-        target = film.GetFrame(integ, a.spp, first_sample=f * a.spp)
+        target = get_frame(f)
         rays += integ.stats["closest_rays"] + integ.stats["shadow_rays"]
         ms += integ.stats["ms_total"]
     rows = texture_to_rows(target)[:, :, :3].astype(np.float32)

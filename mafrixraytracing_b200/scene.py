@@ -403,9 +403,12 @@ class MultiGpuPixelIntegrator:
         self.n_devices = n.value
         self.texture = np.zeros((self.width, self.height, 4), dtype=np.float64)
         self.stats = None
+        self._films = weakref.WeakSet()
 
     def close(self):
         if getattr(self, "_h", None):
+            for f in list(getattr(self, "_films", ())):      # mfx_multi_destroy refuses while a film of the handle lives
+                f.close()
             _lib.load().mfx_multi_destroy(self._h)
             self._h = None
 
@@ -504,4 +507,68 @@ class Film:
         """Scene.PostProcessAndToScreenBuffer (Scene.fs:315-330) -> (height, width, 4) uint8."""
         out = np.zeros((self.scene.height, self.scene.width, 4), dtype=np.uint8)
         _lib.check(_lib.load().mfx_film_post_process(self._h, _lib.ptr(out)))
+        return out
+
+
+class MultiGpuFilm:
+    """Film over several GPUs (mfx_multi_film_*): every device of `multi` accumulates, divides and tone-maps its own
+    column stripes in its own HBM.  Same surface and the same results, bit for bit, as Film on one GPU."""
+
+    def __init__(self, multi: MultiGpuPixelIntegrator):
+        self.multi = multi
+        h = C.c_void_p()
+        _lib.check(_lib.load().mfx_multi_film_create(multi._h, C.byref(h)))
+        self._h = h
+        multi._films.add(self)
+        self.target = np.zeros((multi.width, multi.height, 4), dtype=np.float64)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            _lib.load().mfx_multi_film_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def Reset(self):
+        _lib.check(_lib.load().mfx_multi_film_reset(self._h))
+
+    def FrameCount(self):
+        fc = C.c_double()
+        _lib.check(_lib.load().mfx_multi_film_frame_count(self._h, C.byref(fc)))
+        return fc.value
+
+    def GetFrame(self, samples, first_sample=None, download=True):
+        """Film.GetFrame over every device -> target as Color[w,h]; download=False keeps it on the devices (a host that
+        only displays calls PostProcess next) and returns None."""
+        if first_sample is None:
+            first_sample = int(self.FrameCount()) * int(samples)     # fresh samples every frame
+        m = self.multi
+        p = _lib.MfxSampleParams(m.precision, int(samples), m.seed, int(first_sample), 0, 0, 1, 0)
+        _lib.check(_lib.load().mfx_multi_film_get_frame(self._h, C.byref(p), _lib.ptr(self.target) if download else None))
+        m._after()
+        return self.target if download else None
+
+    def Export(self):
+        """Checkpoint: (running sum Color[w,h], frameCount), the same as Film.Export."""
+        s = np.zeros((self.multi.width, self.multi.height, 4), dtype=np.float64)
+        fc = C.c_double()
+        _lib.check(_lib.load().mfx_multi_film_export(self._h, _lib.ptr(s), C.byref(fc)))
+        return s, fc.value
+
+    def Import(self, sum_wh, frame_count):
+        sum_wh = np.ascontiguousarray(sum_wh, dtype=np.float64)
+        want = (self.multi.width, self.multi.height, 4)
+        if sum_wh.shape != want:
+            raise ValueError(f"MultiGpuFilm.Import: running sum has shape {sum_wh.shape}, the film is Color[w,h] = {want}")
+        _lib.check(_lib.load().mfx_multi_film_import(self._h, _lib.ptr(sum_wh), float(frame_count)))
+
+    def PostProcess(self, out=None):
+        """Scene.PostProcessAndToScreenBuffer (Scene.fs:315-330) -> (height, width, 4) uint8."""
+        if out is None:
+            out = np.zeros((self.multi.height, self.multi.width, 4), dtype=np.uint8)
+        _lib.check(_lib.load().mfx_multi_film_post_process(self._h, _lib.ptr(out)))
         return out
