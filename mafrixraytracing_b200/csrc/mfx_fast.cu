@@ -1012,11 +1012,6 @@ __global__ void __launch_bounds__(256) k_film_display_sky(TileMap tm, int width,
     }
 }
 
-__global__ void __launch_bounds__(256) k_fill_zero(double *p, long long n)
-{
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) p[i] = 0.;
-}
-
 // ---------------------------------------------------------------- launchers
 void mfx_f_raygen(const LaunchCfg &c, const SceneF &sc, const WaveF &w, TileMap tm, int pix0, int npix, int s0, int S, uint64_t seed)
 {
@@ -1107,8 +1102,4 @@ void mfx_film_tonemap(cudaStream_t s, TileMap tm, int width, const double *targe
 void mfx_film_display_sky(cudaStream_t s, TileMap tm, int width, const double *target_wh, uint8_t *rgba8)
 {
     k_film_display_sky<<<592, 256, 0, s>>>(tm, width, target_wh, rgba8);
-}
-void mfx_fill_zero_f64(cudaStream_t s, double *p, long long n)
-{
-    k_fill_zero<<<592, 256, 0, s>>>(p, n);
 }

@@ -1101,6 +1101,18 @@ static int stripe_pixels(int width, int height, int stripe, int rank, int world)
     return (int)n;
 }
 
+// The pixels of `rank`'s column stripes out of `world`; world 1 = the whole frame (pixel_of's identity).
+static TileMap stripe_tilemap(int width, int height, int stripe, int rank, int world)
+{
+    TileMap tm;
+    memset(&tm, 0, sizeof(tm));
+    tm.height = height;
+    if (world <= 1) { tm.n_pix = width * height; return tm; }
+    tm.stripe = stripe; tm.rank = rank; tm.world = world;
+    tm.n_pix = stripe_pixels(width, height, stripe, rank, world);
+    return tm;
+}
+
 // The stripe rule as a table (same local order as pixel_of computes on the device): for hosts and tests.
 extern "C" int mfx_stripe_map(int32_t width, int32_t height, int32_t stripe, int32_t rank, int32_t world,
                               int32_t *pixels_out, int32_t *n_out)
@@ -1132,8 +1144,7 @@ static int get_tilemap(MfxScene *s, int tile, int rank, int world, bool stripes,
         return MFX_OK;
     }
     if (stripes) {
-        tm->stripe = tile; tm->rank = rank; tm->world = world;
-        tm->n_pix = stripe_pixels(s->width, s->height, tile, rank, world);
+        *tm = stripe_tilemap(s->width, s->height, tile, rank, world);
         return MFX_OK;
     }
     auto key = std::make_tuple(tile, rank, world);
@@ -1742,50 +1753,93 @@ extern "C" int mfx_trace_primary(MfxScene *s, int32_t precision, int64_t n, cons
 }
 
 // ------------------------------------------------------------------ Film (Film.fs:13-34)
+// One device's film.  The steps below touch the pixels `tm` owns: the whole frame for mfx_film_*, a device's column
+// stripes for mfx_multi_film_*.  The buffers are not in the scene's buffer pool (dev_alloc): an mfx_multi_sample_async may
+// be growing a replica's pool list on its worker thread while the caller destroys a film.
+struct FilmBuffers {
+    double *d_sum = nullptr, *d_target = nullptr;   // Color[w,h], x-major
+    uint8_t *d_rgba8 = nullptr;                     // row-major
+};
+
 struct MfxFilm {
     MfxScene *scene;
-    double *d_sum = nullptr, *d_target = nullptr;   // Color[w,h]
-    uint8_t *d_rgba8 = nullptr;
+    FilmBuffers buf;
     double frame_count = 0.;
 };
 
-// The pixels a film kernel works on: `rank`'s column stripes out of `world`; world 1 = the whole frame (pixel_of's identity).
-static TileMap film_tilemap(int width, int height, int stripe, int rank, int world)
+static void film_free(MfxScene *s, FilmBuffers &b)
 {
-    TileMap tm;
-    memset(&tm, 0, sizeof(tm));
-    tm.height = height;
-    if (world <= 1) { tm.n_pix = width * height; return tm; }
-    tm.stripe = stripe; tm.rank = rank; tm.world = world;
-    tm.n_pix = stripe_pixels(width, height, stripe, rank, world);
-    return tm;
+    cudaSetDevice(s->device);
+    cudaFree(b.d_sum); cudaFree(b.d_target); cudaFree(b.d_rgba8);
+    b = FilmBuffers();
+}
+
+static int film_alloc(MfxScene *s, FilmBuffers &b)
+{
+    MFX_TRY(bind_device(s->device));
+    const size_t npx = (size_t)s->width * s->height;
+    auto alloc3 = [&]() {
+        return cudaMalloc(&b.d_sum, 4 * npx * sizeof(double)) == cudaSuccess && cudaMalloc(&b.d_target, 4 * npx * sizeof(double)) == cudaSuccess &&
+               cudaMalloc(&b.d_rgba8, 4 * npx) == cudaSuccess;
+    };
+    if (alloc3()) return MFX_OK;
+    cudaGetLastError();     // memory parked in the buffer pool is not in use: give it back and retry once
+    film_free(s, b);
+    pool_trim(s->device);
+    if (alloc3()) return MFX_OK;
+    cudaGetLastError();
+    film_free(s, b);
+    return fail(MFX_ERR_OUT_OF_MEMORY, "film allocation failed");
+}
+
+static int film_reset(MfxScene *s, const FilmBuffers &b)
+{
+    const size_t bytes = (size_t)s->width * s->height * 4 * sizeof(double);
+    CUDA_TRY(cudaMemsetAsync(b.d_sum, 0, bytes, s->stream));
+    CUDA_TRY(cudaMemsetAsync(b.d_target, 0, bytes, s->stream));
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    return MFX_OK;
+}
+
+// Film.GetFrame (Film.fs:18-23): one Sample into the scene's Color[w,h], then sum += frame, target = sum / frame_count
+static int film_frame(MfxScene *s, const TileMap &tm, const FilmBuffers &b, const MfxSampleParams *p, double frame_count)
+{
+    MFX_TRY(ensure_frame_buffers(s));
+    MFX_TRY(run_sample(s, p, s->d_color_wh, nullptr));
+    mfx_film_add(s->stream, tm, s->width, b.d_sum, s->d_color_wh, b.d_target, frame_count);
+    CUDA_TRY(cudaGetLastError());
+    return MFX_OK;
+}
+
+// ACES (Scene.fs:315-330), or under MFX_SKY_TRACER the sphere sample's sqrt(c) flipped vertically (RayTracing.fs:456-460)
+static int film_screen(MfxScene *s, const TileMap &tm, const FilmBuffers &b)
+{
+    if (s->integrator == MFX_SKY_TRACER) mfx_film_display_sky(s->stream, tm, s->width, b.d_target, b.d_rgba8);
+    else mfx_film_tonemap(s->stream, tm, s->width, b.d_target, b.d_rgba8);
+    CUDA_TRY(cudaGetLastError());
+    return MFX_OK;
+}
+
+// target = sum / frameCount (Film.fs:23) after an import: Film.AddSample of a zero frame with the restored count
+static int film_retarget(MfxScene *s, const TileMap &tm, const FilmBuffers &b, double frame_count)
+{
+    if (frame_count > 0.) {
+        MFX_TRY(ensure_frame_buffers(s));
+        CUDA_TRY(cudaMemsetAsync(s->d_color_wh, 0, (size_t)s->width * s->height * 4 * sizeof(double), s->stream));
+        mfx_film_add(s->stream, tm, s->width, b.d_sum, s->d_color_wh, b.d_target, frame_count);
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaStreamSynchronize(s->stream));
+    }
+    return MFX_OK;
 }
 
 extern "C" int mfx_film_create(MfxScene *s, MfxFilm **out)
 {
     if (!s || !out) return fail(MFX_ERR_INVALID_ARGUMENT, "null argument");
-    MFX_TRY(bind_device(s->device));
-    MfxFilm *f = new MfxFilm();
-    f->scene = s;
-    const size_t npx = (size_t)s->width * s->height;
-    auto alloc3 = [&]() {
-        return cudaMalloc(&f->d_sum, 4 * npx * sizeof(double)) == cudaSuccess && cudaMalloc(&f->d_target, 4 * npx * sizeof(double)) == cudaSuccess &&
-               cudaMalloc(&f->d_rgba8, 4 * npx) == cudaSuccess;
-    };
-    bool ok = alloc3();
-    if (!ok) {      // memory parked in the buffer pool is not in use: give it back and retry once
-        cudaGetLastError();
-        cudaFree(f->d_sum); cudaFree(f->d_target); cudaFree(f->d_rgba8); f->d_sum = f->d_target = nullptr; f->d_rgba8 = nullptr;
-        pool_trim(s->device);
-        ok = alloc3();
-    }
-    if (!ok) {
-        cudaGetLastError();
-        cudaFree(f->d_sum); cudaFree(f->d_target); cudaFree(f->d_rgba8); delete f;
-        return fail(MFX_ERR_OUT_OF_MEMORY, "film allocation failed");
-    }
-    *out = f;
-    return mfx_film_reset(f);
+    FilmBuffers b;
+    MFX_TRY(film_alloc(s, b));
+    *out = new MfxFilm{ s, b };
+    return mfx_film_reset(*out);
 }
 
 extern "C" int mfx_film_destroy(MfxFilm *f)
@@ -1793,7 +1847,7 @@ extern "C" int mfx_film_destroy(MfxFilm *f)
     if (!f) return MFX_OK;
     cudaSetDevice(f->scene->device);
     cudaStreamSynchronize(f->scene->stream);
-    cudaFree(f->d_sum); cudaFree(f->d_target); cudaFree(f->d_rgba8);
+    film_free(f->scene, f->buf);
     delete f;
     return MFX_OK;
 }
@@ -1802,25 +1856,18 @@ extern "C" int mfx_film_reset(MfxFilm *f)                      // Film.Reset, Fi
 {
     if (!f) return fail(MFX_ERR_INVALID_ARGUMENT, "null film");
     MFX_TRY(bind_device(f->scene->device));
-    const size_t npx = (size_t)f->scene->width * f->scene->height;
     f->frame_count = 0.;
-    CUDA_TRY(cudaMemsetAsync(f->d_sum, 0, 4 * npx * sizeof(double), f->scene->stream));
-    CUDA_TRY(cudaMemsetAsync(f->d_target, 0, 4 * npx * sizeof(double), f->scene->stream));
-    CUDA_TRY(cudaStreamSynchronize(f->scene->stream));
-    return MFX_OK;
+    return film_reset(f->scene, f->buf);
 }
 
 extern "C" int mfx_film_get_frame(MfxFilm *f, const MfxSampleParams *p, double *texture)   // Film.fs:18-23,32-34
 {
     if (!f || !p) return fail(MFX_ERR_INVALID_ARGUMENT, "null argument");
     MfxScene *s = f->scene;
-    MFX_TRY(bind_device(f->scene->device)); MFX_TRY(ensure_frame_buffers(s));
-    MFX_TRY(run_sample(s, p, s->d_color_wh, nullptr));
+    MFX_TRY(bind_device(s->device));
+    MFX_TRY(film_frame(s, stripe_tilemap(s->width, s->height, 0, 0, 1), f->buf, p, f->frame_count + 1.));
     f->frame_count += 1.;
-    const size_t npx = (size_t)s->width * s->height;
-    mfx_film_add(s->stream, film_tilemap(s->width, s->height, 0, 0, 1), s->width, f->d_sum, s->d_color_wh, f->d_target, f->frame_count);
-    CUDA_TRY(cudaGetLastError());
-    if (texture) return copy_out(s, texture, f->d_target, npx * 4 * sizeof(double));
+    if (texture) return copy_out(s, texture, f->buf.d_target, (size_t)s->width * s->height * 4 * sizeof(double));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
     return MFX_OK;
 }
@@ -1829,13 +1876,9 @@ extern "C" int mfx_film_post_process(MfxFilm *f, uint8_t *rgba8)   // Scene.fs:3
 {
     if (!f || !rgba8) return fail(MFX_ERR_INVALID_ARGUMENT, "null argument");
     MfxScene *s = f->scene;
-    MFX_TRY(bind_device(f->scene->device));
-    // MFX_SKY_TRACER: the sphere sample shows sqrt(c) flipped vertically (RayTracing.fs:456-460), no ACES curve
-    const TileMap tm = film_tilemap(s->width, s->height, 0, 0, 1);
-    if (s->integrator == MFX_SKY_TRACER) mfx_film_display_sky(s->stream, tm, s->width, f->d_target, f->d_rgba8);
-    else mfx_film_tonemap(s->stream, tm, s->width, f->d_target, f->d_rgba8);
-    CUDA_TRY(cudaGetLastError());
-    return copy_out(s, rgba8, f->d_rgba8, (size_t)s->width * s->height * 4);
+    MFX_TRY(bind_device(s->device));
+    MFX_TRY(film_screen(s, stripe_tilemap(s->width, s->height, 0, 0, 1), f->buf));
+    return copy_out(s, rgba8, f->buf.d_rgba8, (size_t)s->width * s->height * 4);
 }
 
 extern "C" int mfx_film_frame_count(const MfxFilm *f, double *out)
@@ -1850,27 +1893,18 @@ extern "C" int mfx_film_export(MfxFilm *f, double *sum, double *frame_count)
     if (!f || !sum || !frame_count) return fail(MFX_ERR_INVALID_ARGUMENT, "null argument");
     MFX_TRY(bind_device(f->scene->device));
     *frame_count = f->frame_count;
-    return copy_out(f->scene, sum, f->d_sum, (size_t)f->scene->width * f->scene->height * 4 * sizeof(double));
+    return copy_out(f->scene, sum, f->buf.d_sum, (size_t)f->scene->width * f->scene->height * 4 * sizeof(double));
 }
 
 extern "C" int mfx_film_import(MfxFilm *f, const double *sum, double frame_count)
 {
     if (!f || !sum || frame_count < 0.) return fail(MFX_ERR_INVALID_ARGUMENT, "bad argument");
-    MFX_TRY(bind_device(f->scene->device));
     MfxScene *s = f->scene;
-    const size_t npx = (size_t)s->width * s->height;
-    CUDA_TRY(cudaMemcpyAsync(f->d_sum, sum, npx * 4 * sizeof(double), cudaMemcpyHostToDevice, s->stream));
+    MFX_TRY(bind_device(s->device));
+    CUDA_TRY(cudaMemcpyAsync(f->buf.d_sum, sum, (size_t)s->width * s->height * 4 * sizeof(double), cudaMemcpyHostToDevice, s->stream));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
     f->frame_count = frame_count;
-    if (frame_count > 0.) {   // target = sum / frameCount (Film.fs:23)
-        MFX_TRY(ensure_frame_buffers(s));
-        CUDA_TRY(cudaMemsetAsync(s->d_color_wh, 0, npx * 4 * sizeof(double), s->stream));
-        // reuse Film.AddSample with a zero frame and the restored count: sum + 0, target = sum / count
-        mfx_film_add(s->stream, film_tilemap(s->width, s->height, 0, 0, 1), s->width, f->d_sum, s->d_color_wh, f->d_target, frame_count);
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaStreamSynchronize(s->stream));
-    }
-    return MFX_OK;
+    return film_retarget(s, stripe_tilemap(s->width, s->height, 0, 0, 1), f->buf, frame_count);
 }
 
 #include "mfx_multi.inl"

@@ -294,4 +294,3 @@ void mfx_accum_ray_totals(cudaStream_t, const int *counts, int ext_lo, int ext_n
 void mfx_film_add(cudaStream_t, TileMap tm, int width, double *sum, const double *frame, double *target, double frame_count);
 void mfx_film_tonemap(cudaStream_t, TileMap tm, int width, const double *target_wh, uint8_t *rgba8);
 void mfx_film_display_sky(cudaStream_t, TileMap tm, int width, const double *target_wh, uint8_t *rgba8);
-void mfx_fill_zero_f64(cudaStream_t, double *p, long long n);

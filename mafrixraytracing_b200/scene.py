@@ -454,20 +454,27 @@ class MultiGpuPixelIntegrator:
         return img
 
 
-class Film:
-    """Film (Film.fs:13-34): sum += frame; target = sum / frameCount -- kept in HBM."""
+class _FilmBase:
+    """What Film and MultiGpuFilm share: sum += frame; target = sum / frameCount, kept in HBM.  `_c` is the prefix of the
+    subclass's C functions; `owner` is the Scene or MultiGpuPixelIntegrator the film lives on, whose close() closes the
+    film first."""
 
-    def __init__(self, scene: Scene):
-        self.scene = scene
+    _c = None
+
+    def __init__(self, owner):
+        self._owner = owner
         h = C.c_void_p()
-        _lib.check(_lib.load().mfx_film_create(scene._h, C.byref(h)))
+        _lib.check(self._fn("create")(owner._h, C.byref(h)))
         self._h = h
-        scene._films.add(self)
-        self.target = np.zeros((scene.width, scene.height, 4), dtype=np.float64)
+        owner._films.add(self)
+        self.target = np.zeros((owner.width, owner.height, 4), dtype=np.float64)
+
+    def _fn(self, name):
+        return getattr(_lib.load(), f"{self._c}_{name}")
 
     def close(self):
         if getattr(self, "_h", None):
-            _lib.load().mfx_film_destroy(self._h)
+            self._fn("destroy")(self._h)
             self._h = None
 
     def __del__(self):
@@ -477,69 +484,62 @@ class Film:
             pass
 
     def Reset(self):
-        _lib.check(_lib.load().mfx_film_reset(self._h))
+        _lib.check(self._fn("reset")(self._h))
+
+    def FrameCount(self):
+        fc = C.c_double()
+        _lib.check(self._fn("frame_count")(self._h, C.byref(fc)))
+        return fc.value
+
+    def Export(self):
+        """Checkpoint: (running sum Color[w,h], frameCount) -- all the state Film carries (Film.fs:14-17)."""
+        s = np.zeros((self._owner.width, self._owner.height, 4), dtype=np.float64)
+        fc = C.c_double()
+        _lib.check(self._fn("export")(self._h, _lib.ptr(s), C.byref(fc)))
+        return s, fc.value
+
+    def Import(self, sum_wh, frame_count):
+        sum_wh = np.ascontiguousarray(sum_wh, dtype=np.float64)
+        want = (self._owner.width, self._owner.height, 4)
+        if sum_wh.shape != want:
+            raise ValueError(f"{type(self).__name__}.Import: running sum has shape {sum_wh.shape}, the film is Color[w,h] = {want}")
+        _lib.check(self._fn("import")(self._h, _lib.ptr(sum_wh), float(frame_count)))
+
+    def PostProcess(self, out=None):
+        """Scene.PostProcessAndToScreenBuffer (Scene.fs:315-330) -> (height, width, 4) uint8."""
+        if out is None:
+            out = np.zeros((self._owner.height, self._owner.width, 4), dtype=np.uint8)
+        _lib.check(self._fn("post_process")(self._h, _lib.ptr(out)))
+        return out
+
+
+class Film(_FilmBase):
+    """Film (Film.fs:13-34) on one GPU."""
+
+    _c = "mfx_film"
+
+    def __init__(self, scene: Scene):
+        self.scene = scene
+        super().__init__(scene)
 
     def GetFrame(self, integrator: CudaPixelIntegrator, samples, first_sample=None):
-        fc = C.c_double()
-        _lib.check(_lib.load().mfx_film_frame_count(self._h, C.byref(fc)))
         if first_sample is None:
-            first_sample = int(fc.value) * int(samples)     # fresh samples every frame
+            first_sample = int(self.FrameCount()) * int(samples)     # fresh samples every frame
         p = integrator._params(samples, first_sample)
         _lib.check(_lib.load().mfx_film_get_frame(self._h, C.byref(p), _lib.ptr(self.target)))
         integrator._after()
         return self.target
 
-    def Export(self):
-        """Checkpoint: (running sum Color[w,h], frameCount) -- all the state Film carries (Film.fs:14-17)."""
-        s = np.zeros((self.scene.width, self.scene.height, 4), dtype=np.float64)
-        fc = C.c_double()
-        _lib.check(_lib.load().mfx_film_export(self._h, _lib.ptr(s), C.byref(fc)))
-        return s, fc.value
 
-    def Import(self, sum_wh, frame_count):
-        sum_wh = np.ascontiguousarray(sum_wh, dtype=np.float64)
-        want = (self.scene.width, self.scene.height, 4)
-        if sum_wh.shape != want:
-            raise ValueError(f"Film.Import: running sum has shape {sum_wh.shape}, the film is Color[w,h] = {want}")
-        _lib.check(_lib.load().mfx_film_import(self._h, _lib.ptr(sum_wh), float(frame_count)))
-
-    def PostProcess(self):
-        """Scene.PostProcessAndToScreenBuffer (Scene.fs:315-330) -> (height, width, 4) uint8."""
-        out = np.zeros((self.scene.height, self.scene.width, 4), dtype=np.uint8)
-        _lib.check(_lib.load().mfx_film_post_process(self._h, _lib.ptr(out)))
-        return out
-
-
-class MultiGpuFilm:
+class MultiGpuFilm(_FilmBase):
     """Film over several GPUs (mfx_multi_film_*): every device of `multi` accumulates, divides and tone-maps its own
     column stripes in its own HBM.  Same surface and the same results, bit for bit, as Film on one GPU."""
 
+    _c = "mfx_multi_film"
+
     def __init__(self, multi: MultiGpuPixelIntegrator):
         self.multi = multi
-        h = C.c_void_p()
-        _lib.check(_lib.load().mfx_multi_film_create(multi._h, C.byref(h)))
-        self._h = h
-        multi._films.add(self)
-        self.target = np.zeros((multi.width, multi.height, 4), dtype=np.float64)
-
-    def close(self):
-        if getattr(self, "_h", None):
-            _lib.load().mfx_multi_film_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def Reset(self):
-        _lib.check(_lib.load().mfx_multi_film_reset(self._h))
-
-    def FrameCount(self):
-        fc = C.c_double()
-        _lib.check(_lib.load().mfx_multi_film_frame_count(self._h, C.byref(fc)))
-        return fc.value
+        super().__init__(multi)
 
     def GetFrame(self, samples, first_sample=None, download=True):
         """Film.GetFrame over every device -> target as Color[w,h]; download=False keeps it on the devices (a host that
@@ -551,24 +551,3 @@ class MultiGpuFilm:
         _lib.check(_lib.load().mfx_multi_film_get_frame(self._h, C.byref(p), _lib.ptr(self.target) if download else None))
         m._after()
         return self.target if download else None
-
-    def Export(self):
-        """Checkpoint: (running sum Color[w,h], frameCount), the same as Film.Export."""
-        s = np.zeros((self.multi.width, self.multi.height, 4), dtype=np.float64)
-        fc = C.c_double()
-        _lib.check(_lib.load().mfx_multi_film_export(self._h, _lib.ptr(s), C.byref(fc)))
-        return s, fc.value
-
-    def Import(self, sum_wh, frame_count):
-        sum_wh = np.ascontiguousarray(sum_wh, dtype=np.float64)
-        want = (self.multi.width, self.multi.height, 4)
-        if sum_wh.shape != want:
-            raise ValueError(f"MultiGpuFilm.Import: running sum has shape {sum_wh.shape}, the film is Color[w,h] = {want}")
-        _lib.check(_lib.load().mfx_multi_film_import(self._h, _lib.ptr(sum_wh), float(frame_count)))
-
-    def PostProcess(self, out=None):
-        """Scene.PostProcessAndToScreenBuffer (Scene.fs:315-330) -> (height, width, 4) uint8."""
-        if out is None:
-            out = np.zeros((self.multi.height, self.multi.width, 4), dtype=np.uint8)
-        _lib.check(_lib.load().mfx_multi_film_post_process(self._h, _lib.ptr(out)))
-        return out
