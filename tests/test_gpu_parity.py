@@ -644,9 +644,9 @@ def test_wave_shrinks_when_the_gpu_is_nearly_full():
     assert np.allclose(got, want, rtol=1e-5, atol=1e-7)
 
 
-@pytest.mark.parametrize("n_tris", [1, 2, 3, 5, 9])
-def test_tiny_own_trees(n_tris):
-    """One-record trees with 1..4 leaves and the first two-level trees: fast ids must equal the oracle's."""
+def tiny_tree_scene(n_tris):
+    """n_tris random triangles on a 3-wide grid: one to nine of them give a one-record tree with 1..4 leaves (a
+    single-leaf root, empty links) or the first two-level trees."""
     rng = np.random.default_rng(n_tris)
     prims = make_prims(n_tris)
     for i in range(n_tris):
@@ -655,7 +655,15 @@ def test_tiny_own_trees(n_tris):
     mats = make_materials([("lambert", (0.7, 0.7, 0.7))])
     light = AreaLight(np.array([(-1, 3, 1), (-1, 3, -1), (1, 3, -1), (1, 3, 1)], float), (0, -1, 0), (10, 10, 10))
     cam = PinholeCamera((0, 0, 4), (0, 0, -1), 120.0, 1.0)
-    desc = SceneDesc(prims, mats, light, cam, 64, 64, 2, PATH_INTEGRATOR)
+    return SceneDesc(prims, mats, light, cam, 64, 64, 2, PATH_INTEGRATOR)
+
+
+@pytest.mark.parametrize("n_tris", [1, 2, 3, 5, 9])
+def test_tiny_own_trees(n_tris):
+    """One-record trees with 1..4 leaves and the first two-level trees: fast ids must equal the oracle's."""
+    rng = np.random.default_rng(n_tris)
+    rng.uniform(-0.45, 0.45, (n_tris, 3, 3))                # the draws tiny_tree_scene made: the same rays as before
+    desc = tiny_tree_scene(n_tris)
     s, o = Scene(desc), oracle.OracleScene(desc)
     uv = rng.random((20000, 2))
     op, ot = o.trace_primary(uv)
