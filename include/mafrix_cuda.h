@@ -243,6 +243,11 @@ MFX_API int mfx_scene_device_bytes(const MfxScene *scene, uint64_t *exact_bytes,
 MFX_API int mfx_bvh_hit(MfxScene *scene, int32_t precision, int32_t any_hit, int64_t n,
                         const double *origins, const double *dirs, double tmin, double tmax,
                         int32_t *prim, int32_t *sub, double *t);
+/* Bvh.Hit from a surface: as mfx_bvh_hit, but ray r starts on primitive src[r] (caller's index, -1 none) and is
+ * traced by the kernel bounces >= 1 and shadow rays use (k_f_trace6), never the id-exact kernel.  MFX_FAST_F32 only.
+ * src == NULL: no ray has a source. */
+MFX_API int mfx_bvh_hit_from(MfxScene *scene, int32_t any_hit, int64_t n, const double *origins, const double *dirs,
+                             const int32_t *src, double tmin, double tmax, int32_t *prim, int32_t *sub, double *t);
 /* cam.GetRay(u,v) (Camera.fs:134-139) + bvh.Hit(ray, 1e-6, 99999999.) (Integrators.fs:108).
  * uv == NULL: pixel centres, n == width*height, ray r = y*width+x. */
 MFX_API int mfx_trace_primary(MfxScene *scene, int32_t precision, int64_t n, const double *uv,

@@ -85,6 +85,7 @@ SYMBOLS = {
     "mfx_scene_get_bvh": (C.c_int, [_P, _P, _P]),
     "mfx_scene_device_bytes": (C.c_int, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "mfx_bvh_hit": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int64, _P, _P, C.c_double, C.c_double, _P, _P, _P]),
+    "mfx_bvh_hit_from": (C.c_int, [_P, C.c_int32, C.c_int64, _P, _P, _P, C.c_double, C.c_double, _P, _P, _P]),
     "mfx_trace_primary": (C.c_int, [_P, C.c_int32, C.c_int64, _P, _P, _P]),
     "mfx_pixel_integrator_sample": (C.c_int, [_P, C.POINTER(MfxSampleParams), _P]),
     "mfx_pixel_integrator_sample_async": (C.c_int, [_P, C.POINTER(MfxSampleParams), _P]),

@@ -881,12 +881,14 @@ __global__ void __launch_bounds__(256) k_f_resolve(SceneF sc, WaveF w, TileMap t
 }
 
 // Finer seams (Bvh.Hit, GetRay + Hit) routed through the PRODUCTION traversal kernel: rays are written
-// into the wave's queues, traced by k_f_trace6, and read back.
+// into the wave's queues, traced by k_f_trace6, and read back.  src (nullptr: none): per ray, the id the fast slots carry
+// for the primitive it starts on, or -1 -- what the shade kernels write into ray_o.w / sh_o.w.
 __global__ void __launch_bounds__(256) k_f_seam_setup(SceneF sc, WaveF w, int n, const double *o, const double *d, const double *uv,
-                                                      long long first, float tmax, int any_hit)
+                                                      const int *src, long long first, float tmax, int any_hit)
 {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const long long r = first + i;
+        const int sp = src ? src[r] : -1;
         F3 oo, dd;
         if (d) {
             oo = f3((float)o[3 * r], (float)o[3 * r + 1], (float)o[3 * r + 2]);
@@ -906,9 +908,9 @@ __global__ void __launch_bounds__(256) k_f_seam_setup(SceneF sc, WaveF w, int n,
             oo = f3(sc.cam.pos[0], sc.cam.pos[1], sc.cam.pos[2]);
             dd = camera_dir_f64(sc.camx, u, v);
         }
-        w.ray_o[0][i] = make_float4(oo.x, oo.y, oo.z, __int_as_float(-1));
+        w.ray_o[0][i] = make_float4(oo.x, oo.y, oo.z, __int_as_float(sp));
         w.ray_d[0][i] = make_float4(dd.x, dd.y, dd.z, __int_as_float(i));   // tMax of the closest query is w.tmax
-        w.sh_o[i] = make_float4(oo.x, oo.y, oo.z, __int_as_float(-1));
+        w.sh_o[i] = make_float4(oo.x, oo.y, oo.z, __int_as_float(sp));
         w.sh_d[i] = make_float4(dd.x, dd.y, dd.z, tmax + 1e-6f);      // the shadow kernel subtracts 1e-6 (Integrators.fs:44)
         w.sh_c[i] = make_float4(1.f, 0.f, 0.f, __int_as_float(i));    // unoccluded rays add this to rad[i]
         w.rad[i] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1079,9 +1081,9 @@ void mfx_f_resolve(const LaunchCfg &c, const SceneF &sc, const WaveF &w, TileMap
     k_f_resolve<<<persistent_blocks(k_f_resolve, 256, c.blocks), 256, 0, c.stream>>>(sc, w, tm, pix0, npix, S, pixsum);
 }
 void mfx_f_seam_setup(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int n, const double *o, const double *d, const double *uv,
-                      long long first, float tmax, int any_hit)
+                      const int *src, long long first, float tmax, int any_hit)
 {
-    k_f_seam_setup<<<persistent_blocks(k_f_seam_setup, 256, c.blocks), 256, 0, c.stream>>>(sc, w, n, o, d, uv, first, tmax, any_hit);
+    k_f_seam_setup<<<persistent_blocks(k_f_seam_setup, 256, c.blocks), 256, 0, c.stream>>>(sc, w, n, o, d, uv, src, first, tmax, any_hit);
 }
 void mfx_f_seam_read(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int n, long long first, int any_hit, int *prim, int *sub, double *t)
 {

@@ -1663,9 +1663,10 @@ static int with_ray_buffers(MfxScene *s, int64_t n, const double *a, size_t a_pe
 }
 
 // The fast-precision seams run the PRODUCTION wavefront traversal kernel: the rays go through the wave's
-// queues in chunks of its capacity (bounce 0, closest or shadow queue), exactly like rays of a frame.
+// queues in chunks of its capacity (bounce 0, closest or shadow queue), exactly like rays of a frame.  src (device, per
+// ray, nullptr: none): the slot id of the primitive the ray starts on, or -1.
 static void fast_seam(MfxScene *s, const SceneF *sfp, const LaunchCfg &cfg, int any_hit, int64_t n, const double *o, const double *d, const double *uv,
-                      float tmin, float tmax, int *prim, int *sub, double *t)
+                      const int *src, float tmin, float tmax, int *prim, int *sub, double *t)
 {
     WaveF w = s->wf;
     w.tmin = tmin;
@@ -1674,7 +1675,7 @@ static void fast_seam(MfxScene *s, const SceneF *sfp, const LaunchCfg &cfg, int 
     for (int64_t first = 0; first < n; first += w.P) {
         const int m = (int)std::min<int64_t>(w.P, n - first);
         cudaMemsetAsync(w.counts, 0, MFX_COUNTS_LEN * sizeof(int), s->stream);
-        mfx_f_seam_setup(cfg, *sfp, w, m, o, d, uv, first, tmax, any_hit);
+        mfx_f_seam_setup(cfg, *sfp, w, m, o, d, uv, src, first, tmax, any_hit);
         if (any_hit) mfx_f_shadow(cfg, *sfp, w, 0, nullptr); else mfx_f_extend(cfg, *sfp, w, 0, nullptr);
         mfx_f_seam_read(cfg, *sfp, w, m, first, any_hit, prim, sub, t);
     }
@@ -1719,10 +1720,41 @@ extern "C" int mfx_bvh_hit(MfxScene *s, int32_t precision, int32_t any_hit, int6
         if (hyb) { MFX_TRY(flatten_hybrid(s)); MFX_TRY(ensure_wave_hybrid(s)); }
         return with_ray_buffers(s, n, origins, 3, dirs, 3, prim, sub, t, [&](double *o, double *d, int *p, int *sb, double *tt) {
             if (hyb) hybrid_seam(s, sfp, cfg, n, o, d, nullptr, tmin, tmax, p, sb, tt);
-            else fast_seam(s, sfp, cfg, any_hit, n, o, d, nullptr, (float)tmin, (float)tmax, p, sb, tt);
+            else fast_seam(s, sfp, cfg, any_hit, n, o, d, nullptr, nullptr, (float)tmin, (float)tmax, p, sb, tt);
         });
     }
     return fail(MFX_ERR_INVALID_ARGUMENT, "unknown precision %d", precision);
+}
+
+// Rays that start on a surface, as the rays of bounces >= 1 and the shadow rays of a fast frame: always k_f_trace6 (the
+// id-exact kernel only ever traces bounce 0, whose rays have no source).
+extern "C" int mfx_bvh_hit_from(MfxScene *s, int32_t any_hit, int64_t n, const double *origins, const double *dirs, const int32_t *src,
+                                double tmin, double tmax, int32_t *prim, int32_t *sub, double *t)
+{
+    if (!s || !origins || !dirs || !prim || !t) return fail(MFX_ERR_INVALID_ARGUMENT, "mfx_bvh_hit_from: null argument");
+    if (n <= 0) return MFX_OK;
+    const int np = (int)s->prims.size();
+    if (src)
+        for (int64_t r = 0; r < n; r++)
+            if (src[r] < -1 || src[r] >= np) return fail(MFX_ERR_INVALID_ARGUMENT, "mfx_bvh_hit_from: src[%lld] = %d outside [-1, %d)", (long long)r, src[r], np);
+    MFX_TRY(bind_device(s->device));
+    LaunchCfg cfg{ s->sm_count, 128, s->stream, 0, 0 };
+    MFX_TRY(flatten_fast(s));
+    MFX_TRY(ensure_wave_fast(s, (size_t)n));
+    int *dsrc = nullptr;
+    if (src) {
+        // the id leaf_f3 compares with a ray's src is b.w of the primitive's slots without the half bit, and the own
+        // tree's slots carry the caller's index there (build_own_tree_host: make_fast_slots(prims[i], i, ..)), so the
+        // caller's indices go to the device as they are
+        cudaError_t e = cudaMalloc(&dsrc, (size_t)n * sizeof(int));
+        if (e == cudaSuccess) e = cudaMemcpyAsync(dsrc, src, (size_t)n * sizeof(int), cudaMemcpyHostToDevice, s->stream);
+        if (e != cudaSuccess) { cudaFree(dsrc); return fail(MFX_ERR_CUDA, "mfx_bvh_hit_from: source ids: %s", cudaGetErrorString(e)); }
+    }
+    const int rc = with_ray_buffers(s, n, origins, 3, dirs, 3, prim, sub, t, [&](double *o, double *d, int *p, int *sb, double *tt) {
+        fast_seam(s, &s->sf, cfg, any_hit, n, o, d, nullptr, dsrc, (float)tmin, (float)tmax, p, sb, tt);
+    });
+    cudaFree(dsrc);
+    return rc;
 }
 
 extern "C" int mfx_trace_primary(MfxScene *s, int32_t precision, int64_t n, const double *uv, int32_t *prim, double *t)
@@ -1746,7 +1778,7 @@ extern "C" int mfx_trace_primary(MfxScene *s, int32_t precision, int64_t n, cons
         return with_ray_buffers(s, n, uv, 2, nullptr, 0, prim, nullptr, t, [&](double *u, double *, int *p, int *, double *tt) {
             const bool sky = (s->integrator == MFX_SKY_TRACER);      // ListHit(ray, 0.00001, 10000000), RayTracing.fs:368
             if (hyb) { hybrid_seam(s, sfp, cfg, n, nullptr, nullptr, u, sky ? MFX_SKY_TMIN : 1e-6, sky ? MFX_SKY_TMAX : 99999999., p, nullptr, tt); return; }
-            fast_seam(s, sfp, cfg, 0, n, nullptr, nullptr, u, sky ? (float)MFX_SKY_TMIN : 1e-6f, sky ? (float)MFX_SKY_TMAX : 99999999.f, p, nullptr, tt);
+            fast_seam(s, sfp, cfg, 0, n, nullptr, nullptr, u, nullptr, sky ? (float)MFX_SKY_TMIN : 1e-6f, sky ? (float)MFX_SKY_TMAX : 99999999.f, p, nullptr, tt);
         });
     }
     return fail(MFX_ERR_INVALID_ARGUMENT, "unknown precision %d", precision);

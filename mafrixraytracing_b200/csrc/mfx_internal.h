@@ -268,7 +268,7 @@ void mfx_f_shade_sky(const LaunchCfg &, const SceneF &, const WaveF &, TileMap t
 void mfx_f_resolve(const LaunchCfg &, const SceneF &, const WaveF &, TileMap tm, int pix0, int npix, int S,
                    double *pixsum);
 void mfx_f_seam_setup(const LaunchCfg &, const SceneF &, const WaveF &, int n, const double *o, const double *d, const double *uv,
-                      long long first, float tmax, int any_hit);
+                      const int *src, long long first, float tmax, int any_hit);
 void mfx_f_seam_read(const LaunchCfg &, const SceneF &, const WaveF &, int n, long long first, int any_hit, int *prim, int *sub, double *t);
 
 // hybrid (mfx_hybrid.cu, --fmad=false): id-exact closest hits on the own tree

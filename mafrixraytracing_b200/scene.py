@@ -308,6 +308,21 @@ class Scene:
                                            float(tmin), float(tmax), _lib.ptr(prim), _lib.ptr(sub), _lib.ptr(t)))
         return prim, sub, t
 
+    def HitFrom(self, origins, dirs, src, tmin, tmax, any_hit=False):
+        """Bvh.Hit for n rays that start on primitive src[i] (-1: none; None: none at all), traced by the f32 kernel of
+        bounces >= 1 and shadow rays -> (prim, sub, t)."""
+        o = np.ascontiguousarray(origins, np.float64).reshape(-1, 3)
+        d = np.ascontiguousarray(dirs, np.float64).reshape(-1, 3)
+        n = len(o)
+        sp = None if src is None else np.ascontiguousarray(src, np.int32).reshape(n)
+        prim = np.full(n, -1, np.int32)
+        sub = np.zeros(n, np.int32)
+        t = np.zeros(n, np.float64)
+        _lib.check(_lib.load().mfx_bvh_hit_from(self._h, int(any_hit), n, _lib.ptr(o), _lib.ptr(d),
+                                                None if sp is None else _lib.ptr(sp), float(tmin), float(tmax),
+                                                _lib.ptr(prim), _lib.ptr(sub), _lib.ptr(t)))
+        return prim, sub, t
+
     def TracePrimary(self, uv=None, precision=EXACT_F64):
         """cam.GetRay(u,v) + bvh.Hit(ray,1e-6,99999999.) -> (prim, t); uv None = pixel centres (row-major)."""
         if uv is None:

@@ -1,5 +1,6 @@
 /* brute_hit.c -- brute-force f64 classifier of closest-hit and any-hit queries, for the f32 traversal tests
- * (tests/test_gpu_f32_traversal.py).  Test infrastructure only: no tree, every ray against every primitive.
+ * (tests/test_gpu_f32_traversal.py, and tests/test_gpu_f32_from_surface.py for rays that start on a primitive).  Test
+ * infrastructure only: no tree, every ray against every primitive.
  *
  * Semantics are those of the fast path (DESIGN.md 4.3, leaf_f3 in mfx_fast.cu), not the reference's quirks:
  *   - a triangle is Moller-Trumbore with leaf_f3's acceptance predicate: |div| >= 1e-6 absolute, b1 in [0,1],
@@ -8,7 +9,7 @@
  *   - a sphere solves Sphere.Hit's quadratic (a = 1: the direction is taken as a unit vector, so spheres are only
  *     queried with unit directions) and takes the near root if it lies in the window, otherwise the far root; big
  *     spheres (r >= 32, the kernel's f64 branch) get the same treatment;
- *   - no source primitive (the seams start every ray with src = -1).
+ *   - a ray may start on a source primitive (brute_classify_from, SOURCE RULES below); brute_classify has none.
  *
  * Every (ray, primitive) pair is a CLEAR HIT, a CLEAR MISS or AMBIGUOUS, with margins taken from the f32 kernel's error.
  * The kernel sees o, d, v0 (a sphere's centre) and the edges e1 = v1 - v0, e2 = v2 - v0 rounded to f32, 2^-24 relative
@@ -44,6 +45,33 @@
  *     before every other candidate (its least possible t) by at least 1e-4 t_w + u_w + u_j (coincident copies and
  *     shared Rect diagonals are therefore not robust);
  *   - any hit: occluded if a clear hit lies in the window, clear if there is no candidate at all.
+ *
+ * SOURCE RULES (leaf_f3: the rays of bounces >= 1 and the shadow rays start on the primitive they left, src = its index):
+ *   - a source triangle or Rect is a clear miss, both halves of a Rect (the kernel compares the id without the half
+ *     bit), a non-planar Rect included;
+ *   - a source sphere is decided by the sign of hb = (o - c).d (d a unit vector): the kernel skips it when its f32 hb
+ *     is >= 0 (leaving) and otherwise takes the far root, or the chord -2 hb when its f32 discriminant comes out <= 0.
+ *     The kernel's hb differs from the f64 one by the rounding of o and c (sqrt(3) 2^-24 (|o|_inf + |c|_inf)), of d
+ *     (sqrt(3) 2^-24 |o - c|, d unit), of the subtraction o - c (sqrt(3) 2^-24 |o - c|) and of the three products and
+ *     two sums of the dot product (3 2^-24 |o - c|): at most about 2^-24 (2 (|c|_inf + |o|_inf) + 7 |o - c|).  With a
+ *     factor of two to spare, in the constants of eps,
+ *         eps_h = 2^-24 (K_IN (|c|_inf + |o|_inf) + K_AR |o - c|),
+ *     and a big sphere (r >= 32, solved in f64 from its f64 centre) drops |c|_inf: only o and d are rounded there.
+ *       hb >= eps_h: clear miss (leaving);
+ *       hb <= -eps_h: the far root, when the f64 discriminant hb^2 - (|o - c|^2 - r^2) is within its rounding of 0
+ *         the chord -2 hb (on a point exactly on the surface the two are the same).  The kernel's t lies in
+ *           [max(t - u, |hb| - eps_h),  min(t + u, 2 (|hb| + eps_h) + sqrt(4 r eps_h))],
+ *         u = eps / (|d| cos) the t margin above (cos = sqrt(disc) / r at the far root, |hb| / r at the chord), and
+ *         the pair is classified by that interval (its centre and half-width stand for t and u).  The second bound
+ *         of each end holds whichever of the root or the chord fires: the far root -hb + sqrt(disc) is at least
+ *         |hb_f32| and the chord is 2 |hb_f32|, |hb_f32| >= |hb| - eps_h; the f32 discriminant is hb_f32^2 plus an
+ *         error delta -- the origin's distance from the surface (at most eps_h / 2, times 2 r), the error of the
+ *         perpendicular part of o - c (at most eps_h, times 2 r) and the roundings of r^2 and |perp|^2 (4 2^-24 r^2)
+ *         -- so |delta| <= 4 r eps_h and the root is at most 2 |hb_f32| + sqrt(4 r eps_h).  Near the tangent plane,
+ *         where u exceeds t and the kernel's chord fires (|hb| up to ~1e-3 r), an entering ray is therefore a clear
+ *         hit of its source once |hb| - eps_h clears tMin: the chord rule is held ray by ray;
+ *       |hb| < eps_h: ambiguous (skipped, or re-entered at a t anywhere from 0 to the f32 root's error), at tMin.
+ *   - every other pair is classified as without a source.
  */
 #include <math.h>
 #include <pthread.h>
@@ -70,6 +98,7 @@ typedef struct {
     const double *o, *d; int n;
     double tmin, tmax, max_abs;
     int any_hit, normalize;
+    const int32_t *src;             /* caller's index of the primitive ray i starts on, -1 none; NULL: none at all */
     int8_t *robust; int32_t *prim, *sub, *n_amb; double *t, *terr, *eps;
     int next; pthread_mutex_t mu;
 } Job;
@@ -155,6 +184,37 @@ static int classify_sphere(const BPrim *p, const double *o, const double *d, dou
     return MISS;
 }
 
+/* a sphere the ray starts on (SOURCE RULES in the header); eps_o = K_IN 2^-24 |o|_inf, the rounding of o alone */
+static int classify_src_sphere(const BPrim *p, const double *o, const double *d, double dl, double eps_in, double eps_o,
+                               double tmin, double tmax, double *t_out, double *u_out, double *eps_out)
+{
+    double oc[3];
+    for (int k = 0; k < 3; k++) oc[k] = o[k] - p->c[k];
+    const double oc2 = dot3(oc, oc), ocl = sqrt(oc2);
+    const double eps = eps_in + K_AR * ldexp(1.0, -24) * (ocl + 2.0 * p->size);
+    *eps_out = eps;
+    const double cmax = fmax(fabs(p->c[0]), fmax(fabs(p->c[1]), fabs(p->c[2])));
+    const double eps_h = eps_o + K_AR * ldexp(1.0, -24) * ocl + (p->r >= 32.0 ? 0.0 : K_IN * ldexp(1.0, -24) * cmax);
+    const double hb = dot3(oc, d);
+    if (hb >= eps_h) return MISS;                                           /* leaving */
+    if (hb > -eps_h) { *t_out = tmin; *u_out = 0.0; return AMB; }           /* along the tangent plane */
+    const double cc = oc2 - p->r * p->r, disc = hb * hb - cc;
+    double t, cosv;
+    if (disc <= 4.0 * ldexp(1.0, -52) * (hb * hb + oc2 + p->r * p->r)) { t = -2.0 * hb; cosv = -hb / (p->r * dl); }
+    else {
+        const double root = sqrt(disc), q = root - hb;                      /* hb < 0: q is the far root */
+        t = fmax(q, cc / q);
+        cosv = root / (p->r * dl);
+    }
+    const double u = eps / (dl * cosv);
+    const double lo = fmax(t - u, -hb - eps_h), hi = fmin(t + u, 2.0 * (eps_h - hb) + sqrt(4.0 * p->r * eps_h));
+    const double tc = 0.5 * (lo + hi), uc = 0.5 * (hi - lo);
+    *t_out = tc; *u_out = uc;
+    const int w = window(tc, uc + 1e-5 * tc, tmin, tmax);
+    if (w == -1 || w == 2) return MISS;
+    return w == 1 ? AMB : HIT;
+}
+
 static void classify_ray(Job *J, int i, Cand **buf, int *cap)
 {
     double d[3] = { J->d[3 * i], J->d[3 * i + 1], J->d[3 * i + 2] };
@@ -162,14 +222,17 @@ static void classify_ray(Job *J, int i, Cand **buf, int *cap)
     double dl = sqrt(dot3(d, d));
     if (J->normalize) { for (int k = 0; k < 3; k++) d[k] /= dl; dl = sqrt(dot3(d, d)); }
     const double omax = fmax(fabs(o[0]), fmax(fabs(o[1]), fabs(o[2])));
-    const double eps_in = K_IN * ldexp(1.0, -24) * (J->max_abs + omax);
+    const double eps_in = K_IN * ldexp(1.0, -24) * (J->max_abs + omax), eps_o = K_IN * ldexp(1.0, -24) * omax;
+    const int src = J->src ? J->src[i] : -1;
     int nc = 0, namb = 0, any_clear = 0;
     int wp = -1, ws = 0; double wt = INFINITY, wu = 0.0, weps = eps_in;
     for (int j = 0; j < J->np; j++) {
         const BPrim *p = J->p + j;
         double t = 0.0, u = 0.0, eps = 0.0;
-        const int c = p->sphere ? classify_sphere(p, o, d, dl, eps_in, J->tmin, J->tmax, &t, &u, &eps)
-                                : classify_tri(p, o, d, dl, eps_in, J->tmin, J->tmax, &t, &u, &eps);
+        int c;
+        if (p->prim == src) c = p->sphere ? classify_src_sphere(p, o, d, dl, eps_in, eps_o, J->tmin, J->tmax, &t, &u, &eps) : MISS;
+        else c = p->sphere ? classify_sphere(p, o, d, dl, eps_in, J->tmin, J->tmax, &t, &u, &eps)
+                           : classify_tri(p, o, d, dl, eps_in, J->tmin, J->tmax, &t, &u, &eps);
         if (c == MISS) continue;
         if (c == AMB) namb++;
         else {
@@ -233,10 +296,11 @@ static void set_tri(BPrim *b, const double *a, const double *p1, const double *p
  * window; any_hit selects the query; normalize: divide each direction by its length first (the sphere sample's Ray).
  * Out per ray: robust flag, expected (prim, sub, t) -- prim >= 0 means occluded for an any-hit query -- the allowed
  * |t_f32 - t| of a robust closest hit, eps of the nearest clear hit (of a ray without one: its first term) and the
- * number of ambiguous pairs.  Returns max_abs. */
-double brute_classify(int n_prims, const int32_t *kind, const double *v, int n, const double *o, const double *d,
-                      double tmin, double tmax, int any_hit, int normalize, int threads,
-                      int8_t *robust, int32_t *prim, int32_t *sub, double *t, double *terr, double *eps, int32_t *n_amb)
+ * number of ambiguous pairs.  src: per ray, the caller's index of the primitive it starts on or -1 (NULL: -1 for every
+ * ray); indices outside [0, n_prims) match no primitive.  Returns max_abs. */
+double brute_classify_from(int n_prims, const int32_t *kind, const double *v, int n, const double *o, const double *d,
+                           const int32_t *src, double tmin, double tmax, int any_hit, int normalize, int threads,
+                           int8_t *robust, int32_t *prim, int32_t *sub, double *t, double *terr, double *eps, int32_t *n_amb)
 {
     BPrim *P = (BPrim *)calloc((size_t)2 * n_prims + 1, sizeof(BPrim));
     int np = 0;
@@ -261,7 +325,7 @@ double brute_classify(int n_prims, const int32_t *kind, const double *v, int n, 
     Job J;
     memset(&J, 0, sizeof(J));
     J.p = P; J.np = np; J.o = o; J.d = d; J.n = n; J.tmin = tmin; J.tmax = tmax; J.max_abs = max_abs;
-    J.any_hit = any_hit; J.normalize = normalize;
+    J.any_hit = any_hit; J.normalize = normalize; J.src = src;
     J.robust = robust; J.prim = prim; J.sub = sub; J.t = t; J.terr = terr; J.eps = eps; J.n_amb = n_amb;
     pthread_mutex_init(&J.mu, NULL);
     if (threads < 1) threads = 1;
@@ -272,4 +336,13 @@ double brute_classify(int n_prims, const int32_t *kind, const double *v, int n, 
     pthread_mutex_destroy(&J.mu);
     free(P);
     return max_abs;
+}
+
+/* the rays of brute_classify_from without a source primitive */
+double brute_classify(int n_prims, const int32_t *kind, const double *v, int n, const double *o, const double *d,
+                      double tmin, double tmax, int any_hit, int normalize, int threads,
+                      int8_t *robust, int32_t *prim, int32_t *sub, double *t, double *terr, double *eps, int32_t *n_amb)
+{
+    return brute_classify_from(n_prims, kind, v, n, o, d, NULL, tmin, tmax, any_hit, normalize, threads,
+                               robust, prim, sub, t, terr, eps, n_amb);
 }
