@@ -189,7 +189,6 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
     extern __shared__ float s_dyn[];
     float *lvl_entry = s_dyn + threadIdx.x;
     const unsigned FULL = 0xffffffffu;
-    const unsigned lane = threadIdx.x & 31u;
     const int n = ANY ? w.counts[CNT_SH(bounce)] : w.counts[bounce];
     const float4 *ro = ANY ? w.sh_o : w.ray_o[bounce & 1], *rd = ANY ? w.sh_d : w.ray_d[bounce & 1];
     int *cursor = &w.counts[ANY ? CUR_SH(bounce) : CUR_EXT(bounce)];
@@ -205,34 +204,21 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
     unsigned iters = 0u;
 
     for (;;) {
-        const unsigned idle = __ballot_sync(FULL, pid < 0);
-        unsigned idle_now = idle;
-        if (++iters > (1u << 22)) { if (lane == 0) atomicAdd(&w.counts[MFX_COUNTS_LEN - 1], 1); break; }   // watchdog
-        if (!exhausted && __popc(idle) >= TRACE4_REFILL_T) {
-            const int nidle = __popc(idle);
-            int base = 0;
-            if (lane == 0) base = atomicAdd(cursor, nidle);
-            base = __shfl_sync(FULL, base, 0);
-            if (base + nidle >= n) exhausted = true;
-            if (pid < 0) {
-                const int idx = base + __popc(idle & ((1u << lane) - 1u));
-                if (idx < n) {
-                    pid = idx;                                          // the ray lives at its queue position
-                    const float4 o = ro[pid];
-                    const float4 d = rd[pid];
-                    r = make_ray_fast(f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), w.tmin, __float_as_int(o.w));
-                    best_t = ANY ? d.w - 1e-6f : w.tmax;                // shadow: dist - 1e-6 (Integrators.fs:44); closest: tMax (:108)
-                    best_slot = -1; pend = 0u; leafA = leafB = -1; h = 1u; depth = 0u;
-                    float e;
-                    local[0]++;
-                    const bool in = box_f(r, sc.root_min[0], sc.root_min[1], sc.root_min[2], sc.root_max[0], sc.root_max[1], sc.root_max[2], best_t, e);
-                    needPop = !in || sc.root_meta >= 0;     // nothing to descend into: the (empty) trail pop ends the ray
-                    if (in && sc.root_meta >= 0) leafA = sc.root_meta;
-                }
-            }
-            idle_now = __ballot_sync(FULL, pid < 0);
-        }
-        if (idle_now == FULL) { if (exhausted) break; continue; }
+        unsigned idle = __ballot_sync(FULL, pid < 0);
+        if (watchdog_tripped(iters, 1u << 22, w.counts)) break;
+        idle = warp_refill(idle, TRACE4_REFILL_T, cursor, n, exhausted, pid, [&] {       // the ray lives at its queue position
+            const float4 o = ro[pid];
+            const float4 d = rd[pid];
+            r = make_ray_fast(f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), w.tmin, __float_as_int(o.w));
+            best_t = ANY ? d.w - 1e-6f : w.tmax;                // shadow: dist - 1e-6 (Integrators.fs:44); closest: tMax (:108)
+            best_slot = -1; pend = 0u; leafA = leafB = -1; h = 1u; depth = 0u;
+            float e;
+            local[0]++;
+            const bool in = box_f(r, sc.root_min[0], sc.root_min[1], sc.root_min[2], sc.root_max[0], sc.root_max[1], sc.root_max[2], best_t, e);
+            needPop = !in || sc.root_meta >= 0;     // nothing to descend into: the (empty) trail pop ends the ray
+            if (in && sc.root_meta >= 0) leafA = sc.root_meta;
+        });
+        if (idle == FULL) { if (exhausted) break; continue; }
 
         // ---- node step(s) (lanes holding a node to visit and no parked leaves); TRACE4_NSTEP > 1 amortises the
         //      loop skeleton (ballots, vote, refill test) over several tree levels
@@ -264,16 +250,12 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
         }
         // ---- leaf phase by vote
         bool finished = false;
-        const unsigned lp = __ballot_sync(FULL, pid >= 0 && leafA >= 0);
-        if (lp) {
-            const unsigned nd = ~idle_now & ~lp;
-            if (__popc(lp) >= TRACE4_LEAF_T || nd == 0u) {
-                if (pid >= 0 && leafA >= 0) {
-                    bool found = leaf_f3<true, BIG>(sc, r, leafA, best_t, best_slot, local);
-                    if (leafB >= 0 && !(ANY && found) && eB <= best_t) found |= leaf_f3<true, BIG>(sc, r, leafB, best_t, best_slot, local);
-                    leafA = leafB = -1;
-                    if (ANY && found) finished = true;
-                }
+        if (leaf_vote(__ballot_sync(FULL, pid >= 0 && leafA >= 0), idle, TRACE4_LEAF_T)) {
+            if (pid >= 0 && leafA >= 0) {
+                bool found = leaf_f3<true, BIG>(sc, r, leafA, best_t, best_slot, local);
+                if (leafB >= 0 && !(ANY && found) && eB <= best_t) found |= leaf_f3<true, BIG>(sc, r, leafB, best_t, best_slot, local);
+                leafA = leafB = -1;
+                if (ANY && found) finished = true;
             }
         }
         // ---- pop the deepest deferred sibling that can still beat the best hit
@@ -303,10 +285,9 @@ __global__ void __launch_bounds__(FAST_BLOCK) k_f_trace4(SceneF sc, WaveF w, int
 // ---------------------------------------------------------------- own tree: SAH, four children per record, child links
 // Same warp organisation as k_f_trace4 (ray replacement, two node steps per iteration, vote-postponed
 // leaves), with a sorted 4-wide node step over the library's own binned-SAH tree (SceneF.own_tree, built by
-// flatten_fast_own in mfx_host.cpp).  The tree is not heap-shaped, so the deferred hits go to a real stack:
-// 8-byte entries (sort key, record that holds the child) in shared memory [entry][thread]; trees deeper than the
-// shared-memory budget overflow into a per-thread global column.  A pop re-reads the child link (one 4-byte load
-// from a record the lane fetched a few steps earlier) instead of carrying it through the sorting network.
+// flatten_fast_own in mfx_host.cpp).  The tree is not heap-shaped, so the deferred hits go to a real stack; its layout,
+// the child order (sort4), push, pop and launch geometry are shared with k_h_trace (mfx_fast_dev.cuh), like the ray
+// replacement, leaf vote and watchdog of all three persistent-warp kernels.
 // MFX_SKY_TRACER, late bounces (TAIL): the lane that finishes a closest-hit query shades it on the spot (one level of
 // GetColor: sky_scatter_f, the function k_f_shade_sky calls too -- NOINLINE, so both run the same machine code and a
 // frame does not depend on which of them shaded a vertex) and carries the scattered ray on until the path ends.  One
@@ -333,7 +314,6 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
     uint2 *my_spill = sc.stack_spill + ((size_t)blockIdx.x * FAST_BLOCK + threadIdx.x);
     const size_t spill_stride = (size_t)sc.spill_threads;
     const unsigned FULL = 0xffffffffu;
-    const unsigned lane = threadIdx.x & 31u;
     const int n = ANY ? w.counts[CNT_SH(bounce)] : w.counts[bounce];
     const float4 *ro = ANY ? w.sh_o : w.ray_o[bounce & 1], *rd = ANY ? w.sh_d : w.ray_d[bounce & 1];
     int *cursor = &w.counts[ANY ? CUR_SH(bounce) : CUR_EXT(bounce)];
@@ -352,31 +332,18 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
     float4 thr = make_float4(1.f, 1.f, 1.f, 0.f);   // TAIL: product of the attenuations so far
 
     for (;;) {
-        const unsigned idle = __ballot_sync(FULL, pid < 0);
-        unsigned idle_now = idle;
-        if (++iters > (TAIL ? (1u << 26) : (1u << 22))) { if (lane == 0) atomicAdd(&w.counts[MFX_COUNTS_LEN - 1], 1); break; }   // watchdog
-        if (!exhausted && __popc(idle) >= TRACE6_REFILL_T) {
-            const int nidle = __popc(idle);
-            int base = 0;
-            if (lane == 0) base = atomicAdd(cursor, nidle);
-            base = __shfl_sync(FULL, base, 0);
-            if (base + nidle >= n) exhausted = true;
-            if (pid < 0) {
-                const int idx = base + __popc(idle & ((1u << lane) - 1u));
-                if (idx < n) {
-                    pid = idx;                                          // the ray lives at its queue position
-                    float4 o = make_float4(sc.cam.pos[0], sc.cam.pos[1], sc.cam.pos[2], __int_as_float(-1));
-                    if (!cam0) o = ro[pid];
-                    const float4 d = rd[pid];
-                    r = make_ray_fast(f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), w.tmin, __float_as_int(o.w));
-                    best_t = ANY ? d.w - 1e-6f : w.tmax;                // shadow: dist - 1e-6 (Integrators.fs:44); closest: tMax (:108)
-                    best_slot = -1; sp = 0; leafA = -1; node = 0; needPop = false;
-                    if (TAIL) { path = __float_as_int(d.w); bnc = bounce; thr = w.thr[bounce & 1][pid]; }
-                }
-            }
-            idle_now = __ballot_sync(FULL, pid < 0);
-        }
-        if (idle_now == FULL) { if (exhausted) break; continue; }
+        unsigned idle = __ballot_sync(FULL, pid < 0);
+        if (watchdog_tripped(iters, TAIL ? (1u << 26) : (1u << 22), w.counts)) break;
+        idle = warp_refill(idle, TRACE6_REFILL_T, cursor, n, exhausted, pid, [&] {       // the ray lives at its queue position
+            float4 o = make_float4(sc.cam.pos[0], sc.cam.pos[1], sc.cam.pos[2], __int_as_float(-1));
+            if (!cam0) o = ro[pid];
+            const float4 d = rd[pid];
+            r = make_ray_fast(f3(o.x, o.y, o.z), f3(d.x, d.y, d.z), w.tmin, __float_as_int(o.w));
+            best_t = ANY ? d.w - 1e-6f : w.tmax;                // shadow: dist - 1e-6 (Integrators.fs:44); closest: tMax (:108)
+            best_slot = -1; sp = 0; leafA = -1; node = 0; needPop = false;
+            if (TAIL) { path = __float_as_int(d.w); bnc = bounce; thr = w.thr[bounce & 1][pid]; }
+        });
+        if (idle == FULL) { if (exhausted) break; continue; }
 
 #pragma unroll
         for (int rep = 0; rep < TRACE6_NSTEP; rep++)
@@ -403,28 +370,13 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
             }
             QUAD_SLOT(0, x) QUAD_SLOT(1, y) QUAD_SLOT(2, z) QUAD_SLOT(3, w)
 #undef QUAD_SLOT
-            // sorting network (0,1)(2,3)(0,2)(1,3)(1,2)
-            unsigned a0 = umin_(key[0], key[1]), a1 = umax_(key[0], key[1]);
-            unsigned a2 = umin_(key[2], key[3]), a3 = umax_(key[2], key[3]);
-            const unsigned k0 = umin_(a0, a2), t2 = umax_(a0, a2);
-            const unsigned t1 = umin_(a1, a3), k3 = umax_(a1, a3);
-            const unsigned k1 = umin_(t1, t2), k2 = umax_(t1, t2);
+            unsigned k0, k1, k2, k3;
+            sort4(key, k0, k1, k2, k3);
             const bool any0 = k0 != KEY_INF;
             const bool leaf0 = any0 && (k0 & 4u);
             const int c0 = pick4(m4, k0 & 3u);
             leafA = leaf0 ? c0 : -1;
-            // deferred hits: everything behind the one consumed now, nearest on top of the stack
-            const int m = (k1 != KEY_INF ? 1 : 0) + (k2 != KEY_INF ? 1 : 0) + (k3 != KEY_INF ? 1 : 0);
-#define STACK_PUT(I, K)                                                                                              \
-            { const int i_ = (I); const uint2 v_ = make_uint2((K), (unsigned)node);                                  \
-              DBG_CHECK(i_ >= 0 && i_ < 3 * sc.own_depth, w.counts);                                                  \
-              DBG_CHECK(i_ < S || blockIdx.x * FAST_BLOCK + threadIdx.x < (unsigned)sc.spill_threads, w.counts);       \
-              if (i_ < S) my_stack[(size_t)i_ * FAST_BLOCK] = v_; else my_spill[(size_t)(i_ - S) * spill_stride] = v_; }
-            if (m >= 1) STACK_PUT(sp + m - 1, k1)
-            if (m >= 2) STACK_PUT(sp + m - 2, k2)
-            if (m >= 3) STACK_PUT(sp, k3)
-#undef STACK_PUT
-            sp += m;
+            sp = own_push(my_stack, my_spill, S, spill_stride, sp, k1, k2, k3, node, sc, w.counts);
             const bool descend = any0 && !leaf0;
             needPop = !descend;
             if (descend) node = ~c0;
@@ -432,30 +384,19 @@ __global__ void __launch_bounds__(FAST_BLOCK, MINB) k_f_trace6(SceneF sc, WaveF 
             DBG_CHECK(leafA < 0 || ((leafA >> 3) >= 0 && (leafA >> 3) + (leafA & 7) <= sc.n_slots), w.counts);
         }
         bool finished = false;
-        const unsigned lp = __ballot_sync(FULL, pid >= 0 && leafA >= 0);
-        if (lp) {
-            const unsigned nd = ~idle_now & ~lp;
-            if (__popc(lp) >= TRACE6_LEAF_T || nd == 0u) {
-                if (pid >= 0 && leafA >= 0) {
-                    const bool found = leaf_f3<COUNT, BIG>(sc, r, leafA, best_t, best_slot, local);
-                    leafA = -1;
-                    if (ANY && found) finished = true;
-                }
+        if (leaf_vote(__ballot_sync(FULL, pid >= 0 && leafA >= 0), idle, TRACE6_LEAF_T)) {
+            if (pid >= 0 && leafA >= 0) {
+                const bool found = leaf_f3<COUNT, BIG>(sc, r, leafA, best_t, best_slot, local);
+                leafA = -1;
+                if (ANY && found) finished = true;
             }
         }
         if (pid >= 0 && needPop && leafA < 0 && !finished) {
-            for (;;) {
-                if (sp == 0) { finished = true; break; }
-                --sp;
-                const uint2 e = (sp < S) ? my_stack[(size_t)sp * FAST_BLOCK] : my_spill[(size_t)(sp - S) * spill_stride];
-                if (ANY || __uint_as_float(e.x & ~7u) <= best_t) {
-                    const int link = __ldg(reinterpret_cast<const int *>(&sc.quads[e.y].meta) + (e.x & 3u));
-                    if (e.x & 4u) leafA = link;
-                    else { node = ~link; needPop = false; }
-                    DBG_CHECK(e.y < (unsigned)sc.n_quads && ((e.x & 4u) ? (link >= 0 && (link >> 3) + (link & 7) <= sc.n_slots) : (unsigned)~link < (unsigned)sc.n_quads), w.counts);
-                    break;
-                }
-            }
+            const OwnPop p = own_pop<ANY>(my_stack, my_spill, S, spill_stride, sp, best_t, sc, w.counts);
+            sp = p.sp;
+            if (!p.found) finished = true;
+            else if (p.leaf) leafA = p.link;
+            else { node = ~p.link; needPop = false; }
         }
         if (TAIL && finished) {
             // GetColor's next level, here and now (RayTracing.fs:367-382): a miss ends the path with T * sky, a hit at the
@@ -1025,16 +966,10 @@ static void launch_trace4(const LaunchCfg &c, const SceneF &sc, const WaveF &w, 
     const size_t smem = ANY ? 0 : (size_t)sc.levels * FAST_BLOCK * sizeof(float);
     k_f_trace4<ANY, BIG><<<persistent_blocks(k_f_trace4<ANY, BIG>, FAST_BLOCK, c.blocks, smem), FAST_BLOCK, smem, c.stream>>>(sc, w, bounce, ctr);
 }
-static_assert(MFX_STACK_SMEM_MAX * FAST_BLOCK * sizeof(uint2) <= 48 * 1024, "the own-tree stack must launch without a shared-memory opt-in");
 template <bool ANY, bool BIG, int MB, bool CNT, bool TAIL = false>
 static void launch_trace6(const LaunchCfg &c, const SceneF &sc, const WaveF &w, int bounce, TravCounters *ctr, const SkyCtx &sky = SkyCtx{})
 {
-    const size_t smem = (size_t)sc.stack_smem * FAST_BLOCK * sizeof(uint2);
-    // the spill columns were sized for spill_threads: never launch more threads than that
-    int blocks = persistent_blocks(k_f_trace6<ANY, BIG, MB, CNT, TAIL>, FAST_BLOCK, c.blocks, smem);
-    if (sc.stack_spill && blocks * FAST_BLOCK > sc.spill_threads) blocks = sc.spill_threads / FAST_BLOCK;
-    if (c.max_items > 0) blocks = std::max(1, std::min(blocks, (c.max_items + FAST_BLOCK - 1) / FAST_BLOCK));
-    k_f_trace6<ANY, BIG, MB, CNT, TAIL><<<blocks, FAST_BLOCK, smem, c.stream>>>(sc, w, bounce, ctr, sky);
+    k_f_trace6<ANY, BIG, MB, CNT, TAIL><<<own_tree_blocks(k_f_trace6<ANY, BIG, MB, CNT, TAIL>, c, sc), FAST_BLOCK, own_stack_smem(sc), c.stream>>>(sc, w, bounce, ctr, sky);
 }
 // The layout decides the kernel: the reference tree is passed for the instrumented counting runs (the algorithmic record
 // counts of the roofline are defined on the reference's binary tree) and takes k_f_trace4; the library's SAH tree takes

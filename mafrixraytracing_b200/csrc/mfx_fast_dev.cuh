@@ -1,7 +1,9 @@
 // mfx_fast_dev.cuh -- f32 device helpers shared by the wavefront kernels (mfx_fast.cu) and the id-exact hybrid
-// traversal (mfx_hybrid.cu): ray setup, 256-bit record loads, the 4-key sorting helpers, queue-count indices.
+// traversal (mfx_hybrid.cu): ray setup, 256-bit record loads, queue-count indices, and the own tree's child order,
+// traversal stack and launch geometry.
 #pragma once
 #include "mfx_device.cuh"
+#include <algorithm>
 
 typedef V3<float> F3;
 
@@ -85,4 +87,115 @@ __device__ __forceinline__ int pick4(const float4 &m, unsigned id)
 {
     const float lo = (id & 1u) ? m.y : m.x, hi = (id & 1u) ? m.w : m.z;
     return __float_as_int((id & 2u) ? hi : lo);
+}
+
+// ---------------------------------------------------------------- persistent warps (k_f_trace4, k_f_trace6, k_h_trace)
+// Watchdog: the loop is bounded so a logic error can never hang the GPU; a trip raises the flag in counts[] (Sample fails).
+__device__ __forceinline__ bool watchdog_tripped(unsigned &iters, unsigned limit, int *counts)
+{
+    if (++iters <= limit) return false;
+    if ((threadIdx.x & 31u) == 0) atomicAdd(&counts[MFX_COUNTS_LEN - 1], 1);
+    return true;
+}
+
+// Ray replacement: once >= T lanes of the warp are idle (and the queue is not exhausted) the warp claims that many of the n
+// queue entries with one atomicAdd on the cursor (ballot / popc / shuffle); an idle lane whose entry exists takes it as
+// `pid` (the ray lives at its queue position) and runs start().  `exhausted` is set once a claim reaches the end of the
+// queue.  Returns the mask of the lanes still idle.  A batch of refills pays one cursor round trip for many rays, and rays
+// that start together are neighbours in the queue.
+template <typename Start>
+__device__ __forceinline__ unsigned warp_refill(unsigned idle, int T, int *cursor, int n, bool &exhausted, int &pid, Start start)
+{
+    if (exhausted || __popc(idle) < T) return idle;
+    const unsigned lane = threadIdx.x & 31u;
+    const int nidle = __popc(idle);
+    int base = 0;
+    if (lane == 0) base = atomicAdd(cursor, nidle);
+    base = __shfl_sync(0xffffffffu, base, 0);
+    if (base + nidle >= n) exhausted = true;
+    if (pid < 0) {
+        const int idx = base + __popc(idle & ((1u << lane) - 1u));
+        if (idx < n) { pid = idx; start(); }
+    }
+    return __ballot_sync(0xffffffffu, pid < 0);
+}
+
+// Leaf vote: the lanes in `leaves` run their leaf tests
+// once >= T of them hold a leaf, or no lane has node work left.
+__device__ __forceinline__ bool leaf_vote(unsigned leaves, unsigned idle, int T)
+{
+    return leaves && (__popc(leaves) >= T || (~idle & ~leaves) == 0u);
+}
+
+// ---------------------------------------------------------------- the own tree's traversal stack (k_f_trace6, k_h_trace)
+// Child order of a node step: the sorting network (0,1)(2,3)(0,2)(1,3)(1,2) over the four slot keys, k0 nearest.
+__device__ __forceinline__ void sort4(const unsigned (&key)[4], unsigned &k0, unsigned &k1, unsigned &k2, unsigned &k3)
+{
+    const unsigned a0 = umin_(key[0], key[1]), a1 = umax_(key[0], key[1]);
+    const unsigned a2 = umin_(key[2], key[3]), a3 = umax_(key[2], key[3]);
+    k0 = umin_(a0, a2); const unsigned t2 = umax_(a0, a2);
+    const unsigned t1 = umin_(a1, a3); k3 = umax_(a1, a3);
+    k1 = umin_(t1, t2); k2 = umax_(t1, t2);
+}
+
+// One thread's stack of deferred hits.  An entry is (sort key of the child, record that holds it); the key's low bits are
+// leaf << 2 | slot.  Entries [0, S) sit in dynamic shared memory as [entry][thread] (conflict free: my_stack = s_stack +
+// threadIdx.x), deeper ones in the thread's global spill column (my_spill = stack_spill + blockIdx.x * FAST_BLOCK +
+// threadIdx.x, stride spill_threads: own_tree_blocks keeps a launch inside the columns own_spill_entries sized).
+__device__ __forceinline__ void own_put(uint2 *my_stack, uint2 *my_spill, int S, size_t spill_stride, int i, uint2 v,
+                                        const SceneF &sc, int *counts)
+{
+    DBG_CHECK(i >= 0 && i < 3 * sc.own_depth, counts);
+    DBG_CHECK(i < S || blockIdx.x * FAST_BLOCK + threadIdx.x < (unsigned)sc.spill_threads, counts);
+    if (i < S) my_stack[(size_t)i * FAST_BLOCK] = v; else my_spill[(size_t)(i - S) * spill_stride] = v;
+}
+
+// Defers the hits behind the one a node step consumes now (k1..k3 sorted, KEY_INF: none) with record `node`, nearest on top.
+__device__ __forceinline__ int own_push(uint2 *my_stack, uint2 *my_spill, int S, size_t spill_stride, int sp,
+                                        unsigned k1, unsigned k2, unsigned k3, int node, const SceneF &sc, int *counts)
+{
+    const int m = (k1 != KEY_INF ? 1 : 0) + (k2 != KEY_INF ? 1 : 0) + (k3 != KEY_INF ? 1 : 0);
+    if (m >= 1) own_put(my_stack, my_spill, S, spill_stride, sp + m - 1, make_uint2(k1, (unsigned)node), sc, counts);
+    if (m >= 2) own_put(my_stack, my_spill, S, spill_stride, sp + m - 2, make_uint2(k2, (unsigned)node), sc, counts);
+    if (m >= 3) own_put(my_stack, my_spill, S, spill_stride, sp, make_uint2(k3, (unsigned)node), sc, counts);
+    return sp + m;
+}
+
+// Pops the deepest entry whose entry distance is <= limit (ANY: the top one, never culls) and re-reads its child link from
+// the record that holds it.
+struct OwnPop {
+    int sp;         // stack height after the pop
+    int link;       // the child's link: leaf meta, or ~record of an interior child
+    bool found;     // false: the stack ran empty
+    bool leaf;
+};
+template <bool ANY>
+__device__ __forceinline__ OwnPop own_pop(const uint2 *my_stack, const uint2 *my_spill, int S, size_t spill_stride, int sp,
+                                          float limit, const SceneF &sc, int *counts)
+{
+    OwnPop r;
+    for (;;) {
+        if (sp == 0) { r.sp = 0; r.found = false; r.leaf = false; r.link = 0; return r; }
+        --sp;
+        const uint2 e = (sp < S) ? my_stack[(size_t)sp * FAST_BLOCK] : my_spill[(size_t)(sp - S) * spill_stride];
+        if (ANY || __uint_as_float(e.x & ~7u) <= limit) {
+            const int link = __ldg(reinterpret_cast<const int *>(&sc.quads[e.y].meta) + (e.x & 3u));
+            DBG_CHECK(e.y < (unsigned)sc.n_quads && ((e.x & 4u) ? (link >= 0 && (link >> 3) + (link & 7) <= sc.n_slots) : (unsigned)~link < (unsigned)sc.n_quads), counts);
+            r.sp = sp; r.link = link; r.found = true; r.leaf = (e.x & 4u) != 0;
+            return r;
+        }
+    }
+}
+
+// Launch geometry of the own-tree kernels: the shared part of the stack as dynamic shared memory, a persistent grid that
+// never runs more threads than the spill columns were sized for, nor more blocks than max_items entries can occupy.
+static_assert(MFX_STACK_SMEM_MAX * FAST_BLOCK * sizeof(uint2) <= 48 * 1024, "the own-tree stack must launch without a shared-memory opt-in");
+static inline size_t own_stack_smem(const SceneF &sc) { return (size_t)sc.stack_smem * FAST_BLOCK * sizeof(uint2); }
+template <typename K>
+static inline int own_tree_blocks(K kernel, const LaunchCfg &c, const SceneF &sc)
+{
+    int blocks = persistent_blocks(kernel, FAST_BLOCK, c.blocks, own_stack_smem(sc));
+    if (sc.stack_spill && blocks * FAST_BLOCK > sc.spill_threads) blocks = sc.spill_threads / FAST_BLOCK;
+    if (c.max_items > 0) blocks = std::max(1, std::min(blocks, (c.max_items + FAST_BLOCK - 1) / FAST_BLOCK));
+    return blocks;
 }

@@ -851,12 +851,11 @@ static int flatten_fast(MfxScene *s)
     sf.ref_id = nullptr;                                        // b.w already holds the caller's primitive index
     sf.root_meta = -1;
     sf.own_tree = 1; sf.own_depth = host->depth;
-    const int need = 3 * host->depth;
-    sf.stack_smem = (int)std::min((long)std::min(need, MFX_STACK_SMEM_MAX), std::max(1L, env_long("MFX_STACK_SMEM", 12)));
+    sf.stack_smem = (int)std::min((long)std::min(3 * host->depth, MFX_STACK_SMEM_MAX), std::max(1L, env_long("MFX_STACK_SMEM", 12)));
     sf.spill_threads = s->sm_count * 16 * 128;                  // most threads a persistent 128-thread grid can hold
-    if (need > sf.stack_smem) {
-        MFX_TRY(dev_alloc_t(s, &sf.stack_spill, (size_t)(need - sf.stack_smem) * sf.spill_threads));
-        s->f_bytes += (uint64_t)(need - sf.stack_smem) * sf.spill_threads * sizeof(uint2);
+    if (const size_t spill = own_spill_entries(sf)) {
+        MFX_TRY(dev_alloc_t(s, &sf.stack_spill, spill));
+        s->f_bytes += spill * sizeof(uint2);
     }
     MFX_TRY(fill_fast_common(s, sf));
     sf.n_slots = ns;
@@ -1334,7 +1333,7 @@ static int launch_sample(MfxScene *s, const MfxSampleParams *p, double *d_color_
     const SceneF *sfp_sh = sfp;
     SceneF sf_sh;
     if (two && sfp->stack_spill) {
-        if (!s->spill2) MFX_TRY(dev_alloc_t(s, &s->spill2, (size_t)(3 * sfp->own_depth - sfp->stack_smem) * sfp->spill_threads));
+        if (!s->spill2) MFX_TRY(dev_alloc_t(s, &s->spill2, own_spill_entries(*sfp)));
         sf_sh = *sfp;
         sf_sh.stack_spill = s->spill2;
         sfp_sh = &sf_sh;

@@ -7,7 +7,8 @@
 //     first minimal key (`Array.minBy`, :76-80);
 //     a primitive is tested iff AABB.hit (IHitable.fs:18-54) passes for its leaf and every ancestor.
 // That answer does not depend on the tree that finds it, so this kernel walks the library's own SAH tree with the
-// persistent-warp machinery of k_f_trace6 (mfx_fast.cu) and makes only the DECISIONS in f64:
+// persistent-warp machinery of k_f_trace6 (mfx_fast.cu; the stack, child order, ray replacement, leaf vote, watchdog and
+// launch geometry of mfx_fast_dev.cuh) and makes only the DECISIONS in f64:
 //   * node step: f32 slab tests, boxes padded per ray by 4e-6 x (|scene| + |origin|) -- eight times the worst
 //     accumulated rounding between the f64 ray and the f32 arithmetic (ray rounded to f32, rcp.approx, o/d product,
 //     fma) -- so a box that holds an f64 hit is never culled; the t-shrink limit is best_t rounded UP to f32 and a
@@ -175,7 +176,6 @@ __global__ void __launch_bounds__(FAST_BLOCK, 5) k_h_trace(SceneF sc, const Node
     uint2 *my_spill = sc.stack_spill + ((size_t)blockIdx.x * FAST_BLOCK + threadIdx.x);
     const size_t spill_stride = (size_t)sc.spill_threads;
     const unsigned FULL = 0xffffffffu;
-    const unsigned lane = threadIdx.x & 31u;
     const int n = w.counts[bounce];
     int *cursor = &w.counts[CUR_EXT(bounce)];
 
@@ -190,36 +190,23 @@ __global__ void __launch_bounds__(FAST_BLOCK, 5) k_h_trace(SceneF sc, const Node
     unsigned iters = 0u;
 
     for (;;) {
-        const unsigned idle = __ballot_sync(FULL, pid < 0);
-        unsigned idle_now = idle;
-        if (++iters > (1u << 22)) { if (lane == 0) atomicAdd(&w.counts[MFX_COUNTS_LEN - 1], 1); break; }   // watchdog
-        if (!exhausted && __popc(idle) >= REFILL_T) {
-            const int nidle = __popc(idle);
-            int base = 0;
-            if (lane == 0) base = atomicAdd(cursor, nidle);
-            base = __shfl_sync(FULL, base, 0);
-            if (base + nidle >= n) exhausted = true;
-            if (pid < 0) {
-                const int idx = base + __popc(idle & ((1u << lane) - 1u));
-                if (idx < n) {
-                    pid = idx;
-                    const double *dir = wh.dir64 + 3 * (size_t)pid;
-                    const D3 o64 = hyb_origin(wh, cam_o, cam0, pid);
-                    const F3 o = f3((float)o64.x, (float)o64.y, (float)o64.z);
-                    const F3 d = f3((float)dir[0], (float)dir[1], (float)dir[2]);
-                    const RayF r = make_ray_fast(o, d, HYB_TMIN_BOX, -1);
-                    idir = r.idir;
-                    // per-ray pad: every box plane moves outward by `pad` in space = pad * |1/d| in t
-                    const float pad = sh.pad_factor * (sh.max_abs + fmaxf(fabsf(o.x), fmaxf(fabsf(o.y), fabsf(o.z))));
-                    const F3 pt = f3(pad * fabsf(idir.x), pad * fabsf(idir.y), pad * fabsf(idir.z));
-                    ood_n = r.ood + pt; ood_f = r.ood - pt;
-                    limit = 3.0e38f;                         // triangles ignore tMax (Trangle.fs:148): nothing is culled by it
-                    best.t = 0.; best.ref = -1; sp = 0; leafA = -1; node = 0; needPop = false;
-                }
-            }
-            idle_now = __ballot_sync(FULL, pid < 0);
-        }
-        if (idle_now == FULL) { if (exhausted) break; continue; }
+        unsigned idle = __ballot_sync(FULL, pid < 0);
+        if (watchdog_tripped(iters, 1u << 22, w.counts)) break;
+        idle = warp_refill(idle, REFILL_T, cursor, n, exhausted, pid, [&] {       // the ray lives at its queue position
+            const double *dir = wh.dir64 + 3 * (size_t)pid;
+            const D3 o64 = hyb_origin(wh, cam_o, cam0, pid);
+            const F3 o = f3((float)o64.x, (float)o64.y, (float)o64.z);
+            const F3 d = f3((float)dir[0], (float)dir[1], (float)dir[2]);
+            const RayF r = make_ray_fast(o, d, HYB_TMIN_BOX, -1);
+            idir = r.idir;
+            // per-ray pad: every box plane moves outward by `pad` in space = pad * |1/d| in t
+            const float pad = sh.pad_factor * (sh.max_abs + fmaxf(fabsf(o.x), fmaxf(fabsf(o.y), fabsf(o.z))));
+            const F3 pt = f3(pad * fabsf(idir.x), pad * fabsf(idir.y), pad * fabsf(idir.z));
+            ood_n = r.ood + pt; ood_f = r.ood - pt;
+            limit = 3.0e38f;                         // triangles ignore tMax (Trangle.fs:148): nothing is culled by it
+            best.t = 0.; best.ref = -1; sp = 0; leafA = -1; node = 0; needPop = false;
+        });
+        if (idle == FULL) { if (exhausted) break; continue; }
 
         const bool px = idir.x >= 0.f, py = idir.y >= 0.f, pz = idir.z >= 0.f;
 #pragma unroll
@@ -241,27 +228,13 @@ __global__ void __launch_bounds__(FAST_BLOCK, 5) k_h_trace(SceneF sc, const Node
             }
             QUAD_SLOT(0, x) QUAD_SLOT(1, y) QUAD_SLOT(2, z) QUAD_SLOT(3, w)
 #undef QUAD_SLOT
-            // sorting network (0,1)(2,3)(0,2)(1,3)(1,2)
-            unsigned a0 = umin_(key[0], key[1]), a1 = umax_(key[0], key[1]);
-            unsigned a2 = umin_(key[2], key[3]), a3 = umax_(key[2], key[3]);
-            const unsigned k0 = umin_(a0, a2), t2 = umax_(a0, a2);
-            const unsigned t1 = umin_(a1, a3), k3 = umax_(a1, a3);
-            const unsigned k1 = umin_(t1, t2), k2 = umax_(t1, t2);
+            unsigned k0, k1, k2, k3;
+            sort4(key, k0, k1, k2, k3);
             const bool any0 = k0 != KEY_INF;
             const bool leaf0 = any0 && (k0 & 4u);
             const int c0 = pick4(m4, k0 & 3u);
             leafA = leaf0 ? c0 : -1;
-            const int m = (k1 != KEY_INF ? 1 : 0) + (k2 != KEY_INF ? 1 : 0) + (k3 != KEY_INF ? 1 : 0);
-#define STACK_PUT(I, K)                                                                                              \
-            { const int i_ = (I); const uint2 v_ = make_uint2((K), (unsigned)node);                                  \
-              DBG_CHECK(i_ >= 0 && i_ < 3 * sc.own_depth, w.counts);                                                  \
-              DBG_CHECK(i_ < S || blockIdx.x * FAST_BLOCK + threadIdx.x < (unsigned)sc.spill_threads, w.counts);       \
-              if (i_ < S) my_stack[(size_t)i_ * FAST_BLOCK] = v_; else my_spill[(size_t)(i_ - S) * spill_stride] = v_; }
-            if (m >= 1) STACK_PUT(sp + m - 1, k1)
-            if (m >= 2) STACK_PUT(sp + m - 2, k2)
-            if (m >= 3) STACK_PUT(sp, k3)
-#undef STACK_PUT
-            sp += m;
+            sp = own_push(my_stack, my_spill, S, spill_stride, sp, k1, k2, k3, node, sc, w.counts);
             const bool descend = any0 && !leaf0;
             needPop = !descend;
             if (descend) node = ~c0;
@@ -269,30 +242,20 @@ __global__ void __launch_bounds__(FAST_BLOCK, 5) k_h_trace(SceneF sc, const Node
             DBG_CHECK(leafA < 0 || ((leafA >> 3) >= 0 && (leafA >> 3) + (leafA & 7) <= sc.n_slots), w.counts);
         }
         bool finished = false;
-        const unsigned lp = __ballot_sync(FULL, pid >= 0 && leafA >= 0);
-        if (lp) {
-            const unsigned nd = ~idle_now & ~lp;
-            if (__popc(lp) >= LEAF_T || nd == 0u) {
-                if (pid >= 0 && leafA >= 0) {
-                    best = hyb_leaf(sh.prims_h, sh.leaf_of_ref, ref_id, hyb_origin(wh, cam_o, cam0, pid), wh.dir64 + 3 * (size_t)pid,
-                                    leafA, q.tmin, q.tmax, q.sky, best);
-                    if (best.ref >= 0) limit = __double2float_ru(best.t);
-                    leafA = -1;
-                }
+        if (leaf_vote(__ballot_sync(FULL, pid >= 0 && leafA >= 0), idle, LEAF_T)) {
+            if (pid >= 0 && leafA >= 0) {
+                best = hyb_leaf(sh.prims_h, sh.leaf_of_ref, ref_id, hyb_origin(wh, cam_o, cam0, pid), wh.dir64 + 3 * (size_t)pid,
+                                leafA, q.tmin, q.tmax, q.sky, best);
+                if (best.ref >= 0) limit = __double2float_ru(best.t);
+                leafA = -1;
             }
         }
         if (pid >= 0 && needPop && leafA < 0) {
-            for (;;) {
-                if (sp == 0) { finished = true; break; }
-                --sp;
-                const uint2 e = (sp < S) ? my_stack[(size_t)sp * FAST_BLOCK] : my_spill[(size_t)(sp - S) * spill_stride];
-                if (__uint_as_float(e.x & ~7u) <= limit) {
-                    const int link = __ldg(reinterpret_cast<const int *>(&sc.quads[e.y].meta) + (e.x & 3u));
-                    if (e.x & 4u) leafA = link;
-                    else { node = ~link; needPop = false; }
-                    break;
-                }
-            }
+            const OwnPop p = own_pop<false>(my_stack, my_spill, S, spill_stride, sp, limit, sc, w.counts);
+            sp = p.sp;
+            if (!p.found) finished = true;
+            else if (p.leaf) leafA = p.link;
+            else { node = ~p.link; needPop = false; }
         }
         if (finished) {
             int ref = best.ref;
@@ -540,12 +503,8 @@ void mfx_h_seam_setup(const LaunchCfg &c, const SceneX &sx, const WaveF &w, cons
 void mfx_h_extend(const LaunchCfg &c, const SceneF &sc, const SceneX &sx, const SceneH &sh, const WaveF &w, const WaveH &wh, int bounce, HybQuery q, int seam)
 {
     cudaMemsetAsync(wh.fix_n, 0, sizeof(int), c.stream);
-    const size_t smem = (size_t)sc.stack_smem * FAST_BLOCK * sizeof(uint2);
-    int blocks = persistent_blocks(k_h_trace, FAST_BLOCK, c.blocks, smem);
-    if (sc.stack_spill && blocks * FAST_BLOCK > sc.spill_threads) blocks = sc.spill_threads / FAST_BLOCK;
-    if (c.max_items > 0) blocks = std::max(1, std::min(blocks, (c.max_items + FAST_BLOCK - 1) / FAST_BLOCK));
     D3 cam_o; cam_o.x = sx.cam.pos[0]; cam_o.y = sx.cam.pos[1]; cam_o.z = sx.cam.pos[2];
-    k_h_trace<<<blocks, FAST_BLOCK, smem, c.stream>>>(sc, sx.nodes, sx.ref_id, sh, w, wh, bounce, q, cam_o, w.cam_origin, seam);
+    k_h_trace<<<own_tree_blocks(k_h_trace, c, sc), FAST_BLOCK, own_stack_smem(sc), c.stream>>>(sc, sx.nodes, sx.ref_id, sh, w, wh, bounce, q, cam_o, w.cam_origin, seam);
     k_h_fixup<<<c.blocks * 4, 128, 0, c.stream>>>(sx, sh, w, wh, bounce, q, w.cam_origin, seam);
 }
 void mfx_h_extend_x(const LaunchCfg &c, const SceneF &sc, const SceneX &sx, const SceneH &sh, const WaveX &wx, const WaveF &w, const WaveH &wh, int bounce, HybQuery q)

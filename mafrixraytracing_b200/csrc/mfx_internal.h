@@ -146,6 +146,13 @@ struct SceneF {
                             // launch that may run beside another one needs columns of its own
     int    spill_threads;
 };
+// Entries of a stack_spill buffer: what 3 * own_depth entries per thread leave beyond the stack_smem in shared memory, for
+// each of spill_threads threads; 0 when shared memory holds the whole stack.
+static inline size_t own_spill_entries(const SceneF &sf)
+{
+    const int over = 3 * sf.own_depth - sf.stack_smem;
+    return over > 0 ? (size_t)over * sf.spill_threads : 0;
+}
 
 // Path state lives at QUEUE POSITIONS, not at path ids: the shade kernel of bounce b reads entry i of buffer b&1 and
 // writes the survivors densely into buffer (b+1)&1 (and the shadow rays densely into sh_*), so every kernel of the
